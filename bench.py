@@ -1,7 +1,10 @@
 #!/usr/bin/env python
 """Benchmark of the AlterEgo-construction hot path (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg2|...]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg2|...] [--dump-outputs DIR]
+
+--dump-outputs DIR (--impl ours only: the reference arm times a CPU port on samples and returns no tables) writes
+what the last timed step returned, the neighbour tables of engine.SimTables, as DIR/<name>.npy.
 
 A "step" is one pass of the similarity stage (all item rows: co-rating SpGEMM +
 epilogue + top-k selection, passes 1 and 2) over the synthetic two-domain
@@ -110,6 +113,36 @@ def make_pipelines(name):
 def make_workload(name):
     """First (for a two-domain shape: the only) pipeline of a workload."""
     return make_pipelines(name)[0]
+
+
+DUMP_BUDGET = 48 << 20       # bytes --dump-outputs may write (the tables of a large workload: a fixed sample of rows)
+DUMP_FIELDS = (("row_flags", np.float32), ("row_npairs", np.float64), ("row_nkept", np.float64), ("tab_len", np.float32),
+               ("tab_idx", np.float32), ("tab_sim", np.float64), ("tab_mutu", np.float32), ("tab_n", np.float32))
+
+
+def dump_rows(pipes, k):
+    """Item rows whose tables --dump-outputs writes, per pipeline: all of them if they fit DUMP_BUDGET, else a fixed,
+    seeded sample (the same rows in every run with the same arguments), sorted."""
+    n_rows = DUMP_BUDGET // (len(pipes) * (36 + 40 * k))        # bytes per row of the files DUMP_FIELDS make
+    return [np.arange(wl["n_items"]) if wl["n_items"] <= n_rows else
+            np.sort(np.random.default_rng(0).choice(wl["n_items"], n_rows, replace=False)) for wl in pipes]
+
+
+def snapshot_tables(tabs_all, rows_all):
+    """Host copy of what a caller of the similarity step receives (engine.SimTables), on the dumped rows: ids and
+    counts of items and users as float32 (exact below 2^24), pair counts and similarities as float64."""
+    import torch
+    out = {}
+    for q, (tabs, rows) in enumerate(zip(tabs_all, rows_all)):
+        pre = "" if len(tabs_all) == 1 else "pipeline%d_" % q
+        r = torch.as_tensor(rows, device=tabs.tab_sim.device)
+        out[pre + "rows"] = rows.astype(np.float64)
+        out[pre + "n_pairs_total"] = np.array([tabs.n_pairs_total], dtype=np.float64)
+        for name, dt in DUMP_FIELDS:
+            a = getattr(tabs, name).index_select(0, r).cpu().numpy()
+            assert dt != np.float32 or a.size == 0 or np.abs(a).max() < 1 << 24, name
+            out[pre + name] = a.astype(dt)
+    return out
 
 
 def workload_label(wl, method):
@@ -273,7 +306,14 @@ def main():
     ap.add_argument("--method", default="adjust_cosine")
     ap.add_argument("--no-pipeline", action="store_true", help="skip the extension/generation timing")
     ap.add_argument("--no-cpu", action="store_true", help="skip the CPU baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the neighbour tables of the last timed step to DIR/<name>.npy (float32 / float64; "
+                         "a fixed sample of item rows when they exceed %d MB)" % (DUMP_BUDGET >> 20))
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the tables of the GPU path (--impl ours)")
     # exactly one JSON line may reach stdout: libraries (NCCL's version banner) write there too, so
     # stdout is pointed at stderr for the duration of the run and restored for the final print
     sys.stdout.flush()
@@ -349,6 +389,8 @@ def main():
     for wl in pipes:
         wl["eng"]._check_error()
     launches = sum(wl["eng"].launches for wl in pipes) - l0
+    # the tables live in engine buffers that the next steps overwrite: copy what the last timed step computed now
+    dumped = snapshot_tables(tabs_all, dump_rows(pipes, k)) if args.dump_outputs and rank == 0 else None
     # per-kernel CUDA-event times: a second set of steps with every launch serialised on one stream
     for wl in pipes:
         wl["eng"].enable_profile()
@@ -552,6 +594,11 @@ def main():
             line["multi_parity"] = multi_parity
         if not args.no_cpu:
             line["cpu_baseline"] = cpu_baseline(pipes[0], args.method)
+        if dumped is not None:
+            assert sum(a.nbytes for a in dumped.values()) <= 64 * 10 ** 6
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in dumped.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
         emit(line)
     if world > 1:
         dist.barrier()

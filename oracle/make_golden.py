@@ -106,7 +106,7 @@ def build_case(name):
 
     if sim_only:
         out["ref_seconds"] = np.array([dt_sim, 0.0, 0.0])
-        return out
+        return compact_sim_only(out)
     xs, dt_ext = H.run_extend(tool, simRDD, k)
     xrows = xs.collect()
     out.update(xs_start=np.array([ipos[t] for t, lst in xrows for _ in lst], dtype=np.int32),
@@ -147,6 +147,37 @@ def build_case(name):
     return out
 
 
+MID_SAMPLE_RATE = 0.1      # share of the remaining pairs whose similarity a sim-only golden keeps
+
+
+def compact_sim_only(out, seed=13):
+    """Shrinks a sim-only case to well under 1 MB.  The reference's similarity records are symmetric (checked here),
+    so the keys, mutualities and labels of the pairs i < j are stored whole and the tests mirror them.  Similarity and
+    frac are kept for a fixed sample of those pairs: every pair in a neighbour list (the near-tie checks look their
+    similarity up), every pair with |sim| < 1e-9 (the rounding residues of cancelling inner products) and a seeded
+    MID_SAMPLE_RATE of the rest.  The rating times are dropped: the similarity stage does not read them."""
+    n_items = len(out["iids"])
+    si, sj = out["sim_i"].astype(np.int64), out["sim_j"].astype(np.int64)
+    key, mirror = si * n_items + sj, sj * n_items + si
+    o = np.argsort(mirror)
+    assert np.array_equal(key, mirror[o]), "similarity records are not symmetric"
+    for name in ("sim_val", "sim_mutu", "sim_frac", "sim_label"):
+        assert np.array_equal(out[name], out[name][o]), name
+    up = si < sj
+    listed = np.zeros(n_items * n_items, dtype=bool)
+    for name in ("BB_BB", "BB_NB", "NB_BB", "NB_NN"):
+        ptr, nbr = out[name + "_ptr"], out[name + "_nbr"].astype(np.int64)
+        rows = np.repeat(np.arange(n_items), np.diff(ptr))
+        listed[rows * n_items + nbr] = listed[nbr * n_items + rows] = True
+    val = out["sim_val"][up]
+    keep = listed[key[up]] | (np.abs(val) < 1e-9) | (np.random.default_rng(seed).random(len(val)) < MID_SAMPLE_RATE)
+    sample = np.flatnonzero(keep).astype(np.int32)
+    small = {k: v for k, v in out.items() if k != "ts" and not k.startswith("sim_")}
+    return dict(small, pair_ptr=np.searchsorted(si[up], np.arange(n_items + 1)).astype(np.int32),
+                pair_j=out["sim_j"][up], pair_mutu=out["sim_mutu"][up], pair_label=out["sim_label"][up],
+                sample=sample, sample_sim=val[sample], sample_frac=out["sim_frac"][up][sample])
+
+
 def hash_det(u, i):
     """Deterministic (process-independent) parity bit for the half-rating case."""
     return sum(ord(c) for c in u) + sum(ord(c) for c in i)
@@ -161,7 +192,7 @@ def main():
         path = os.path.join(gdir, name + ".npz")
         np.savez_compressed(path, **out)
         print("%-18s pairs=%d bb=%d xsim=%d  ref s=%s  (%.1fs) -> %s (%d KB)" % (
-            name, len(out["sim_i"]), int(out["bb"].sum()), len(out.get("xs_val", ())),
+            name, len(out["sim_i"]) if "sim_i" in out else 2 * len(out["pair_j"]), int(out["bb"].sum()), len(out.get("xs_val", ())),
             np.round(out["ref_seconds"], 2), time.time() - t0, path,
             os.path.getsize(path) // 1024))
 

@@ -19,7 +19,27 @@ SIM_RTOL = 1e-5          # BASELINE.json north_star: similarities within 1e-5 re
 
 def load_golden(name):
     g = np.load(os.path.join(GOLDEN_DIR, name + ".npz"))
-    return {k: g[k] for k in g.files}
+    g = {k: g[k] for k in g.files}
+    return expand_pairs(g) if "pair_ptr" in g else g
+
+
+def expand_pairs(g):
+    """A compact sim-only golden (oracle/make_golden.compact_sim_only: the pairs i < j, similarity and frac on a
+    sample of them) -> every directed pair sorted by (i, j), as the other goldens hold them; sim_val and sim_frac
+    are NaN where the sample has no value."""
+    n_items = len(g["iids"])
+    i = np.repeat(np.arange(n_items), np.diff(g["pair_ptr"]))
+    j = g["pair_j"].astype(np.int64)
+    val = np.full(len(j), np.nan)
+    val[g["sample"]] = g["sample_sim"]
+    frac = np.full(len(j), np.nan, dtype=np.float32)
+    frac[g["sample"]] = g["sample_frac"]
+    ii, jj = np.concatenate([i, j]), np.concatenate([j, i])
+    o = np.argsort(ii * n_items + jj)
+    idt = g["pair_j"].dtype
+    return dict(g, sim_i=ii[o].astype(idt), sim_j=jj[o].astype(idt), sim_val=np.concatenate([val, val])[o],
+                sim_mutu=np.concatenate([g["pair_mutu"]] * 2)[o], sim_label=np.concatenate([g["pair_label"]] * 2)[o],
+                sim_frac=np.concatenate([frac, frac])[o])
 
 
 def golden_meta(g):

@@ -45,12 +45,15 @@ def test_sim_matches_reference_mid_size_golden():
     gi, gj = pairs["i"].cpu().numpy(), pairs["j"].cpu().numpy()
     assert np.array_equal(gi, g["sim_i"]) and np.array_equal(gj, g["sim_j"]), "kept-pair sets differ"
     assert np.array_equal(pairs["mutu"].cpu().numpy(), g["sim_mutu"]) and np.array_equal(pairs["label"].cpu().numpy(), g["sim_label"])
-    assert np.array_equal(pairs["frac"].cpu().numpy().astype(np.float32), g["sim_frac"])
-    rel = np.abs(pairs["sim"].cpu().numpy() - g["sim_val"]) / np.abs(g["sim_val"])
+    known = np.isfinite(g["sim_val"])          # similarity and frac are stored for a fixed sample of the pairs
+    assert known.sum() > 70000
+    assert np.array_equal(pairs["frac"].cpu().numpy()[known].astype(np.float32), g["sim_frac"][known])
+    rel = np.zeros(len(known))
+    rel[known] = np.abs(pairs["sim"].cpu().numpy()[known] - g["sim_val"][known]) / np.abs(g["sim_val"][known])
     # |sim| < 1e-13 is the rounding residue of an inner product that cancels exactly (here one pair of two co-raters,
     # 1.1e-19 in the reference, 1.5e-19 here): not comparable digit by digit, see DESIGN.md 6.1
-    rel[np.abs(g["sim_val"]) < PT.FRAGILE_SIM] = 0.0
-    assert int((np.abs(g["sim_val"]) < PT.FRAGILE_SIM).sum()) <= 2
+    rel[known & (np.abs(g["sim_val"]) < PT.FRAGILE_SIM)] = 0.0
+    assert int((np.abs(g["sim_val"][known]) < PT.FRAGILE_SIM).sum()) <= 2
     if rel.max() > PT.SIM_RTOL:
         bad = np.flatnonzero(rel > PT.SIM_RTOL)
         cnt = its[:, 3]

@@ -1,63 +1,53 @@
-"""CPU: the host-side clean / split stages against the unmodified reference run through the
-oracle shim (needs /root/reference; skipped where it is not mounted)."""
-import os
+"""CPU: the host-side clean / split stages against the unmodified reference run through the oracle shim (needs the
+original X-MAP source, XMAP_REFERENCE_CODE; skipped without it), and against the records stored in
+tests/golden/cleansplit.npz (oracle/make_golden_cleansplit.py), which run everywhere."""
 import subprocess
 import sys
-import textwrap
 
 import pytest
 
+from oracle import harness as H
+from oracle import make_golden_cleansplit as CS
 from tests import parity as PT
 
-needs_ref = pytest.mark.skipif(not os.path.isdir("/root/reference/code/xmap"),
-                               reason="reference tree not mounted")
-
-_SCRIPT = textwrap.dedent("""
-    import sys, json
-    sys.path.insert(0, %(root)r)
-    from xmap_b200 import synth
-    from xmap_b200.core import (BaselinerClean, BaselinerSplit, baseliner_clean_data_pipeline,
-                                baseliner_split_data_pipeline)
-    sr = synth.make_ratings(400, 60, 9000, overlap=0.3, seed=4)
-    paths = []
-    for d, nm in ((0, "book"), (1, "movie")):
-        lines = synth.to_text_lines(sr, d)
-        # duplicates with other timestamps / out-of-period years exercise the filters
-        extra = [l.rsplit("\\t", 1)[0] + "\\t" + str(int(l.rsplit("\\t", 1)[1]) + k * 40000000)
-                 for k, l in enumerate(lines[:200])]
-        p = %(tmp)r + "/" + nm + ".txt"
-        open(p, "w").write("\\n".join(lines + extra) + "\\n")
-        paths.append(p)
-    def run(mods, sc):
-        cs = mods["BaselinerClean"](5, 150, 2012, 2013, "S:"); ct = mods["BaselinerClean"](5, 150, 2012, 2013, "T:")
-        sp = mods["BaselinerSplit"](0, 0.2, 0.8, 666666)
-        out = {}
-        for dbg in (True, False):
-            s = mods["clean"](sc, cs, paths[0], dbg, 30); t = mods["clean"](sc, ct, paths[1], dbg, 30)
-            tr, te = mods["split"](sc, sp, s, t)
-            norm = lambda rdd: sorted((u, sorted((i, r, str(x)) for i, r, x in l)) for u, l in rdd.collect())
-            out[str(dbg)] = [norm(s), norm(t), norm(tr), norm(te)]
-        return out
-    mine = run(dict(BaselinerClean=BaselinerClean, BaselinerSplit=BaselinerSplit,
-                    clean=baseliner_clean_data_pipeline, split=baseliner_split_data_pipeline), None)
-    from oracle import harness as H
-    R = H.load_reference()
-    ref = run(dict(BaselinerClean=R["BaselinerClean"], BaselinerSplit=R["BaselinerSplit"],
-                   clean=R["assist"].baseliner_clean_data_pipeline,
-                   split=R["assist"].baseliner_split_data_pipeline), R["sc"])
-    for dbg in ("True", "False"):
-        for k, (a, b) in enumerate(zip(mine[dbg], ref[dbg])):
-            assert a == b, (dbg, k, len(a), len(b))
-        assert len(mine[dbg][2]) > 0 and len(mine[dbg][3]) > 0
-    print("ok")
-""")
+_REFERENCE_RUN = """
+import sys
+sys.path.insert(0, %(root)r)
+from oracle import make_golden_cleansplit as CS
+paths = CS.write_inputs(%(tmp)r)
+mine, ref = CS.run_host(paths), CS.run_reference(paths)
+for mode in mine:
+    for stage, a, b in zip(CS.STAGES, mine[mode], ref[mode]):
+        assert a == b, (mode, stage, len(a), len(b))
+    assert len(mine[mode][2]) > 0 and len(mine[mode][3]) > 0
+print("ok")
+"""
 
 
-@needs_ref
+@pytest.mark.skipif(not H.reference_available(), reason="needs the original X-MAP source (XMAP_REFERENCE_CODE)")
 def test_clean_and_split_match_reference(tmp_path):
-    code = _SCRIPT % dict(root=PT.ROOT, tmp=str(tmp_path))
+    """Both modes (debug sample and full data), in the local time zone: the four record sets of the clean and split
+    stages equal those of the unmodified reference on the same input."""
+    code = _REFERENCE_RUN % dict(root=PT.ROOT, tmp=str(tmp_path))
     r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=600, cwd=PT.ROOT)
     assert r.returncode == 0 and "ok" in r.stdout, (r.stdout[-2000:], r.stderr[-3000:])
+
+
+def test_clean_and_split_match_stored_records(tmp_path):
+    """Both modes, under TZ=UTC: the four record sets equal those stored in tests/golden/cleansplit.npz.  The file says
+    where its records come from; the committed one is a regression snapshot of the host classes (the original source
+    was not available when it was recorded), so this pins the stages to their earlier output, not to the reference:
+    test_clean_and_split_match_reference does that where the source is available."""
+    want, digest, source = CS.load()
+    assert source in CS.SOURCES, source
+    with CS.utc():
+        paths = CS.write_inputs(str(tmp_path))
+        assert CS.inputs_digest(paths) == digest, "the synthetic input is not the one the stored records were made from"
+        mine = CS.run_host(paths)
+    for mode in want:
+        for stage, a, b in zip(CS.STAGES, mine[mode], want[mode]):
+            assert a == b, (mode, stage, source, len(a), len(b))
+        assert len(mine[mode][2]) > 0 and len(mine[mode][3]) > 0
 
 
 def test_local_rdd_surface():

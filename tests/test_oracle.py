@@ -1,10 +1,9 @@
 """CPU: the oracle restatement (oracle/restate.py) is pinned against the golden vectors that
 the UNMODIFIED reference produced (oracle/make_golden.py), stage by stage."""
-import os
-
 import numpy as np
 import pytest
 
+from oracle import harness as H
 from oracle import restate as RS
 from tests import parity as PT
 
@@ -61,9 +60,9 @@ def test_restatement_selection_extension_generation_vs_reference(name):
     assert np.array_equal(rows4[ok], g["nonpriv_rows"]) and np.array_equal(chn[ok], g["nonpriv_chosen"])
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/code/xmap"), reason="reference tree not mounted")
+@pytest.mark.skipif(not H.reference_available(), reason="needs the original X-MAP source (XMAP_REFERENCE_CODE)")
 def test_harness_runs_the_reference_and_agrees_with_golden():
-    """Where /root/reference exists, re-run the reference itself on the smallest case."""
+    """Where the original X-MAP source is available, re-run the reference itself on the smallest case."""
     import subprocess, sys
     code = ("import numpy as np;from oracle import make_golden as M;"
             "o=M.build_case('adj_all_bridge');g=np.load('tests/golden/adj_all_bridge.npz');"
@@ -112,8 +111,10 @@ def test_restatement_vs_reference_mid_size():
     assert len(g["user"]) > 85000 and len(g["sim_i"]) > 300000
     assert np.array_equal(P["i"], g["sim_i"]) and np.array_equal(P["j"], g["sim_j"])
     assert np.array_equal(P["mutu"], g["sim_mutu"]) and np.array_equal(P["label"], g["sim_label"])
-    assert np.array_equal(P["frac"].astype(np.float32), g["sim_frac"])      # stored as its float32 image
-    np.testing.assert_allclose(P["sim"], g["sim_val"], rtol=1e-10)
+    known = np.isfinite(g["sim_val"])          # similarity and frac are stored for a fixed sample of the pairs
+    assert known.sum() > 70000
+    assert np.array_equal(P["frac"][known].astype(np.float32), g["sim_frac"][known])      # stored as its float32 image
+    np.testing.assert_allclose(P["sim"][known], g["sim_val"][known], rtol=1e-10)
     assert np.array_equal(P["stats"]["mu"], g["user_avg"])
     knn = RS.select_knn(P, nI, int(g["k"]), meta["dom_code"], meta["contains"])
     assert np.array_equal(knn["bb"], g["bb"]) and np.array_equal(knn["valid_nb"], g["valid_nb"])
