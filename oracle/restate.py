@@ -355,10 +355,12 @@ def choose(rows, cands, mode, uniforms=None, epsilon=0.6, mapping_range=1, gs=2)
 
 
 def invert_mapping(rows, chosen, n_items):
-    """assist.py:215 with rows consumed in ascending target index: largest wins."""
+    """assist.py:215 with rows consumed in ascending target index: largest wins.  A row without a
+    candidate (chosen = -1, the device's marker) maps nothing."""
     mp = np.full(n_items, -1, dtype=np.int64)
     for t, s in zip(rows, chosen):
-        mp[s] = t
+        if s >= 0:
+            mp[s] = t
     return mp
 
 
@@ -479,13 +481,16 @@ def bound_rating(x):
 
 
 def recommender_predict(p_user, p_item, p_rating, p_ts, nb_ptr, nb_idx, nb_sim, item_avg,
-                        t_user, t_item, t_rating, alpha=0.03):
+                        t_user, t_item, t_rating, alpha=0.03, raw=False):
     """Item-based prediction of every test (user, item) pair: (no-decay, decay) predictions (-1 where the item
-    has no neighbour list) and the two MAEs (recommenderPrediction.py:26-139).  Profile records in list order."""
+    has no neighbour list) and the two MAEs (recommenderPrediction.py:26-139).  Profile records in list order.
+    raw=True also returns the no-decay and decay values before bound_rating (NaN where the item has no
+    neighbour list), so a caller can tell a value at a rounding boundary from a real mismatch."""
     by_ui = {}
     for q, (u, i) in enumerate(zip(p_user, p_item)):
         by_ui.setdefault((int(u), int(i)), []).append(q)          # profile order within (user, item)
     out0, out1 = np.full(len(t_user), -1.0), np.full(len(t_user), -1.0)
+    raw0, raw1 = np.full(len(t_user), np.nan), np.full(len(t_user), np.nan)
     for q, (u, it) in enumerate(zip(t_user, t_item)):
         a, b = nb_ptr[it], nb_ptr[it + 1]
         if b == a:
@@ -509,9 +514,12 @@ def recommender_predict(p_user, p_item, p_rating, p_ts, nb_ptr, nb_idx, nb_sim, 
         else:
             nd = dc = avg
         out0[q], out1[q] = bound_rating(nd), bound_rating(dc)
+        raw0[q], raw1[q] = nd, dc
     ok = out0 >= 0
     mae0 = float(np.abs(t_rating[ok] - out0[ok]).sum() / ok.sum()) if ok.any() else float("nan")
     mae1 = float(np.abs(t_rating[ok] - out1[ok]).sum() / ok.sum()) if ok.any() else float("nan")
+    if raw:
+        return out0, out1, mae0, mae1, raw0, raw1
     return out0, out1, mae0, mae1
 
 

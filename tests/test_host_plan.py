@@ -136,3 +136,21 @@ def test_engine_host_helpers():
     assert tuple(rec.shape) == (5000, 2) and tuple(rec_n.shape) == (5000,) and rec_n.dtype == torch.int32
     rec.fill_(-1); rec_n.fill_(7)
     assert int((rec != -1).sum()) == 0 and int((rec_n != 7).sum()) == 0
+
+
+def test_predict_rejects_out_of_range_test_pairs_on_the_host():
+    """recsim.predict checks test_user against [0, n_users) and test_item against the neighbour tables before it
+    launches anything (the kernel indexes the profile and the tables without a bound check).  Every call here
+    raises, so the CPU tensors never reach the kernel."""
+    import torch
+    from xmap_b200 import recsim
+    nI, K = 5, 3
+    R = recsim.RecSim(torch.zeros(1, dtype=torch.int32), torch.zeros(1, dtype=torch.int32), torch.ones(1, dtype=torch.int64),
+                      torch.zeros(1, dtype=torch.float64), torch.zeros(1, dtype=torch.float64),
+                      torch.zeros((nI, 3), dtype=torch.float64), 0)
+    nb = recsim.Neighbors(torch.full((nI, K), -1, dtype=torch.int32), torch.zeros((nI, K), dtype=torch.float64),
+                          torch.zeros(nI, dtype=torch.int32))
+    prof = ([0, 1], [2, 3], [4.0, 3.5], [10, 20], 2, R, nb)
+    for tu, ti in (([0, 2], [0, 0]), ([-1], [0]), ([0], [nI]), ([1, 0], [0, -1]), ([2 ** 32], [0]), ([0], [0, 1])):
+        with pytest.raises(ValueError):
+            recsim.predict(*prof, tu, ti)

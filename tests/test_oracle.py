@@ -162,3 +162,61 @@ def test_restatement_private_neighbors_vs_reference(name):
     # the draw is not the arg-max: the mechanism really samples
     nb = RS.recommender_neighbors(P, nI, 1)
     assert 0 < int((ch != nb[1]).sum())
+
+
+def test_restatement_alterego_merge_rule_hand_computed():
+    """generator.py:140-157 on a merge (SURVEY.md:394, :577; DESIGN.md 3.4): the ratings a user gave to several
+    sources mapped onto one target become ONE record with their mean and the time of the smallest source item --
+    not the earliest time, and not the first record in input order.  A real "T:" rating of the same (user, target)
+    is kept next to it.  Expected values written out by hand."""
+    #        user  item  rating  ts      items: 1 = s1, 2 = s2 (both -> 3), 3 = T (a "T:" item)
+    recs = [(0, 2, 2.5, 100),
+            (0, 1, 1.25, 300),
+            (0, 3, 4.0, 50),
+            (1, 2, 3.5, 70)]
+    user, item, rating, ts = (np.array(c) for c in zip(*recs))
+    mapping = np.array([-1, 3, 3, -1])
+    has_T = np.array([False, False, False, True])
+    ae = RS.build_alterego(user, item, rating.astype(np.float32), ts, mapping, has_T)
+    assert ae["user"].tolist() == [0, 0, 1]
+    assert ae["item"].tolist() == [3, 3, 3]
+    assert ae["rating"].tolist() == [4.0, 1.875, 3.5]
+    assert ae["ts"].tolist() == [50, 300, 70]
+    assert ae["synthetic"].tolist() == [False, True, True]
+
+
+def test_restatement_invert_mapping_largest_target_wins_and_skips_empty_rows():
+    """assist.py:215: rows in ascending target order, so the largest target choosing a source wins; a row
+    without a candidate (chosen = -1) maps nothing."""
+    mp = RS.invert_mapping(np.array([2, 5, 7, 9]), np.array([1, 1, -1, 1]), 10)
+    assert mp.tolist() == [-1, 9, -1, -1, -1, -1, -1, -1, -1, -1]
+    mp = RS.invert_mapping(np.array([2, 5, 7]), np.array([4, 1, -1]), 6)
+    assert mp.tolist() == [-1, 5, -1, -1, 2, -1]
+
+
+def test_restatement_prediction_tied_times_share_a_rank():
+    """recommenderPrediction.py:36-49: entry times [5, 5, 9] rank [1, 1, 2], cur = 3, so the decay weights are
+    e^{-2 alpha}, e^{-2 alpha}, e^{-alpha}.  Also: no neighbour list -> -1, no matching record -> the item
+    average, and raw=True returns the values before bounding while leaving the default output as it was."""
+    import math
+    a = 0.5
+    # profile of user 0 in list order: item 3 at t = 9, item 1 at t = 5, item 2 at t = 5; user 1 rates item 4 only
+    p_user, p_item = np.array([0, 0, 0, 1]), np.array([3, 1, 2, 4])
+    p_rating, p_ts = np.array([3.0, 4.0, 2.0, 1.0]), np.array([9, 5, 5, 7])
+    nb_ptr = np.array([0, 3, 3, 3, 3, 3])                  # item 0: neighbours 1, 2, 3; no other item has a list
+    nb_idx, nb_sim = np.array([1, 2, 3]), np.array([0.5, -0.25, 1.0])
+    avg = np.array([3.0, 3.5, 2.5, 2.0, 1.0])
+    t_user, t_item, t_rating = np.array([0, 1, 0]), np.array([0, 0, 2]), np.array([4.0, 3.0, 2.0])
+    # entries (sim * (r - avg_n), |sim|): (0.25, 0.5) t=5, (0.125, 0.25) t=5, (1.0, 1.0) t=9
+    nd = 3.0 + (0.25 + 0.125 + 1.0) / (0.5 + 0.25 + 1.0)
+    w5, w9 = math.exp(-2 * a), math.exp(-a)
+    dc = 3.0 + (0.25 * w5 + 0.125 * w5 + 1.0 * w9) / (0.5 * w5 + 0.25 * w5 + 1.0 * w9)
+    assert abs(dc - 3.8436667) < 1e-7                      # distinct ranks 1, 2, 3 would give 3.8743713
+    args = (p_user, p_item, p_rating, p_ts, nb_ptr, nb_idx, nb_sim, avg, t_user, t_item, t_rating, a)
+    p0, p1, m0, m1, r0, r1 = RS.recommender_predict(*args, raw=True)
+    assert r0[0] == nd and abs(r1[0] - dc) <= 1e-15 * dc
+    assert r0[1] == r1[1] == 3.0 and np.isnan(r0[2]) and np.isnan(r1[2])
+    assert p0.tolist() == [4.0, 3.0, -1.0] and p1.tolist() == [4.0, 3.0, -1.0]
+    assert m0 == m1 == 0.0
+    q0, q1, n0, n1 = RS.recommender_predict(*args)
+    assert np.array_equal(q0, p0) and np.array_equal(q1, p1) and (n0, n1) == (m0, m1)

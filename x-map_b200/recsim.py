@@ -147,9 +147,20 @@ def predict(user, item, rating, ts, n_users, rs, nb, test_user, test_item, test_
     p_item = torch.as_tensor(item, dtype=torch.int32).to(dev)[ou].contiguous()
     p_rating = torch.as_tensor(rating, dtype=torch.float64).to(dev)[ou].contiguous()
     p_ts = torch.as_tensor(ts, dtype=torch.int64).to(dev)[ou].contiguous()
-    tu = torch.as_tensor(test_user, dtype=torch.int32).to(dev).contiguous()
-    ti = torch.as_tensor(test_item, dtype=torch.int32).to(dev).contiguous()
+    # checked in int64 before the narrowing copy: the kernel indexes the profile by user and the neighbour
+    # tables by item without a bound check
+    tu = torch.as_tensor(test_user, dtype=torch.int64).flatten()
+    ti = torch.as_tensor(test_item, dtype=torch.int64).flatten()
     n_test = int(tu.numel())
+    if int(ti.numel()) != n_test:
+        raise ValueError("test_user and test_item differ in length (%d, %d)" % (n_test, int(ti.numel())))
+    n_tab = int(nb.idx.shape[0])
+    if n_test and (int(tu.min()) < 0 or int(tu.max()) >= n_users):
+        raise ValueError("test_user outside [0, %d)" % n_users)
+    if n_test and (int(ti.min()) < 0 or int(ti.max()) >= n_tab):
+        raise ValueError("test_item outside [0, %d)" % n_tab)
+    tu = tu.to(device=dev, dtype=torch.int32).contiguous()
+    ti = ti.to(device=dev, dtype=torch.int32).contiguous()
     p0 = torch.empty(n_test, dtype=torch.float64, device=dev)
     p1 = torch.empty(n_test, dtype=torch.float64, device=dev)
     err = torch.zeros(1, dtype=torch.int32, device=dev)
