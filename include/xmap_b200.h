@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define XMAP_B200_ABI_VERSION 6
+#define XMAP_B200_ABI_VERSION 7
 #define XMAP_KMAX 64                 /* largest supported top-k (extend_among_topk) */
 #define XMAP_METHOD_ADJUST_COSINE 0  /* baselinerSim.py:144-174 */
 #define XMAP_METHOD_COSINE 1         /* baselinerSim.py:115-142 */
@@ -46,9 +46,9 @@ const char *xmap_last_error(void);
  * In : nnz deduplicated (user, item, rating) triples in any order.
  * Out: CSR by user (entries ascending by item) and CSC by item (entries
  *      ascending by user).  Entry formats (8 bytes each):
- *        csr_ent[k] = { item | cls(item)<<24 | ge_avg<<29 , float bits of rating }
- *        csc_ent[k] = { user | ge_avg<<31                  , float bits of rating }
- *      cls(item) = ceil(log2(count(item))); ge_avg = (rating >= item average),
+ *        csr_ent[k] = { item | ge_avg<<29 , float bits of rating }
+ *        csc_ent[k] = { user | ge_avg<<31 , float bits of rating }
+ *      ge_avg = (rating >= item average),
  *      the comparison retrieve_path_info makes (baselinerSim.py:106-111).
  *      csr_src[k] = index of the input triple stored at CSR position k.
  *      user_mu[u] = mean rating of u (baselinerSim.py:30).
@@ -77,23 +77,26 @@ int xmap_row_work(const int32_t *csr_ptr, const int32_t *csc_ptr, const uint64_t
  * the less popular item, so row i only needs, for each of its raters u, the part
  * of u's ratings that lies on more popular items.  With the user's ratings
  * sorted by ord that part is a suffix:
- *   tcsr_ent[k]  = { ord(item) | cls(item)<<24 | ge_avg<<29 , float bits of rating }
- *                  same extents as csr_ptr, entries ascending by ord;
+ *   tcsr_ent[k]  = { ord(item) | (x & 31)<<24 | ge_avg<<29 | (x >> 5)<<30 , float bits of rating }
+ *                  same extents as csr_ptr, entries ascending by ord; x = x(item) below;
  *   csc_aux[e]   = 16 bytes { uint32 pos, uint32 len, double mu }: CSC entry e = (i, u) sits at
  *                  tcsr position pos, the len entries after it are u's ratings of items more
  *                  popular than i, and mu = user_mu[u] (0 for the cosine method);
  *   tri_work[i]  = sum of len over the raters of i = products row i evaluates
  *                  (sum over i = W / 2);
- *   ostat[o]     = 16 bytes per ord o: { double den; uint32 item; uint32 prefix<<8 | cls }
+ *   ostat[o]     = 16 bytes per ord o: { double den; uint32 item; uint32 prefix<<8 | x }
  *                  den = norm2 (cosine) or adjusted norm2 (adjust_cosine) of the item,
- *                  baselinerSim.py:131-132,164-165.
+ *                  baselinerSim.py:131-132,164-165;
+ *                  x = clamp(E - e_base, 0, 127) with 2^(E-1) <= den < 2^E, 0 when den == 0:
+ *                  the item's exponent, which scales the fixed-point inner products of its pairs.
+ *                  e_base = max E - 127 over the items with den > 0 keeps every x in the field.
  * workspace >= xmap_tri_workspace_bytes(nnz). */
 size_t xmap_tri_workspace_bytes(int64_t nnz);
 int xmap_build_tri_layout(const int32_t *csr_ptr, const uint64_t *csr_ent,
                           const int32_t *csc_ptr, const uint64_t *csc_ent,
                           const double *user_mu, const double *item_stats, const int32_t *prefix_code,
                           const int32_t *ord, int32_t n_users, int32_t n_items, int64_t nnz, int32_t method,
-                          uint64_t *tcsr_ent, void *csc_aux, void *ostat, int64_t *tri_work,
+                          int32_t e_base, uint64_t *tcsr_ent, void *csc_aux, void *ostat, int64_t *tri_work,
                           void *workspace, size_t workspace_bytes, void *stream);
 
 /* ---------------------------------------------------------------------------
@@ -142,7 +145,8 @@ typedef struct xmap_sim_args {
     const uint8_t *dom_code;       /* iid[-2:] -- extender.py:29     */
     const uint8_t *contains;       /* bit d: label d is a substring of iid -- extender.py:32,34 */
     int32_t n_items; int32_t method; int32_t num_atleast; int32_t k;
-    int32_t r2_bits;               /* ceil(log2(max |product|)) for the fixed-point scale */
+    int32_t r2_bits;               /* 2 * e_base of xmap_build_tri_layout: the inner product of items i, j is
+                                      summed in units of 2^-(62 - r2_bits - x_i - x_j) */
     int32_t count_only;            /* 1: sizing pass -- bump the list cursors, write no record (rec_ptr unused) */
     /* neighbour-record lists */
     const int64_t *rec_ptr;        /* [n_items + 1] list extents (capacity) */

@@ -96,13 +96,12 @@ def multi_domain_cases(n_users, n_items, n_draws, overlap, seed, n_domains=3):
             for d in range(n_domains - 1)]
 
 
-def run_gpu_sim(user, item, rating, n_users, n_items, meta, method, num_atleast, k, emit=True,
-                max_smem_cells=None):
+def run_gpu_sim(user, item, rating, n_users, n_items, meta, method, num_atleast, k, emit=True, **engine_kw):
+    """engine_kw: SimEngine options (max_smem_cells, rec_budget)."""
     import torch
     from xmap_b200 import engine as E
     lay = E.build_layout(user, item, rating, n_users, n_items)
-    kw = {} if max_smem_cells is None else dict(max_smem_cells=max_smem_cells)
-    eng = E.SimEngine(lay, to_device_meta(meta), method, num_atleast, k, **kw)
+    eng = E.SimEngine(lay, to_device_meta(meta), method, num_atleast, k, **engine_kw)
     tabs = eng.run()
     pairs = eng.emit_pairs() if emit else None
     torch.cuda.synchronize()
@@ -233,11 +232,10 @@ def restate_lists(knn, pairs):
     return out
 
 
-def check_sim_against_restatement(case, method, num_atleast, k, max_smem_cells=None):
+def check_sim_against_restatement(case, method, num_atleast, k, **engine_kw):
     from oracle import restate as RS
     lay, eng, tabs, pairs = run_gpu_sim(case["user"], case["item"], case["rating"], case["n_users"],
-                                        case["n_items"], case["meta"], method, num_atleast, k,
-                                        max_smem_cells=max_smem_cells)
+                                        case["n_items"], case["meta"], method, num_atleast, k, **engine_kw)
     P = RS.sim_pairs(case["user"], case["item"], case["rating"], case["n_users"], case["n_items"],
                      case["meta"]["prefix_code"], method, num_atleast)
     compare_layout(lay, P["stats"])

@@ -116,14 +116,12 @@ def test_no_cpu_fallback_without_gpu():
 
 
 def test_engine_host_helpers():
-    """Device-agnostic helpers of the engine: popularity rank, fixed-point head-room, threads per table,
-    and the hand-over pool of record buffers."""
+    """Device-agnostic helpers of the engine: popularity rank, threads per table and the hand-over pool of
+    record buffers."""
     import torch
     from xmap_b200 import engine as E
     cnt = torch.tensor([3., 1., 3., 7., 1.], dtype=torch.float64)
     assert E.popularity_order(cnt).tolist() == [2, 0, 3, 4, 1]          # ascending count, ties by index
-    assert E.r2_bits_for("adjust_cosine", 1.0, 5.0) == 5 and E.r2_bits_for("cosine", 0.5, 5.0) == 6
-    assert E.r2_bits_for("cosine", 0.0, 0.0) == 0
     assert [E._threads_for_cells(c) for c in (32, 256, 512, 1024, 1536, 4096, 12288)] == [32, 32, 64, 128, 192, 512, 512]
     E._REC_POOL.pop("cpu", None)
     a = torch.empty(E._rec_words(100), dtype=torch.int64); b = torch.empty(E._rec_words(1000), dtype=torch.int64)
@@ -154,3 +152,27 @@ def test_predict_rejects_out_of_range_test_pairs_on_the_host():
     for tu, ti in (([0, 2], [0, 0]), ([-1], [0]), ([0], [nI]), ([1, 0], [0, -1]), ([2 ** 32], [0]), ([0], [0, 1])):
         with pytest.raises(ValueError):
             recsim.predict(*prof, tu, ti)
+
+
+def test_exponent_base():
+    """e_base of the fixed-point scale: max E - 127 over the items with a non-zero norm (2^(E-1) <= den < 2^E),
+    from the norm the method divides by; up to 16 octaves below the field are clamped, more raise."""
+    import torch
+    from xmap_b200 import engine as E
+
+    def stats(norm2, adj):                                        # item_stats columns: avg, norm2, adj_norm2, count
+        n = len(norm2)
+        return torch.tensor([[1.0] * n, norm2, adj, [2.0] * n], dtype=torch.float64).T.contiguous()
+
+    st = stats([5.0, 0.75, 0.0], [0.0, 4.0, 0.0])
+    assert E.exponent_base("cosine", st) == 3 - 127                # frexp(5) = 0.625 * 2^3
+    assert E.exponent_base("adjust_cosine", st) == 3 - 127          # 4 = 0.5 * 2^3; zero norms are ignored
+    assert E.exponent_base("adjust_cosine", stats([5.0, 1.0], [0.0, 0.0])) == 0      # every norm zero
+    assert E.exponent_base("cosine", stats([1.0, 0.5], [2.0 ** 40, 1.0])) == 1 - 127
+    assert E.exponent_base("adjust_cosine", stats([1.0, 0.5], [2.0 ** 40, 1.0])) == 41 - 127
+    assert E.exponent_base("cosine", stats([2.0 ** 100, 2.0 ** -27], [1.0, 1.0])) == 101 - 127    # spread 127: fits
+    assert E.exponent_base("cosine", stats([2.0 ** 100, 2.0 ** -43], [1.0, 1.0])) == 101 - 127    # clamped by 16
+    with pytest.raises(ValueError):
+        E.exponent_base("cosine", stats([2.0 ** 100, 2.0 ** -44], [1.0, 1.0]))
+    with pytest.raises(ValueError):
+        E.exponent_base("adjust_cosine", stats([1.0, 1.0], [2.0 ** -60, 2.0 ** 100]))

@@ -14,7 +14,7 @@ KMAX = 64
 XSIM_MAX_CELLS_LG = 13    # XMAP_XSIM_MAX_CELLS_LG
 METHODS = {"adjust_cosine": 0, "cosine": 1}
 SELECT_LONG = 8192            # XMAP_SELECT_LONG
-ABI_VERSION = 6
+ABI_VERSION = 7
 ROW_HDR_BYTES = 48          # XMAP_SIM_ROW_HDR_BYTES
 
 _p = C.c_void_p
@@ -59,7 +59,7 @@ _SIGS = {
     "xmap_row_work": (C.c_int, [_p, _p, _p, C.c_int32, _p, _p]),
     "xmap_tri_workspace_bytes": (C.c_size_t, [C.c_int64]),
     "xmap_build_tri_layout": (C.c_int, [_p, _p, _p, _p, _p, _p, _p, _p, C.c_int32, C.c_int32, C.c_int64, C.c_int32,
-                                        _p, _p, _p, _p, _p, C.c_size_t, _p]),
+                                        C.c_int32, _p, _p, _p, _p, _p, C.c_size_t, _p]),
     "xmap_sim_row_cells": (C.c_int64, [C.c_int64, C.c_int32]),
     "xmap_sim_accumulate": (C.c_int, [C.POINTER(SimArgs), _p, C.c_int32, C.c_int32, C.c_int32, _p, C.c_int32, _p]),
     "xmap_sim_row_headers": (C.c_int, [C.POINTER(SimArgs), _p, C.c_int32, _p, _p, _p, _p]),

@@ -29,19 +29,13 @@ inline int fail_msg(const char *msg) {
 
 // ---- entry formats (include/xmap_b200.h) ---------------------------------
 constexpr uint32_t ITEM_MASK = 0x00FFFFFFu;
-constexpr int CLS_SHIFT = 24;
 constexpr int GE_SHIFT = 29;
+constexpr int EXP_MAX = 127;          // tcsr entries: 7-bit item exponent in bits 24-28 (low 5) and 30-31 (high 2)
 
 __device__ __forceinline__ int ent_item(uint32_t w0) { return int(w0 & ITEM_MASK); }
-__device__ __forceinline__ int ent_cls(uint32_t w0) { return int((w0 >> CLS_SHIFT) & 31u); }
 __device__ __forceinline__ int ent_ge(uint32_t w0) { return int((w0 >> GE_SHIFT) & 1u); }
-
-__host__ __device__ __forceinline__ int ceil_log2_u32(uint32_t c) {
-    // smallest b with 2^b >= c ; c >= 1
-    int b = 0;
-    while ((1u << b) < c && b < 31) ++b;
-    return b;
-}
+__device__ __forceinline__ int ent_exp(uint32_t w0) { return int(((w0 >> 24) & 31u) | ((w0 >> 25) & 0x60u)); }
+__device__ __forceinline__ uint32_t exp_bits(uint32_t e) { return ((e & 31u) << 24) | ((e >> 5) << 30); }
 
 // 2^e as a double, e in [-1022, 1023]
 __device__ __forceinline__ double pow2d(int e) {

@@ -95,10 +95,8 @@ __global__ void pack_csr_kernel(const uint64_t *__restrict__ keys_u, const int32
     int32_t src = perm[k];
     float r = rating[src];
     double avg = stats[4 * (int64_t)item + 0];
-    uint32_t cnt = (uint32_t)stats[4 * (int64_t)item + 3];
-    uint32_t cls = (uint32_t)ceil_log2_u32(cnt);
     uint32_t ge = ((double)r >= avg) ? 1u : 0u;
-    uint32_t w0 = item | (cls << CLS_SHIFT) | (ge << GE_SHIFT);
+    uint32_t w0 = item | (ge << GE_SHIFT);
     csr_ent[k] = ((uint64_t)__float_as_uint(r) << 32) | w0;
     csr_src[k] = src;
 }
@@ -147,13 +145,13 @@ __global__ void row_work_kernel(const int32_t *__restrict__ csr_ptr, const int32
 struct __align__(16) OStat {
     double den;
     uint32_t item;
-    uint32_t prefix_cls;      // prefix << 8 | cls
+    uint32_t prefix_exp;      // prefix << 8 | item exponent (tri_ostat_kernel)
 };
 
-// key = user << 32 | ord(item), value = the CSR entry with the item replaced by its ord
+// key = user << 32 | ord(item), value = the CSR entry with the item replaced by its ord, plus the item's exponent
 __global__ void tri_keys_kernel(const int32_t *__restrict__ csr_ptr, const uint64_t *__restrict__ csr_ent,
-                                const int32_t *__restrict__ ord, int32_t n_users, int64_t nnz,
-                                uint64_t *__restrict__ keys, uint64_t *__restrict__ vals) {
+                                const int32_t *__restrict__ ord, const OStat *__restrict__ ostat, int32_t n_users,
+                                int64_t nnz, uint64_t *__restrict__ keys, uint64_t *__restrict__ vals) {
     int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (k >= nnz) return;
     int32_t lo = 0, hi = n_users;                       // largest u with csr_ptr[u] <= k
@@ -165,7 +163,8 @@ __global__ void tri_keys_kernel(const int32_t *__restrict__ csr_ptr, const uint6
     const uint32_t w0 = (uint32_t)e;
     const uint32_t o = (uint32_t)__ldg(ord + (w0 & ITEM_MASK));
     keys[k] = ((uint64_t)(uint32_t)lo << 32) | o;
-    vals[k] = (e & 0xFFFFFFFF00000000ull) | (uint64_t)((w0 & ~ITEM_MASK) | o);
+    const uint32_t ex = ostat[o].prefix_exp & 0xFFu;
+    vals[k] = (e & 0xFFFFFFFF00000000ull) | (uint64_t)((w0 & ~ITEM_MASK) | exp_bits(ex) | o);
 }
 
 // One thread per CSC entry (i, u): position of the entry in u's ord-sorted row, suffix length, and
@@ -209,8 +208,10 @@ __global__ void tri_aux_kernel(const int32_t *__restrict__ csr_ptr, const int32_
     }
 }
 
+// The item exponent: E with 2^(E-1) <= den < 2^E, stored as clamp(E - e_base, 0, EXP_MAX); 0 for den == 0
+// (every product of such an item is 0).
 __global__ void tri_ostat_kernel(const double *__restrict__ item_stats, const int32_t *__restrict__ prefix_code,
-                                 const int32_t *__restrict__ ord, int32_t n_items, int32_t method,
+                                 const int32_t *__restrict__ ord, int32_t n_items, int32_t method, int32_t e_base,
                                  OStat *__restrict__ ostat) {
     int32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n_items) return;
@@ -218,7 +219,12 @@ __global__ void tri_ostat_kernel(const double *__restrict__ item_stats, const in
     OStat o;
     o.den = (method == XMAP_METHOD_COSINE) ? s[1] : s[2];
     o.item = (uint32_t)i;
-    o.prefix_cls = ((uint32_t)prefix_code[i] << 8) | (uint32_t)ceil_log2_u32((uint32_t)s[3]);
+    int ex = 0;
+    if (o.den > 0.0) {
+        frexp(o.den, &ex);
+        ex = min(max(ex - e_base, 0), EXP_MAX);
+    }
+    o.prefix_exp = ((uint32_t)prefix_code[i] << 8) | (uint32_t)ex;
     ostat[ord[i]] = o;
 }
 
@@ -347,12 +353,12 @@ extern "C" int xmap_build_tri_layout(const int32_t *csr_ptr, const uint64_t *csr
                                      const int32_t *csc_ptr, const uint64_t *csc_ent,
                                      const double *user_mu, const double *item_stats, const int32_t *prefix_code,
                                      const int32_t *ord, int32_t n_users, int32_t n_items, int64_t nnz, int32_t method,
-                                     uint64_t *tcsr_ent, void *csc_aux, void *ostat, int64_t *tri_work,
+                                     int32_t e_base, uint64_t *tcsr_ent, void *csc_aux, void *ostat, int64_t *tri_work,
                                      void *workspace, size_t workspace_bytes, void *stream_) {
     cudaStream_t st = (cudaStream_t)stream_;
     const int T = 256;
     if (n_items > 0) {
-        tri_ostat_kernel<<<(n_items + T - 1) / T, T, 0, st>>>(item_stats, prefix_code, ord, n_items, method,
+        tri_ostat_kernel<<<(n_items + T - 1) / T, T, 0, st>>>(item_stats, prefix_code, ord, n_items, method, e_base,
                                                               reinterpret_cast<OStat *>(ostat));
         XMAP_LAUNCH_CHECK();
         XMAP_CUDA(cudaMemsetAsync(tri_work, 0, sizeof(int64_t) * (size_t)n_items, st));
@@ -365,7 +371,8 @@ extern "C" int xmap_build_tri_layout(const int32_t *csr_ptr, const uint64_t *csr
     uint64_t *keys_a = (uint64_t *)base, *keys_b = (uint64_t *)(base + seg), *vals_a = (uint64_t *)(base + 2 * seg);
     void *cub_ws = base + 3 * seg;
     const unsigned gN = (unsigned)((nnz + T - 1) / T);
-    tri_keys_kernel<<<gN, T, 0, st>>>(csr_ptr, csr_ent, ord, n_users, nnz, keys_a, vals_a);
+    tri_keys_kernel<<<gN, T, 0, st>>>(csr_ptr, csr_ent, ord, reinterpret_cast<const OStat *>(ostat), n_users, nnz,
+                                      keys_a, vals_a);
     XMAP_LAUNCH_CHECK();
     XMAP_CUDA(cub::DeviceRadixSort::SortPairs(cub_ws, cub_bytes, keys_a, keys_b, vals_a, tcsr_ent, nnz, 0,
                                               32 + bits_for(n_users), st));

@@ -18,9 +18,13 @@
 //
 // Numerics.  Per pair three exact integer accumulators: n_ij, the mutuality
 // count, and the inner product in 64-bit fixed point with 2^-q resolution,
-// q = 62 - r2_bits - min(cls_i, cls_j), cls = ceil(log2(item count)).
-// n_ij <= min(count_i, count_j) <= 2^cls, so the sum cannot overflow, and
-// because integer addition is associative the result does not depend on the
+// q = 62 - E_i - E_j, where 2^(E-1) <= den < 2^E for the item's norm den
+// (entries and ostat carry E - e_base in 7 bits; r2_bits = 2 e_base).  By
+// Cauchy-Schwarz every product and every partial co-rater sum is at most
+// den_i den_j < 2^(E_i + E_j), so the final sum is below 2^62 + n and fits
+// (the lo/hi words may wrap on the way; only the final sum matters), and the
+// rounding error of the cosine is at most n 2^-61 whatever the rating scale.
+// Because integer addition is associative the result does not depend on the
 // order products arrive in: any split of a row over lanes, warps or GPUs gives
 // bit-identical output.  The 64-bit sum is kept as two 32-bit shared-memory
 // words (native 32-bit atomics; the carry out of the low word is recovered from
@@ -37,7 +41,7 @@ constexpr int KMAX = XMAP_KMAX;
 struct __align__(16) OStat {
     double den;
     uint32_t item;
-    uint32_t prefix_cls;      // prefix << 8 | cls
+    uint32_t prefix_exp;      // prefix << 8 | item exponent
 };
 
 // 16-byte accumulator cell.
@@ -68,7 +72,7 @@ struct __align__(16) RowHdr {
     long long work;               // tri_work[row]
     double den;                   // ostat[oi].den
     long long rec_base;           // rec_ptr[row]
-    unsigned prefix_cls;          // ostat[oi].prefix_cls
+    unsigned prefix_exp;          // ostat[oi].prefix_exp
     int rec_cap;                  // rec_ptr[row + 1] - rec_ptr[row]
 };
 static_assert(sizeof(RowHdr) == 48, "RowHdr layout");
@@ -81,7 +85,7 @@ __device__ __forceinline__ RowHdr load_hdr(const RowHdr *p) {
     h.work = (long long)(((unsigned long long)b.y << 32) | b.x);
     h.den = __hiloint2double((int)b.w, (int)b.z);
     h.rec_base = (long long)(((unsigned long long)c.y << 32) | c.x);
-    h.prefix_cls = c.z; h.rec_cap = (int)c.w;
+    h.prefix_exp = c.z; h.rec_cap = (int)c.w;
     return h;
 }
 
@@ -98,7 +102,7 @@ __global__ void row_headers_kernel(xmap_sim_args a, const int32_t *__restrict__ 
     h.hi = seg_hi ? seg_hi[r] : a.csc_ptr[row + 1];
     h.work = a.tri_work[row];
     const OStat si = ostat[h.oi];
-    h.den = si.den; h.prefix_cls = si.prefix_cls;
+    h.den = si.den; h.prefix_exp = si.prefix_exp;
     h.rec_base = a.rec_ptr[row];
     h.rec_cap = (int)(a.rec_ptr[row + 1] - a.rec_ptr[row]);
     out[r] = h;
@@ -162,8 +166,8 @@ __device__ void tri_row(const xmap_sim_args &a, Cell *__restrict__ T, IDX *__res
 
     const RowHdr hd = load_hdr(hdr_p);
     const int row = hd.row, oi = hd.oi;
-    const int cls_i = int(hd.prefix_cls & 0xFFu);
-    const unsigned prefix_i = hd.prefix_cls >> 8;
+    const int e_i = int(hd.prefix_exp & 0xFFu);
+    const unsigned prefix_i = hd.prefix_exp >> 8;
     const int lo = hd.lo, hi = hd.hi;
     const long long work = hd.work;
     const int rtop = a.n_items - 1 - oi;                   // items more popular than `row`
@@ -181,7 +185,7 @@ __device__ void tri_row(const xmap_sim_args &a, Cell *__restrict__ T, IDX *__res
     group_sync<CTA_ROW>();
 
     // ---- accumulate: batches of 32 raters per warp, products flattened over the lanes ----------
-    const int qbase = 62 - a.r2_bits;
+    const int qbase = 62 - a.r2_bits;                      // 62 - 2 e_base
     const int top_ord = a.n_items - 1;
     // Many raters: one batch per warp.  Few raters (fewer batches than warps): every warp walks every
     // batch and takes every gwarps-th chunk of 32 products, so the whole group stays busy.
@@ -228,7 +232,7 @@ __device__ void tri_row(const xmap_sim_args &a, Cell *__restrict__ T, IDX *__res
                 const int oj = ent_item(en[u].x);
                 const double cj = (double)__uint_as_float(en[u].y) - mu_l[u];
                 const double p = __dmul_rn(ci_l[u], cj);
-                const int q = qbase - min(cls_i, ent_cls(en[u].x));
+                const int q = qbase - (e_i + ent_exp(en[u].x));
                 const long long fx = __double2ll_rn(p * pow2d(q));
                 const unsigned agree = ((unsigned)ent_ge(en[u].x) == (st_l[u] >> 31)) ? 1u : 0u;
                 int slot;
@@ -352,7 +356,7 @@ __device__ void tri_row(const xmap_sim_args &a, Cell *__restrict__ T, IDX *__res
         for (int u = 0; u < EU; ++u) {
             if (sidx[u] < 0) continue;
             uint4 out = make_uint4(0u, 0u, 0u, 0u);
-            const int q = qbase - min(cls_i, int(sj[u].prefix_cls & 0xFFu));
+            const int q = qbase - (e_i + int(sj[u].prefix_exp & 0xFFu));
             const long long fx = (long long)(((unsigned long long)cv[u].w << 32) | (unsigned long long)cv[u].z);
             if (fx == 0 || mutu[u] == 0u) { T4[sidx[u]] = out; continue; }     // sim == 0 or mutu == 0: filtered
             const double inner = (double)fx * pow2d(-q);
@@ -365,7 +369,7 @@ __device__ void tri_row(const xmap_sim_args &a, Cell *__restrict__ T, IDX *__res
                 const unsigned long long sb = (unsigned long long)__double_as_longlong(sim);
                 out = direct ? make_uint4(mutu[u], n[u], (unsigned)sb, (unsigned)(sb >> 32))
                              : make_uint4(sj[u].item, (n[u] << 16) | mutu[u], (unsigned)sb, (unsigned)(sb >> 32));
-                if ((sj[u].prefix_cls >> 8) != prefix_i) { a.bb[row] = 1; a.bb[sj[u].item] = 1; }
+                if ((sj[u].prefix_exp >> 8) != prefix_i) { a.bb[row] = 1; a.bb[sj[u].item] = 1; }
             }
             T4[sidx[u]] = out;
         }

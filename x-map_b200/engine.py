@@ -7,7 +7,6 @@ around the kernels.  The reference-shaped facades in core/ and utils/assist.py
 sit on top of this module.  No CPU fallback exists: without a GPU and the built
 extension these functions raise.
 """
-import math
 import os
 from dataclasses import dataclass, field
 
@@ -55,8 +54,6 @@ class Layout:
     user_mu: torch.Tensor
     item_stats: torch.Tensor      # [n_items, 4] = (avg, norm2, adj_norm2, count)
     row_work: torch.Tensor        # int64 [n_items]
-    r_min: float
-    r_max: float
 
 
 def build_layout(user, item, rating, n_users, n_items, device="cuda"):
@@ -84,25 +81,30 @@ def build_layout(user, item, rating, n_users, n_items, device="cuda"):
     row_work = torch.empty(n_items, dtype=torch.int64, device=device)
     N.check(L.xmap_row_work(N.ptr(csr_ptr), N.ptr(csc_ptr), N.ptr(csc_ent), n_items,
                             N.ptr(row_work), _stream_ptr()), "xmap_row_work")
-    if nnz:
-        r_min, r_max = float(rating.min()), float(rating.max())
-    else:
-        r_min = r_max = 0.0
     del ws
     return Layout(n_users, n_items, nnz, csr_ptr, csr_ent, csr_src, csc_ptr, csc_ent,
-                  user_mu, item_stats, row_work, r_min, r_max)
+                  user_mu, item_stats, row_work)
 
 
-def r2_bits_for(method, r_min, r_max):
-    """ceil(log2(max |product|)) + 1 guard bit for the fixed-point inner product."""
-    if method == "adjust_cosine":
-        span = r_max - r_min            # |r - mean_u| <= span
-    else:
-        span = max(abs(r_min), abs(r_max))
-    r2 = span * span
-    if r2 <= 0:
+EXP_FIELD_MAX = 127           # largest item exponent the 7-bit field of the triangular entries holds
+EXP_CLAMP_MAX = 16            # octaves an item exponent may be raised to fit the field before the input is refused
+
+
+def exponent_base(method, item_stats):
+    """e_base of the item exponents (xmap_build_tri_layout): with 2^(E-1) <= den < 2^E for the norm den of
+    every item with den > 0, e_base = max E - 127, and the kernels scale the inner product of items i, j by
+    2^(62 - E_i - E_j).  An item whose E lies below e_base is raised to it, which costs its pairs that many
+    bits; more than EXP_CLAMP_MAX of them raises ValueError."""
+    den = item_stats[:, 1 if method == "cosine" else 2]
+    den = den[den > 0]
+    if den.numel() == 0:
         return 0
-    return int(math.ceil(math.log2(r2))) + 1
+    e = torch.frexp(den).exponent
+    lo, hi = int(e.min()), int(e.max())
+    if hi - lo > EXP_FIELD_MAX + EXP_CLAMP_MAX:
+        raise ValueError("item norms span 2^%d (from 2^%d to 2^%d): more than the similarity stage's fixed-point "
+                         "inner product resolves (2^%d)" % (hi - lo, lo - 1, hi, EXP_FIELD_MAX + EXP_CLAMP_MAX))
+    return hi - EXP_FIELD_MAX
 
 
 @dataclass
@@ -192,7 +194,7 @@ class SimEngine:
         self.lay, self.meta = layout, meta
         self.method, self.num_atleast, self.k = method, int(num_atleast), int(k)
         self.device = layout.csr_ptr.device
-        self.r2_bits = r2_bits_for(method, layout.r_min, layout.r_max)
+        self.e_base = exponent_base(method, layout.item_stats)
         self.max_smem_cells = int(max_smem_cells)
         self.launches = 0
         I = layout.n_items
@@ -212,7 +214,7 @@ class SimEngine:
         N.check(L.xmap_build_tri_layout(
             N.ptr(layout.csr_ptr), N.ptr(layout.csr_ent), N.ptr(layout.csc_ptr), N.ptr(layout.csc_ent),
             N.ptr(layout.user_mu), N.ptr(layout.item_stats), N.ptr(meta.prefix_code), N.ptr(self.ord),
-            layout.n_users, I, layout.nnz, N.METHODS[method],
+            layout.n_users, I, layout.nnz, N.METHODS[method], self.e_base,
             N.ptr(self.tcsr_ent), N.ptr(self.csc_aux), N.ptr(self.ostat), N.ptr(self.tri_work),
             N.ptr(ws), ws_bytes, _stream_ptr()), "xmap_build_tri_layout")
         del ws
@@ -280,7 +282,7 @@ class SimEngine:
         a.ord_item = N.ptr(self.ord_item)
         a.dom_code, a.contains = N.ptr(m.dom_code), N.ptr(m.contains)
         a.n_items, a.method = lay.n_items, N.METHODS[self.method]
-        a.num_atleast, a.k, a.r2_bits = self.num_atleast, self.k, self.r2_bits
+        a.num_atleast, a.k, a.r2_bits = self.num_atleast, self.k, 2 * self.e_base
         a.rec_ptr, a.rec_cnt, a.rec, a.rec_n = N.ptr(self.rec_ptr), N.ptr(self.rec_cnt), N.ptr(self.rec), N.ptr(self.rec_n)
         a.count_only = 1 if self.rec is None else 0
         a.bb, a.row_npairs = N.ptr(self.bb), N.ptr(self.row_npairs)
