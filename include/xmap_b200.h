@@ -21,6 +21,7 @@
 #ifndef XMAP_B200_H
 #define XMAP_B200_H
 
+#include <stdbool.h>
 #include <stddef.h>
 #include <stdint.h>
 
@@ -28,7 +29,7 @@
 extern "C" {
 #endif
 
-#define XMAP_B200_ABI_VERSION 7
+#define XMAP_B200_ABI_VERSION 8
 #define XMAP_KMAX 64                 /* largest supported top-k (extend_among_topk) */
 #define XMAP_METHOD_ADJUST_COSINE 0  /* baselinerSim.py:144-174 */
 #define XMAP_METHOD_COSINE 1         /* baselinerSim.py:115-142 */
@@ -378,6 +379,69 @@ int xmap_recsim_private_neighbor(const int64_t *row_ptr, const int32_t *nbr, con
 int xmap_clean_records(const int32_t *user, const int32_t *item, const double *ts, const int64_t *order,
                        int64_t n, int32_t n_users, double t_lo, double t_hi, int32_t num_atleast,
                        uint8_t *keep, int32_t *user_items, void *stream);
+
+/* ---------------------------------------------------------------------------
+ * (7) Text ingest of the rating files: the 4-column reader and the per-record work of clean / split.
+ * Replaces LocalContext.textFile (text mode), the per-line work of BaselinerClean.parse_data
+ * (baselinerClean.py:38-56) and the record placement of BaselinerSplit.split_data (baselinerSplit.py:60-106).
+ * The facade is x-map_b200/ingest.py; the per-user steps of the split (randomSplit, random.sample) stay on the host.
+ *
+ * Byte pass: xmap_ingest_line_masks reads the file bytes (16-byte aligned, padded to 16 bytes) with 16-byte loads and
+ * writes one 16-bit mask per 16-byte chunk, bit b = byte 16c+b ends a line (\n, or \r not followed by \n);
+ * block_cnt[blockIdx] = terminators of each 4 096-byte block.  The caller scans block_cnt into block_off (exclusive,
+ * int64) and xmap_ingest_line_offsets writes offs[k] = byte position of the k-th terminator.  Line k is
+ * [offs[k-1] + 1, offs[k]) (offs[-1] = -1); a file that does not end in a terminator gets one appended by the caller.
+ *
+ * xmap_ingest_parse: per line, status (below), rating and timestamp as float64 (NaN unless OK), and the two ids as
+ * big-endian 64-bit words, zero padded, column-major: uid_words[w * ld + line], iid_words the same with the domain
+ * label (<= 16 bytes) appended to the raw item id.  Only the words an id covers are written: the caller zeroes the
+ * word arrays.  Whitespace = Python's ASCII str.split() set; fields after the fourth are ignored.  Numbers:
+ * [+-]?(d+(.d*)?|.d+)([eE][+-]?d+)? with at most 15 significant digits and a decimal exponent within +-22 (one
+ * correctly rounded operation: bit-equal to Python's float()); timestamps within [ts_min, ts_max].
+ *
+ * xmap_ingest_rank_flags / _scatter: over ids sorted by an LSD sequence of stable sorts of their words (perm),
+ * flag[p] = (id at p != id at p-1); the caller scans flag into csum (inclusive, int64); rank[perm[p]] = csum[p] - 1 and
+ * rep[rank] = a line holding that id.
+ * xmap_ingest_first: records in clean order (xmap_clean_records' `order`): first_user[u] = min in-period line of u
+ * (initialised to INT32_MAX by the caller), pair_first[r] = first in-period line of the (user, item) of kept record r.
+ * xmap_ingest_item_suffix: present[key of iid[-2:]] = 1 (65 536 bytes, zeroed by the caller; key = byte[-2] << 8 |
+ * byte[-1], a 1-byte id: byte << 8).  xmap_ingest_item_codes: the codes of encode.item_codes for items in ascending
+ * id order, rep[i] = a line holding item i; labels = the sorted present keys (<= 8); prefix_new[i] = iid[:2] differs
+ * from item i-1's (scanned by the caller into the prefix rank).
+ * xmap_ingest_train_keys: key[r] = group << 58 | upos[user] << 26 | sub, -1 for a test record; grp[u] 0 non-overlap
+ * source, 1 non-overlap target, 2 both, 3 rest, 4 test user; a test user's record without "S:" is drawn into training
+ * if srank[r] >= 0 (sub = 1 + srank, the order of random.sample), else it is a test record.
+ * ------------------------------------------------------------------------- */
+#define XMAP_INGEST_ID_MAX 48          /* longest uid, and longest raw iid + label, in bytes */
+#define XMAP_INGEST_OK 0
+#define XMAP_INGEST_BLANK 1            /* whitespace only: skipped */
+#define XMAP_INGEST_FEW_FIELDS 2
+#define XMAP_INGEST_NON_ASCII 3
+#define XMAP_INGEST_NUL 4
+#define XMAP_INGEST_BAD_TIME 5
+#define XMAP_INGEST_TIME_RANGE 6
+#define XMAP_INGEST_BAD_RATING 7
+#define XMAP_INGEST_UID_LONG 8
+#define XMAP_INGEST_IID_LONG 9
+int xmap_ingest_line_masks(const void *buf, int64_t size, uint16_t *masks, int32_t *block_cnt, void *stream);
+int xmap_ingest_line_offsets(const uint16_t *masks, int64_t size, const int64_t *block_off, int64_t *offs, void *stream);
+int xmap_ingest_parse(const uint8_t *buf, const int64_t *offs, int64_t n_lines, const char *label_h, int32_t label_len,
+                      double ts_min, double ts_max, int64_t ld, uint8_t *status, double *rating, double *ts,
+                      uint64_t *uid_words, uint8_t *uid_len, uint64_t *iid_words, uint8_t *iid_len, void *stream);
+int xmap_ingest_rank_flags(const uint64_t *words, int64_t ld, int32_t n_words, const int64_t *perm, int64_t n,
+                           int32_t *flag, void *stream);
+int xmap_ingest_rank_scatter(const int64_t *perm, const int32_t *flag, const int64_t *csum, int64_t n, int32_t *rank,
+                             int64_t *rep, void *stream);
+int xmap_ingest_first(const int32_t *user, const int32_t *item, const double *ts, const int64_t *order,
+                      const uint8_t *keep, int64_t n, double t_lo, double t_hi, int32_t *first_user, int32_t *pair_first,
+                      void *stream);
+int xmap_ingest_item_suffix(const uint64_t *iid_words, int64_t ld, const uint8_t *iid_len, const int64_t *rep,
+                            int32_t n_items, uint8_t *present, void *stream);
+int xmap_ingest_item_codes(const uint64_t *iid_words, int64_t ld, const uint8_t *iid_len, const int64_t *rep,
+                           int32_t n_items, const int32_t *labels, int32_t n_labels, int32_t *prefix_new,
+                           uint8_t *dom_code, uint8_t *contains, bool *has_S, bool *has_T, void *stream);
+int xmap_ingest_train_keys(const int32_t *user, const int32_t *item, const int8_t *grp, const int32_t *upos,
+                           const bool *has_S, const int32_t *srank, int64_t n, int64_t *key, void *stream);
 
 #ifdef __cplusplus
 }

@@ -14,8 +14,9 @@ KMAX = 64
 XSIM_MAX_CELLS_LG = 13    # XMAP_XSIM_MAX_CELLS_LG
 METHODS = {"adjust_cosine": 0, "cosine": 1}
 SELECT_LONG = 8192            # XMAP_SELECT_LONG
-ABI_VERSION = 7
+ABI_VERSION = 8
 ROW_HDR_BYTES = 48          # XMAP_SIM_ROW_HDR_BYTES
+INGEST_ID_MAX = 48          # XMAP_INGEST_ID_MAX
 
 _p = C.c_void_p
 
@@ -87,6 +88,16 @@ _SIGS = {
     "xmap_alterego_workspace_bytes": (C.c_size_t, [C.c_int64]),
     "xmap_build_alterego": (C.c_int, [_p, _p, _p, _p, C.c_int32, C.c_int64, _p,
                                       _p, _p, _p, _p, C.POINTER(C.c_int64), _p, C.c_size_t, _p]),
+    "xmap_ingest_line_masks": (C.c_int, [_p, C.c_int64, _p, _p, _p]),
+    "xmap_ingest_line_offsets": (C.c_int, [_p, C.c_int64, _p, _p, _p]),
+    "xmap_ingest_parse": (C.c_int, [_p, _p, C.c_int64, C.c_char_p, C.c_int32, C.c_double, C.c_double, C.c_int64,
+                                    _p, _p, _p, _p, _p, _p, _p, _p]),
+    "xmap_ingest_rank_flags": (C.c_int, [_p, C.c_int64, C.c_int32, _p, C.c_int64, _p, _p]),
+    "xmap_ingest_rank_scatter": (C.c_int, [_p, _p, _p, C.c_int64, _p, _p, _p]),
+    "xmap_ingest_first": (C.c_int, [_p, _p, _p, _p, _p, C.c_int64, C.c_double, C.c_double, _p, _p, _p]),
+    "xmap_ingest_item_suffix": (C.c_int, [_p, C.c_int64, _p, _p, C.c_int32, _p, _p]),
+    "xmap_ingest_item_codes": (C.c_int, [_p, C.c_int64, _p, _p, C.c_int32, _p, C.c_int32, _p, _p, _p, _p, _p, _p]),
+    "xmap_ingest_train_keys": (C.c_int, [_p, _p, _p, _p, _p, _p, C.c_int64, _p, _p]),
 }
 
 EXPORTED_SYMBOLS = tuple(_SIGS)

@@ -18,15 +18,27 @@ def period_bounds(date_from, date_to):
 def clean_encoded(user, item, ts, n_users, t_lo, t_hi, num_atleast, device="cuda"):
     """user / item: int32 indices of the records in arrival order, ts: float64 seconds.
     Returns (keep uint8 [n], distinct in-period items per user int32 [n_users])."""
-    L = N.lib()
     dev = torch.device(device)
     user = torch.as_tensor(user, dtype=torch.int32).to(dev).contiguous()
     item = torch.as_tensor(item, dtype=torch.int32).to(dev).contiguous()
     ts = torch.as_tensor(ts, dtype=torch.float64).to(dev).contiguous()
-    n = int(user.numel())
+    order = clean_order(user, item, ts, t_lo, t_hi)
+    return clean_sorted(user, item, ts, order, n_users, t_lo, t_hi, num_atleast)
+
+
+def clean_order(user, item, ts, t_lo, t_hi):
+    """Record indices sorted, stable, by (out-of-period last, user, item): a (user, item) group is a run in arrival
+    order.  user < 2^30."""
     inp = (ts >= t_lo) & (ts < t_hi)
     key = ((~inp).long() << 62) | (user.long() << 32) | item.long()
-    order = torch.argsort(key, stable=True).contiguous()              # CUB radix sort through torch: library plumbing
+    return torch.argsort(key, stable=True).contiguous()                # CUB radix sort through torch: library plumbing
+
+
+def clean_sorted(user, item, ts, order, n_users, t_lo, t_hi, num_atleast):
+    """clean_encoded on device tensors with their clean_order already computed."""
+    L = N.lib()
+    dev = user.device
+    n = int(user.numel())
     keep = torch.empty(n, dtype=torch.uint8, device=dev)
     user_items = torch.empty(max(int(n_users), 1), dtype=torch.int32, device=dev)
     N.check(L.xmap_clean_records(N.ptr(user), N.ptr(item), N.ptr(ts), N.ptr(order), n, int(n_users),

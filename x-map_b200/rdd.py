@@ -106,12 +106,8 @@ class LocalRDD(object):
         return acc
 
     def randomSplit(self, weights, seed=None):
-        w = np.asarray(weights, dtype=np.float64)
-        edges = np.cumsum(w / w.sum())
-        rng = np.random.RandomState(None if seed is None else seed % (2 ** 32))
-        cell = np.minimum(np.searchsorted(edges, rng.random_sample(len(self._data())), side="right"),
-                          len(w) - 1)
-        return [self._new(x for x, c in zip(self._data(), cell) if c == i) for i in range(len(w))]
+        cell = split_cells(weights, seed, len(self._data()))
+        return [self._new(x for x, c in zip(self._data(), cell) if c == i) for i in range(len(weights))]
 
 
 class LazyRDD(LocalRDD):
@@ -127,6 +123,14 @@ class LazyRDD(LocalRDD):
         if self._records is None:
             self._records = list(self._builder())
         return self._records
+
+
+def split_cells(weights, seed, n):
+    """The part randomSplit puts each of n records in: one RandomState(seed % 2**32) uniform per record."""
+    w = np.asarray(weights, dtype=np.float64)
+    edges = np.cumsum(w / w.sum())
+    rng = np.random.RandomState(None if seed is None else seed % (2 ** 32))
+    return np.minimum(np.searchsorted(edges, rng.random_sample(n), side="right"), len(w) - 1)
 
 
 class LocalContext(object):

@@ -15,15 +15,18 @@ from .rdd import records_of
 
 
 class Session(object):
-    def __init__(self, enc, device="cuda"):
+    def __init__(self, enc, device="cuda", user=None, item=None, rating=None, meta=None):
+        """enc: the host-side Encoded.  user / item / rating / meta: the same arrays and item codes already on the
+        device (ingest.clean_split_pipeline), used instead of copying enc's."""
         self.enc = enc
         self.device = torch.device(device)
-        self.layout = E.build_layout(enc.user, enc.item, enc.rating, enc.n_users, enc.n_items,
-                                     device=self.device)
+        dev = lambda t, a: a if t is None else t
+        self.layout = E.build_layout(dev(user, enc.user), dev(item, enc.item), dev(rating, enc.rating), enc.n_users,
+                                     enc.n_items, device=self.device)
         T = lambda a, dt: torch.as_tensor(a, dtype=dt).to(self.device)
-        self.meta = E.ItemMeta(T(enc.prefix_code, torch.int32), T(enc.dom_code, torch.uint8),
-                               T(enc.contains, torch.uint8), T(enc.has_S, torch.bool),
-                               T(enc.has_T, torch.bool))
+        self.meta = meta if meta is not None else E.ItemMeta(
+            T(enc.prefix_code, torch.int32), T(enc.dom_code, torch.uint8), T(enc.contains, torch.uint8),
+            T(enc.has_S, torch.bool), T(enc.has_T, torch.bool))
         self.sim_engine = None      # engine.SimEngine once similarity has run
         self.tables = None
         self.xsim = None            # (plan, engine, result)
