@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define XMAP_B200_ABI_VERSION 8
+#define XMAP_B200_ABI_VERSION 9
 #define XMAP_KMAX 64                 /* largest supported top-k (extend_among_topk) */
 #define XMAP_METHOD_ADJUST_COSINE 0  /* baselinerSim.py:144-174 */
 #define XMAP_METHOD_COSINE 1         /* baselinerSim.py:115-142 */
@@ -259,7 +259,6 @@ typedef struct xmap_xsim_args {
                                                * than cells_lg runs with its table in the warp's slot of the global workspace */
     void *gws; int32_t gcells_lg;             /* workspace: (SMs x warps) slots of 20 B << gcells_lg (NULL: shared memory only) */
     int32_t top_m;                            /* <= XMAP_KMAX */
-    int32_t merge;                            /* 1: also run the per-start merge of the unit results */
     /* per unit: distinct ends, paths, top-m by |xsim| (ties to the smaller end) */
     int32_t *unit_count; int64_t *unit_combos;
     int32_t *unit_top_end; double *unit_top_xsim; int32_t *unit_top_len;
@@ -273,11 +272,12 @@ typedef struct xmap_xsim_args {
 } xmap_xsim_args;
 
 int64_t xmap_xsim_smem_bytes(int32_t cells_lg, int32_t warps);
+/* Both unit launchers write the per-unit results only; xmap_xsim_merge turns them into the per-start ones. */
 int xmap_xsim_extend(const xmap_xsim_args *args_h, void *stream);
 /* CTA-cooperative variant: one CTA of 8 warps per unit (blockIdx b runs unit_order[b]) with ONE table of
- * 2^cells_lg cells (two CTAs per SM); products are routed through shared memory to the warp that owns the
- * end's table region.  Same unit arrays, outputs and determinism contract; unit_counter / warps / unit_clg /
- * gws are not used. */
+ * 2^cells_lg cells (two CTAs per SM, cells_lg >= 9); products are routed through shared memory to the warp that
+ * owns the end's table region.  Same unit arrays, outputs and determinism contract; unit_counter / warps /
+ * unit_clg / gws are not used. */
 int64_t xmap_xsim_cta_smem_bytes(int32_t cells_lg);
 int xmap_xsim_extend_cta(const xmap_xsim_args *args_h, void *stream);
 /* only the per-start merge (multi-GPU: after the unit results of all ranks have been summed) */

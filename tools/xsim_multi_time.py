@@ -37,7 +37,7 @@ z = lambda shape, dt: torch.zeros(shape, dtype=dt, device=dev)
 bufs = [z(nu, torch.int32), z(nu, torch.int64), z((nu, m), torch.int32), z((nu, m), torch.float64), z(nu, torch.int32)]
 a.unit_count, a.unit_combos, a.unit_top_end, a.unit_top_xsim, a.unit_top_len = [N.ptr(t) for t in bufs]
 order = xe.unit_order[rank::world].contiguous()
-a.unit_order, a.n_units, a.merge = N.ptr(order), int(order.numel()), 0
+a.unit_order, a.n_units = N.ptr(order), int(order.numel())
 for rep in range(2):
     torch.cuda.synchronize(); t0 = time.perf_counter()
     N.check(N.lib().xmap_xsim_extend(a, torch.cuda.current_stream().cuda_stream), "x")

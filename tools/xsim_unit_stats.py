@@ -35,7 +35,7 @@ bufs = [z(nu, torch.int32), z(nu, torch.int64), z((nu, m), torch.int32), z((nu, 
 a.unit_count, a.unit_combos, a.unit_top_end, a.unit_top_xsim, a.unit_top_len = [N.ptr(t) for t in bufs]
 cyc = z(nu, torch.int64)
 a.unit_cycles = N.ptr(cyc)
-a.unit_order, a.n_units, a.merge = N.ptr(xe.unit_order), nu, 0
+a.unit_order, a.n_units = N.ptr(xe.unit_order), nu
 N.check(N.lib().xmap_xsim_extend(a, torch.cuda.current_stream().cuda_stream), "x")
 torch.cuda.synchronize()
 ms = cyc.double() / 1.965e6

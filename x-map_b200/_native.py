@@ -14,7 +14,7 @@ KMAX = 64
 XSIM_MAX_CELLS_LG = 13    # XMAP_XSIM_MAX_CELLS_LG
 METHODS = {"adjust_cosine": 0, "cosine": 1}
 SELECT_LONG = 8192            # XMAP_SELECT_LONG
-ABI_VERSION = 8
+ABI_VERSION = 9
 ROW_HDR_BYTES = 48          # XMAP_SIM_ROW_HDR_BYTES
 INGEST_ID_MAX = 48          # XMAP_INGEST_ID_MAX
 
@@ -43,7 +43,7 @@ class XsimArgs(C.Structure):
         ("rs_ptr", _p), ("rs_end", _p), ("rs_n", _p), ("rs_d", _p), ("rs_c", _p),
         ("tile_ptr", _p), ("gb", C.c_int32),
         ("cells_lg", C.c_int32), ("unit_clg", _p), ("gws", _p), ("gcells_lg", C.c_int32),
-        ("top_m", C.c_int32), ("merge", C.c_int32),
+        ("top_m", C.c_int32),
         ("unit_count", _p), ("unit_combos", _p), ("unit_top_end", _p), ("unit_top_xsim", _p), ("unit_top_len", _p),
         ("out_count", _p), ("out_combos", _p), ("top_end", _p), ("top_xsim", _p), ("top_len", _p),
         ("emit_ptr", _p), ("emit_end", _p), ("emit_xsim", _p),

@@ -59,6 +59,16 @@ __device__ __forceinline__ unsigned long long abs_key(double v) {
     return (unsigned long long)__double_as_longlong(v) & 0x7FFFFFFFFFFFFFFFull;
 }
 
+// Histogram bin of a magnitude key (abs_key bits) for the top-k selections of sim.cu and xsim.cu:
+// 16 sub-bins per octave for |v| in [2^-16, 2): bits 62..48 of the double, offset so that 2^-16 maps
+// to bin 0; smaller values share bin 0, values >= 1 clamp to the top bin.
+constexpr int SIM_BINS = 256;
+__device__ __forceinline__ int sim_bin(unsigned long long key_bits) {
+    const int hi = int((key_bits & 0x7FFFFFFFFFFFFFFFull) >> 48);       // 11 exponent bits + 4 mantissa bits
+    const int base = (1023 - 16) << 4;
+    return max(0, min(SIM_BINS - 1, hi - base));
+}
+
 // warp arg-best over (key, tie, pos); every lane gets the winner.
 __device__ __forceinline__ void warp_argbest(unsigned long long &key, int &tie, int &pos) {
 #pragma unroll

@@ -500,17 +500,8 @@ __global__ void __launch_bounds__(512) tri_gmem_kernel(xmap_sim_args a, const Ro
 // --------------------------------------------------------------------------
 // Selection (extender.py:16-44).
 // --------------------------------------------------------------------------
-constexpr int SEL_BINS = 256;
 constexpr int SEL_BUF = 192;                      // survivors per list
-constexpr int SEL_WARP_BYTES = 2 * SEL_BUF * 16;  // two survivor buffers; aliases the 2 x 256-bin histogram
-
-// 16 sub-bins per octave for |sim| in [2^-16, 2): bits 62..48 of the double, offset so that
-// 2^-16 maps to bin 0; smaller values share bin 0, values >= 1 clamp to the top bin.
-__device__ __forceinline__ int sim_bin(unsigned long long key_bits) {
-    const int hi = int((key_bits & 0x7FFFFFFFFFFFFFFFull) >> 48);       // 11 exponent bits + 4 mantissa bits
-    const int base = (1023 - 16) << 4;
-    return max(0, min(SEL_BINS - 1, hi - base));
-}
+constexpr int SEL_WARP_BYTES = 2 * SEL_BUF * 16;  // two survivor buffers; aliases the 2 x 256-bin histogram (sim_bin)
 
 // list membership of neighbour j for row i: bit 0 = list 0, bit 1 = list 1
 //   BB row: list 0 = other-domain neighbours, list 1 = same-domain (extender.py:30-35)
@@ -586,13 +577,13 @@ __global__ void __launch_bounds__(128) select_warp_kernel(xmap_sim_args a, const
         return;
     }
 
-    unsigned *hist = reinterpret_cast<unsigned *>(s_sel[warp]);      // [2][SEL_BINS]
+    unsigned *hist = reinterpret_cast<unsigned *>(s_sel[warp]);      // [2][SIM_BINS]
     Surv *buf[2] = {reinterpret_cast<Surv *>(s_sel[warp]), reinterpret_cast<Surv *>(s_sel[warp]) + SEL_BUF};
     int nb[2] = {0, 0}, want[2] = {0, 0}, bstar[2] = {0, 0};
     bool overflow[2] = {false, false};
     if (m > SEL_DIRECT) {
         // ---- pass A: per-list histogram of |sim| -------------------------------------------------
-        for (int b = lane; b < 2 * SEL_BINS; b += 32) hist[b] = 0u;
+        for (int b = lane; b < 2 * SIM_BINS; b += 32) hist[b] = 0u;
         __syncwarp();
         // long lists: the histogram is built from every 4th block of 128 records.  The threshold bin of
         // the sample has at least min(K, sample members) entries at or above it, so the full list has
@@ -614,7 +605,7 @@ __global__ void __launch_bounds__(128) select_warp_kernel(xmap_sim_args a, const
             for (int u = 0; u < SU; ++u) {
                 const int bin = sim_bin(v[u].sim);
                 if (lb[u] & 1u) { atomicAdd(&hist[bin], 1u); ++n0; }
-                if (lb[u] & 2u) { atomicAdd(&hist[SEL_BINS + bin], 1u); ++n1; }
+                if (lb[u] & 2u) { atomicAdd(&hist[SIM_BINS + bin], 1u); ++n1; }
             }
         }
 #pragma unroll
@@ -629,8 +620,8 @@ __global__ void __launch_bounds__(128) select_warp_kernel(xmap_sim_args a, const
             // largest bin b* such that #(bin >= b*) >= want: scan the histogram from the top
             int run = 0;
             bool found = false;
-            for (int hb = SEL_BINS - 32; hb >= 0 && !found; hb -= 32) {
-                unsigned suf = hist[list * SEL_BINS + hb + lane];      // suffix sums, highest lane = highest bin
+            for (int hb = SIM_BINS - 32; hb >= 0 && !found; hb -= 32) {
+                unsigned suf = hist[list * SIM_BINS + hb + lane];      // suffix sums, highest lane = highest bin
 #pragma unroll
                 for (int off = 1; off < 32; off <<= 1) {
                     const unsigned t = __shfl_down_sync(0xffffffffu, suf, off);

@@ -241,8 +241,8 @@ XSIM_MAX_PASSES = int(os.environ.get("XMAP_XSIM_MAX_PASSES", "1000000000"))   # 
                                 # global memory (L2).  Measured at cfg2: 32 passes + L2 tables 968 ms, shared memory only
                                 # (no cap) 732 ms -- dependent read-modify-writes at L2 latency lose to narrow passes
 XSIM_GCELLS_LG = 16             # largest global-memory table of a unit (cells)
-XSIM_MODE = os.environ.get("XMAP_XSIM_MODE", "hybrid")                # "warp": one warp per unit (xsim.cu, default); "cta": one CTA
-                                                                   # per unit with one 8x larger table (xsim_cta.cu)
+XSIM_MODE = os.environ.get("XMAP_XSIM_MODE", "hybrid")                # "warp": one warp per unit (xsim_warp_kernel); "cta": one CTA
+                                                                   # per unit with one 8x larger table (xsim_cta_kernel)
 XSIM_FUSE = os.environ.get("XMAP_XSIM_FUSE", "1") != "0"          # fused bridge lists B(t) for the joint-only legs
 XSIM_FUSE_MAX = 1 << 31         # entries (28 B each + sort scratch) above which the lists are not fused: a fixed number, not a
                                 # function of free memory, so that every rank takes the same decision
@@ -543,7 +543,6 @@ class XsimEngine:
         L = N.lib()
         hot = self.hot_order if world == 1 else self.hot_order[rank::world].contiguous()
         cold = self.cold_order if world == 1 else self.cold_order[rank::world].contiguous()
-        a.merge = 0
         self._orders = (hot, cold)                         # keep the device arrays alive until the kernels ran
         side = None
         if hot.numel() and cold.numel() and self.device.type == "cuda":
