@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define XMAP_B200_ABI_VERSION 9
+#define XMAP_B200_ABI_VERSION 10
 #define XMAP_KMAX 64                 /* largest supported top-k (extend_among_topk) */
 #define XMAP_METHOD_ADJUST_COSINE 0  /* baselinerSim.py:144-174 */
 #define XMAP_METHOD_COSINE 1         /* baselinerSim.py:115-142 */
@@ -324,17 +324,23 @@ int xmap_build_alterego(const int32_t *csr_ptr, const uint64_t *csr_ent, const i
  * filtered; self pairs (i, i) exist).
  *   xmap_recsim_item_info : info[3*i..] = (average, norm2, count) over the records of item i, the records
  *                           grouped by item (item_ptr [n_items + 1], rating_by_item).
- *   xmap_recsim_fill_entries: records grouped by user in list order (user_ptr [n_users + 1]); user u owns
- *                           entries [ent_off[u], ent_off[u+1]) with ent_off = exclusive scan of d(d-1).
- *                           key[t] = item_a * n_items + item_b, src[t] = pos_a << 32 | pos_b, t in the
- *                           reference's emission order, so a STABLE sort by key keeps arrival order.
+ *   xmap_recsim_fill_rows : the entries of the item rows [i0, i1), i.e. those whose first record lies on an item
+ *                           in the range (rows never share a directed pair, so a block of rows is filled, sorted and
+ *                           reduced by itself).  Records grouped by user in list order (user_ptr [n_users + 1],
+ *                           n_rec records); in_before [n_rec + 1] = exclusive scan of [item in range] over the
+ *                           records; ent_before [n_rec + 1] = exclusive scan of [record in range] (user end - x - 1)
+ *                           + (in-range records after x in its user), total = ent_before[n_rec].
+ *                           key[t] = item_a * n_items + item_b, src[t] = pos_a << 32 | pos_b, t in the reference's
+ *                           emission order restricted to the rows, so a STABLE sort by key keeps arrival order.
+ *                           With [0, n_items) these are all d(d-1) entries of every user.
  *   xmap_recsim_pairs     : per run of equal keys [seg_ptr[g], seg_ptr[g+1]) of the sorted entries:
  *                           (i, j, n, sim, local sensitivity); NaN rule of Python's max() reproduced.
  * ------------------------------------------------------------------------- */
 int xmap_recsim_item_info(const int64_t *item_ptr, const double *rating_by_item, int32_t n_items, double *info,
                           void *stream);
-int xmap_recsim_fill_entries(const int64_t *user_ptr, const int64_t *ent_off, int32_t n_users, const int32_t *item,
-                             int64_t n_items, int64_t total, int64_t *key, int64_t *src, void *stream);
+int xmap_recsim_fill_rows(const int64_t *user_ptr, int32_t n_users, const int64_t *in_before, const int64_t *ent_before,
+                          int64_t n_rec, const int32_t *item, int64_t n_items, int32_t i0, int32_t i1, int64_t total,
+                          int64_t *key, int64_t *src, void *stream);
 int xmap_recsim_pairs(const int64_t *seg_ptr, const int64_t *seg_key, const int64_t *src, const double *rating,
                       const double *info, int64_t n_items, int64_t n_pairs, int32_t num_atleast,
                       int32_t *out_i, int32_t *out_j, int64_t *out_n, double *out_sim, double *out_ls, void *stream);

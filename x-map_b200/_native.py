@@ -14,7 +14,7 @@ KMAX = 64
 XSIM_MAX_CELLS_LG = 13    # XMAP_XSIM_MAX_CELLS_LG
 METHODS = {"adjust_cosine": 0, "cosine": 1}
 SELECT_LONG = 8192            # XMAP_SELECT_LONG
-ABI_VERSION = 9
+ABI_VERSION = 10
 ROW_HDR_BYTES = 48          # XMAP_SIM_ROW_HDR_BYTES
 INGEST_ID_MAX = 48          # XMAP_INGEST_ID_MAX
 
@@ -74,7 +74,8 @@ _SIGS = {
     "xmap_xsim_cta_smem_bytes": (C.c_int64, [C.c_int32]),
     "xmap_xsim_extend_cta": (C.c_int, [C.POINTER(XsimArgs), _p]),
     "xmap_recsim_item_info": (C.c_int, [_p, _p, C.c_int32, _p, _p]),
-    "xmap_recsim_fill_entries": (C.c_int, [_p, _p, C.c_int32, _p, C.c_int64, C.c_int64, _p, _p, _p]),
+    "xmap_recsim_fill_rows": (C.c_int, [_p, C.c_int32, _p, _p, C.c_int64, _p, C.c_int64, C.c_int32, C.c_int32, C.c_int64,
+                                        _p, _p, _p]),
     "xmap_recsim_pairs": (C.c_int, [_p, _p, _p, _p, _p, C.c_int64, C.c_int64, C.c_int32, _p, _p, _p, _p, _p, _p]),
     "xmap_recsim_neighbors": (C.c_int, [_p, _p, _p, C.c_int32, C.c_int32, _p, _p, _p, _p]),
     "xmap_recsim_predict": (C.c_int, [_p, _p, _p, _p, _p, _p, _p, _p, C.c_int32, _p, _p, C.c_int64, C.c_double,

@@ -35,7 +35,8 @@ class ProfileState(object):
         self.ts = np.array([_ts(r[3]) for r in recs], dtype=np.int64)
         self.upos = {s: n for n, s in enumerate(self.uids)}
         self.ipos = {s: n for n, s in enumerate(self.iids)}
-        self.sim = None          # recsim.RecSim
+        self.num_atleast = None  # set by RecommenderSim.calculate_sim
+        self.knn = None          # recsim.ItemKnn: item info and the neighbour tables
         self.nb = None           # recsim.Neighbors
 
 
@@ -66,15 +67,16 @@ class RecommenderSim(object):
         the same.  Anything else (the user-based names) returns None in the reference and raises here."""
         if "cosine_item" not in self.method:
             raise ValueError("only the item-based similarities are offered (got %r)" % (self.method,))
-        if state.sim is None:
-            state.sim = RS.cosine_item(state.user, state.item, state.rating, len(state.iids), self.num_atleast)
+        state.num_atleast = self.num_atleast
 
         def build():
-            s = state.sim
-            i, j = s.i.cpu().numpy(), s.j.cpu().numpy()
-            sim, ls = s.sim.cpu().numpy(), s.ls.cpu().numpy()
-            for q in range(len(i)):
-                yield (str(state.iids[i[q]]), str(state.iids[j[q]])), [sim[q], ls[q]]
+            # only when the records are collected, one block of item rows at a time; the neighbour selection
+            # (recommender_privacy_pipeline) runs from the profile and never needs them
+            for s in RS.pair_passes(state.user, state.item, state.rating, len(state.iids), self.num_atleast):
+                i, j = s.i.cpu().numpy(), s.j.cpu().numpy()
+                sim, ls = s.sim.cpu().numpy(), s.ls.cpu().numpy()
+                for q in range(len(i)):
+                    yield (str(state.iids[i[q]]), str(state.iids[j[q]])), [sim[q], ls[q]]
         return LazyRDD(build, handle=state)
 
 
@@ -104,7 +106,9 @@ class RecommenderPrivacy(object):
         """(iid, [(neighbour, [sim, ls])*]) -- recommenderPrivacy.py:141-150; here the sensitivity is already dropped
         (nonnoise_perturbation, :180-189), which is all the non-private pipeline keeps."""
         state = rdd.handle
-        state.nb = RS.neighbors(state.sim, len(state.iids), int(self.mapping_range))
+        state.knn = RS.item_knn(state.user, state.item, state.rating, len(state.iids), state.num_atleast,
+                                int(self.mapping_range))
+        state.nb = state.knn.nb
         return self._neighbour_rdd(state)
 
     def nonnoise_perturbation(self, rdd):
@@ -118,8 +122,10 @@ class RecommenderPrivacy(object):
         up, un = self.uniforms if self.uniforms is not None else (None, None)
         seed = (self.seed + 0x9E3779B97F4A7C15 * self._calls) & (2 ** 64 - 1)
         self._calls += 1
-        state.nb = RS.private_neighbors(state.sim, len(state.iids), int(self.mapping_range), 2 * self.privacy_epsilon,
-                                        self.rpo, up, un, seed)
+        state.knn = RS.item_knn(state.user, state.item, state.rating, len(state.iids), state.num_atleast,
+                                int(self.mapping_range), private=dict(privacy_epsilon=2 * self.privacy_epsilon, rpo=self.rpo,
+                                                                      u_pick=up, u_noise=un, seed=seed))
+        state.nb = state.knn.nb
         return self._neighbour_rdd(state)
 
     def noise_perturbation(self, rdd):
@@ -140,7 +146,7 @@ class RecommenderPrediction(object):
     def item_based_recommendation(self, test_dataRDD, item_based_dict_bd, itembased_sim_pair_dict_bd, item_info_bd):
         """(uid, [(iid, real rating, prediction, prediction with decay)*])* -- recommenderPrediction.py:105-114."""
         state = getattr(getattr(itembased_sim_pair_dict_bd, "value", itembased_sim_pair_dict_bd), "handle", None)
-        if state is None or state.nb is None:
+        if state is None or state.nb is None or state.knn is None:
             raise TypeError("expected the neighbour dictionary returned by recommender_privacy_pipeline "
                             "(it carries the device-resident tables)")
         test = records_of(test_dataRDD)
@@ -149,7 +155,7 @@ class RecommenderPrediction(object):
             for b, (iid, r, _t) in enumerate(lst):
                 if str(iid) in state.ipos and str(uid) in state.upos:
                     tu.append(state.upos[str(uid)]); ti.append(state.ipos[str(iid)]); tr.append(float(r)); where.append((a, b))
-        p0, p1, _, _ = RS.predict(state.user, state.item, state.rating, state.ts, len(state.uids), state.sim, state.nb,
+        p0, p1, _, _ = RS.predict(state.user, state.item, state.rating, state.ts, len(state.uids), state.knn, state.nb,
                                   np.array(tu, dtype=np.int32), np.array(ti, dtype=np.int32), None, self.alpha)
         p0, p1 = p0.cpu().numpy(), p1.cpu().numpy()
         out = [(uid, [() for _ in lst]) for uid, lst in test]
@@ -177,7 +183,7 @@ def recommender_calculate_sim_pipeline(sc, cross_sim_tool, alterEgo_profile):
     user_based = cross_sim_tool.build_sthbased_profile(flat, "user")
     item_based = cross_sim_tool.build_sthbased_profile(flat, "item")
     sims = cross_sim_tool.calculate_sim(state)
-    info = state.sim.info.cpu().numpy()
+    info = RS.item_info(state.item, state.rating, len(state.iids)).cpu().numpy()
     item_info = {str(s): (info[n, 0], info[n, 1], int(info[n, 2])) for n, s in enumerate(state.iids)}
     user_info = {}
     for uid, lst in user_based.collect():

@@ -13,9 +13,10 @@
 //     and the local sensitivity max |v - sim| over the 2 n leave-one-out similarities (:98-116), where
 //     Python's max() lets a NaN win only if it is the first element.
 //
-// Device design: HBM-bound streaming in three steps.  (1) fill: one thread per co-rating entry computes its
-// directed pair key and the positions of its two records (the entry index follows the reference's emission
-// order, so a STABLE sort by key leaves every pair's entries in arrival order); (2) the caller sorts the keys
+// Device design: HBM-bound streaming in three steps, run on a contiguous block of item rows at a time (rows never
+// share a directed pair, so a block is complete by itself).  (1) fill: one thread per co-rating entry whose first
+// record lies on an item of the block computes its directed pair key and the positions of its two records (in the
+// reference's emission order, so a STABLE sort by key leaves every pair's entries in arrival order); (2) the caller sorts the keys
 // (CUB radix sort through torch: library plumbing); (3) pairs: one warp per pair walks its entries twice --
 // the inner product, then the 2 n leave-one-out deviations, which need the finished inner product.
 #include "common.cuh"
@@ -44,26 +45,42 @@ __global__ void __launch_bounds__(256) recsim_item_info_kernel(const int64_t *__
     }
 }
 
-// entry t of user u (records [lo, lo + d)): combination c = t / 2 in lexicographic (p < q) order, direction t % 2
-__global__ void __launch_bounds__(256) recsim_fill_kernel(const int64_t *__restrict__ user_ptr, const int64_t *__restrict__ ent_off,
-                                                          int32_t n_users, const int32_t *__restrict__ item, int64_t n_items,
-                                                          int64_t total, int64_t *__restrict__ key, int64_t *__restrict__ src) {
+// Entries of the item rows [i0, i1): entry (p -> q) of a user (records [lo, hi), p != q) belongs to the rows when
+// item[p] lies in the range.  The reference emits a user's entries by combination (m, q), m < q, in lexicographic
+// order, (m -> q) before (q -> m) (recommenderSim.py:64-75).  Thread t writes the t-th entry of the rows in that
+// same order, so a STABLE sort by key leaves every pair's entries in arrival order, whatever the range.  Per record x
+// (positions in the user-grouped arrays): in_before[x] = in-range records before x; ent_before[x] = the entries whose
+// smaller position lies before x, i.e. the exclusive scan of [x in range] (hi - x - 1) + (in-range records after x in
+// its user).  With the full range this is the d (d - 1) entries of every user in emission order.
+__global__ void __launch_bounds__(256) recsim_fill_kernel(const int64_t *__restrict__ user_ptr, int32_t n_users,
+                                                          const int64_t *__restrict__ in_before,
+                                                          const int64_t *__restrict__ ent_before, int64_t n_rec,
+                                                          const int32_t *__restrict__ item, int64_t n_items, int32_t i0,
+                                                          int32_t i1, int64_t total, int64_t *__restrict__ key,
+                                                          int64_t *__restrict__ src) {
     const int64_t t = blockIdx.x * (int64_t)256 + threadIdx.x;
     if (t >= total) return;
-    int32_t a = 0, b = n_users;                          // largest u with ent_off[u] <= t (users without entries are skipped)
-    while (b - a > 1) {
-        const int32_t mid = (a + b) >> 1;
-        if (__ldg(ent_off + mid) <= t) a = mid; else b = mid;
+    int64_t m = 0, b = n_rec;                            // the smaller position: largest m with ent_before[m] <= t
+    while (b - m > 1) {
+        const int64_t mid = (m + b) >> 1;
+        if (__ldg(ent_before + mid) <= t) m = mid; else b = mid;
     }
-    const int64_t lo = user_ptr[a], d = user_ptr[a + 1] - lo;
-    const int64_t e = t - ent_off[a], c = e >> 1;
-    // p = the row of combination c: c >= p (2 d - p - 1) / 2
-    int64_t p = (int64_t)floor(((double)(2 * d - 1) - sqrt((double)(2 * d - 1) * (double)(2 * d - 1) - 8.0 * (double)c)) * 0.5);
-    p = max((int64_t)0, min(p, d - 2));
-    while (p > 0 && p * (2 * d - p - 1) / 2 > c) --p;
-    while ((p + 1) * (2 * d - p - 2) / 2 <= c) ++p;
-    const int64_t q = p + 1 + (c - p * (2 * d - p - 1) / 2);
-    const int64_t pa = (e & 1) ? lo + q : lo + p, pb = (e & 1) ? lo + p : lo + q;
+    int32_t ua = 0, ub = n_users;                        // its user: largest u with user_ptr[u] <= m
+    while (ub - ua > 1) {
+        const int32_t mid = (ua + ub) >> 1;
+        if (__ldg(user_ptr + mid) <= m) ua = mid; else ub = mid;
+    }
+    const int64_t hi = user_ptr[ua + 1], e = t - ent_before[m], base = in_before[m + 1];
+    const int32_t im = item[m];
+    const int64_t fm = (im >= i0 && im < i1) ? 1 : 0;
+    // partner q > m: the entries of (m, q') for q' < q number fm (q - m - 1) + in-range records in (m, q)
+    int64_t q = m + 1, qb = hi;                          // largest q with that count <= e
+    while (qb - q > 1) {
+        const int64_t mid = (q + qb) >> 1;
+        if (fm * (mid - m - 1) + __ldg(in_before + mid) - base <= e) q = mid; else qb = mid;
+    }
+    const bool fwd = fm && e == fm * (q - m - 1) + in_before[q] - base;     // (m -> q) comes before (q -> m)
+    const int64_t pa = fwd ? m : q, pb = fwd ? q : m;
     key[t] = (int64_t)item[pa] * n_items + (int64_t)item[pb];
     src[t] = (pa << 32) | pb;
 }
@@ -361,11 +378,13 @@ extern "C" int xmap_recsim_item_info(const int64_t *item_ptr, const double *rati
     return 0;
 }
 
-extern "C" int xmap_recsim_fill_entries(const int64_t *user_ptr, const int64_t *ent_off, int32_t n_users, const int32_t *item,
-                                        int64_t n_items, int64_t total, int64_t *key, int64_t *src, void *stream_) {
+extern "C" int xmap_recsim_fill_rows(const int64_t *user_ptr, int32_t n_users, const int64_t *in_before,
+                                     const int64_t *ent_before, int64_t n_rec, const int32_t *item, int64_t n_items,
+                                     int32_t i0, int32_t i1, int64_t total, int64_t *key, int64_t *src, void *stream_) {
     if (total <= 0) return 0;
-    recsim_fill_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream_>>>(user_ptr, ent_off, n_users, item, n_items,
-                                                                                          total, key, src);
+    if (i0 < 0 || i1 < i0 || i1 > n_items) return fail_msg("xmap_recsim_fill_rows: row range outside [0, n_items]");
+    recsim_fill_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream_>>>(
+        user_ptr, n_users, in_before, ent_before, n_rec, item, n_items, i0, i1, total, key, src);
     XMAP_LAUNCH_CHECK();
     return 0;
 }
