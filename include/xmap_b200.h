@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define XMAP_B200_ABI_VERSION 10
+#define XMAP_B200_ABI_VERSION 11
 #define XMAP_KMAX 64                 /* largest supported top-k (extend_among_topk) */
 #define XMAP_METHOD_ADJUST_COSINE 0  /* baselinerSim.py:144-174 */
 #define XMAP_METHOD_COSINE 1         /* baselinerSim.py:115-142 */
@@ -359,6 +359,29 @@ int xmap_recsim_predict(const int64_t *prof_ptr, const int32_t *prof_item, const
                         const int64_t *prof_ts, const double *info, const int32_t *nb_idx, const double *nb_sim,
                         const int32_t *nb_len, int32_t k, const int32_t *t_user, const int32_t *t_item, int64_t n_test,
                         double alpha, double *pred_nodecay, double *pred_decay, int32_t *error_flag, void *stream);
+
+/* (5d) Top-N recommendation on the AlterEgo profile: every user's first n (1..XMAP_TOPN_MAX) items by the score of
+ * xmap_recsim_predict BEFORE bound_rating (RecommenderPrediction.item_based_prediction, recommenderPrediction.py:26-103;
+ * the reference has no top-N function), without (decay = 0) or with temporal decay.  Candidates are the items with
+ * nb_len > 0 the user has no record on; order: score descending, then the smaller index (-0.0 equals 0.0); NaN scores
+ * are never recommended; an item none of whose neighbours the user rated scores its average info[3*i].
+ *   prof_ptr [n_users + 1]: the records grouped by user and sorted STABLY by item inside each user (so the records on
+ *       one item are a run in list order); info / nb_* as for xmap_recsim_predict (any k);
+ *   rev_ptr [n_items + 1], rev_item: for every item j the items i that list j as a neighbour, ascending;
+ *   fallback [n_fallback]: the items with nb_len > 0 and a non-NaN average, sorted by (average desc, index asc);
+ *   warp_users: users with sum over their distinct items j of |rev(j)| <= XMAP_TOPN_WARP_BOUND (one warp each);
+ *   cta_users: any users (one CTA each; the item axis in tiles of 2^19 items);
+ *   out_idx [n_users][n] (-1 padded), out_score [n_users][n] (NaN padded), out_len [n_users]: written for the listed
+ *   users only; stats[0] += reverse-index entries visited, stats[1] += distinct overlap candidates (unsigned 64-bit).
+ *   error_flag 4: more than 128 matching profile records for one candidate, as in xmap_recsim_predict. */
+#define XMAP_TOPN_MAX 64
+#define XMAP_TOPN_WARP_BOUND 2048
+int xmap_recsim_top_n(const int64_t *prof_ptr, const int32_t *prof_item, const double *prof_rating, const int64_t *prof_ts,
+                      const double *info, const int32_t *nb_idx, const double *nb_sim, const int32_t *nb_len, int32_t k,
+                      int32_t n_items, const int64_t *rev_ptr, const int32_t *rev_item, const int32_t *fallback,
+                      int32_t n_fallback, const int32_t *warp_users, int32_t n_warp_users, const int32_t *cta_users,
+                      int32_t n_cta_users, int32_t n, double alpha, int32_t decay, int32_t *out_idx, double *out_score,
+                      int32_t *out_len, unsigned long long *stats, int32_t *error_flag, void *stream);
 
 /* (5c) PRIVATE neighbour selection + noise perturbation (RecommenderPrivacy.private_neighbor_selection +
  * noise_perturbation, recommenderPrivacy.py:35-139, 152-171) as the reference behaves under Python 3 (one neighbour per

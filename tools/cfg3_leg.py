@@ -21,17 +21,42 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 
 
+def alterego_profile(wl, dev, timed=lambda key, fn: fn()):
+    """The AlterEgo profile of BASELINE.json configs[2] on the workload `wl` (bench.make_workload): similarity, X-SIM,
+    private generation (exponential mechanism, eps = 0.6, mapping_range = 1, Philox draws), then the untouched target
+    ratings followed by the synthetic records (generator.py:156-157), sorted stably by (user, item).  timed(key, fn)
+    runs each stage.  Returns (user, item, rating, ts) on `dev` and the number of synthetic records."""
+    import torch
+    from xmap_b200 import engine as E, extend as X, generate as G
+    meta = E.to_device_meta(wl["meta"], dev)
+    lay = timed("layout_ms", lambda: E.build_layout(wl["user"], wl["item"], wl["rating"], wl["n_users"], wl["n_items"], device=dev))
+    eng = E.SimEngine(lay, meta, "adjust_cosine", 50, wl["k"])
+    tabs = timed("similarity_ms", eng.run)
+    plan = timed("extend_plan_ms", lambda: X.build_plan(tabs, lay.item_stats[:, 3].contiguous(), meta.has_S, meta.has_T))
+    res = timed("extend_ms", lambda: X.XsimEngine(plan, 10).run())
+    ch = timed("choose_exp_mech_ms", lambda: G.choose_mapping(res, "exp_mech", epsilon=0.6, mapping_range=1,
+                                                             sim_method="adjust_cosine", seed=20261018))
+    mp = G.invert_mapping(res.start_item, ch, wl["n_items"])
+    ou, oi, orr, ot = timed("alterego_ms", lambda: G.build_alterego(lay, wl["ts"], mp))
+    item_all = torch.as_tensor(wl["item"], device=dev).long()
+    keep = meta.has_T[item_all]
+    pu = torch.cat([torch.as_tensor(wl["user"], device=dev).long()[keep], ou.long()])
+    pi = torch.cat([item_all[keep], oi.long()])
+    pr = torch.cat([torch.as_tensor(wl["rating"], device=dev).double()[keep], orr])
+    pt = torch.cat([torch.as_tensor(wl["ts"], device=dev)[keep], ot])
+    o = torch.argsort(pu * wl["n_items"] + pi, stable=True)
+    return pu[o], pi[o], pr[o], pt[o], int(ou.numel())
+
+
 def main():
-    import numpy as np
     import torch
     import bench
     from ingest_time import gpu_info
-    from xmap_b200 import engine as E, extend as X, generate as G, recsim as RS
+    from xmap_b200 import recsim as RS
     name = sys.argv[1] if len(sys.argv) > 1 else "cfg2"
     n_test = int(sys.argv[2]) if len(sys.argv) > 2 else 200000
     wl = bench.make_workload(name)
     dev = torch.device("cuda")
-    meta = E.to_device_meta(wl["meta"], dev)
     T = {}
 
     def timed(key, fn):
@@ -40,25 +65,7 @@ def main():
         torch.cuda.synchronize(); T[key] = (time.perf_counter() - t0) * 1e3
         return r
     for rep in range(2):                                   # second pass warm
-        lay = timed("layout_ms", lambda: E.build_layout(wl["user"], wl["item"], wl["rating"], wl["n_users"], wl["n_items"], device=dev))
-        eng = E.SimEngine(lay, meta, "adjust_cosine", 50, wl["k"])
-        tabs = timed("similarity_ms", eng.run)
-        plan = timed("extend_plan_ms", lambda: X.build_plan(tabs, lay.item_stats[:, 3].contiguous(), meta.has_S, meta.has_T))
-        res = timed("extend_ms", lambda: X.XsimEngine(plan, 10).run())
-        # private generation: exponential mechanism, eps = 0.6, mapping_range = 1 (parameters.yaml:22-25), Philox draws
-        ch = timed("choose_exp_mech_ms", lambda: G.choose_mapping(res, "exp_mech", epsilon=0.6, mapping_range=1,
-                                                                 sim_method="adjust_cosine", seed=20261018))
-        mp = G.invert_mapping(res.start_item, ch, wl["n_items"])
-        ou, oi, orr, ot = timed("alterego_ms", lambda: G.build_alterego(lay, wl["ts"], mp))
-        # the AlterEgo profile: untouched target ratings + the synthetic records (generator.py:156-157)
-        item_all = torch.as_tensor(wl["item"], device=dev).long()
-        keep = meta.has_T[item_all]
-        pu = torch.cat([torch.as_tensor(wl["user"], device=dev).long()[keep], ou.long()])
-        pi = torch.cat([item_all[keep], oi.long()])
-        pr = torch.cat([torch.as_tensor(wl["rating"], device=dev).double()[keep], orr])
-        pt = torch.cat([torch.as_tensor(wl["ts"], device=dev)[keep], ot])
-        o = torch.argsort(pu * wl["n_items"] + pi, stable=True)
-        pu, pi, pr, pt = pu[o], pi[o], pr[o], pt[o]
+        pu, pi, pr, pt, n_syn = alterego_profile(wl, dev, timed)
         knn = timed("item_knn_ms", lambda: RS.item_knn(pu, pi, pr, wl["n_items"], 50, 10))
         # hidden test ratings: random (profile user, target item) pairs with integer ratings
         g = torch.Generator(device="cpu").manual_seed(7)
@@ -71,7 +78,7 @@ def main():
     line = {"workload": "cfg3 @ %s" % bench.workload_label(wl, "adjust_cosine"), **gpu_info(),
             "generation": "exponential mechanism, eps=0.6, mapping_range=1, Philox4x32-10(seed, row)",
             "stage_ms": {k: round(v, 3) for k, v in out.items()},
-            "profile_records": int(pu.numel()), "synthetic_records": int(ou.numel()),
+            "profile_records": int(pu.numel()), "synthetic_records": n_syn,
             "recsim_entries": knn.n_entries, "recsim_passes": knn.passes, "recsim_max_row_entries": knn.max_row_entries,
             "recsim_ms_per_pass": round(out["item_knn_ms"] / max(knn.passes, 1), 3),
             "recsim_entries_per_s": knn.n_entries / (out["item_knn_ms"] * 1e-3),

@@ -14,9 +14,11 @@ KMAX = 64
 XSIM_MAX_CELLS_LG = 13    # XMAP_XSIM_MAX_CELLS_LG
 METHODS = {"adjust_cosine": 0, "cosine": 1}
 SELECT_LONG = 8192            # XMAP_SELECT_LONG
-ABI_VERSION = 10
+ABI_VERSION = 11
 ROW_HDR_BYTES = 48          # XMAP_SIM_ROW_HDR_BYTES
 INGEST_ID_MAX = 48          # XMAP_INGEST_ID_MAX
+TOPN_MAX = 64               # XMAP_TOPN_MAX
+TOPN_WARP_BOUND = 2048      # XMAP_TOPN_WARP_BOUND
 
 _p = C.c_void_p
 
@@ -80,6 +82,9 @@ _SIGS = {
     "xmap_recsim_neighbors": (C.c_int, [_p, _p, _p, C.c_int32, C.c_int32, _p, _p, _p, _p]),
     "xmap_recsim_predict": (C.c_int, [_p, _p, _p, _p, _p, _p, _p, _p, C.c_int32, _p, _p, C.c_int64, C.c_double,
                                       _p, _p, _p, _p]),
+    "xmap_recsim_top_n": (C.c_int, [_p, _p, _p, _p, _p, _p, _p, _p, C.c_int32, C.c_int32, _p, _p, _p, C.c_int32,
+                                    _p, C.c_int32, _p, C.c_int32, C.c_int32, C.c_double, C.c_int32, _p, _p, _p, _p, _p,
+                                    _p]),
     "xmap_recsim_private_neighbor": (C.c_int, [_p, _p, _p, _p, C.c_int32, C.c_int32, C.c_double, C.c_double, _p, _p, C.c_uint64,
                                                _p, _p, _p, _p, _p]),
     "xmap_clean_records": (C.c_int, [_p, _p, _p, _p, C.c_int64, C.c_int32, C.c_double, C.c_double, C.c_int32, _p, _p, _p]),

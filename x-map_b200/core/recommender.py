@@ -200,6 +200,22 @@ def recommender_privacy_pipeline(policy_tool, alterEgo_sim, is_private):
     return policy_tool.nonnoise_perturbation(policy_tool.nonprivate_neighbor_selection(alterEgo_sim))
 
 
+def recommend_top_n(simpair_dict_bd, n, decay=False, alpha=0.03):
+    """(uid, [(iid, score)*])* in uid order: every profile user's first n (1..64) items by score, best first.  The
+    reference has no such function: the score is its item-based prediction (recommenderPrediction.py:26-103) before
+    bound_rating rounds it, without or with temporal decay (weight alpha), over the items with a neighbour list the
+    user has no record on; ties go to the smaller item index (iids ordered as strings).  simpair_dict_bd: what
+    recommender_privacy_pipeline(...).collectAsMap() returns, or its broadcast."""
+    state = getattr(getattr(simpair_dict_bd, "value", simpair_dict_bd), "handle", None)
+    if state is None or state.nb is None or state.knn is None:
+        raise TypeError("expected the neighbour dictionary returned by recommender_privacy_pipeline "
+                        "(it carries the device-resident tables)")
+    res = RS.top_n(state.user, state.item, state.rating, state.ts, len(state.uids), state.knn, state.nb, n, decay, alpha)
+    idx, score, ln = res.idx.cpu().numpy(), res.score.cpu().numpy(), res.len.cpu().numpy()
+    return LocalRDD([(str(uid), [(str(state.iids[idx[u, p]]), float(score[u, p])) for p in range(ln[u])])
+                     for u, uid in enumerate(state.uids)])
+
+
 def recommender_prediction_pipeline(recommender_tool, cross_sim_tool, testRDD, simpair_dict_bd,
                                     user_based_dict_bd, item_based_dict_bd, user_info_bd, item_info_bd):
     """assist.py:195-207 (item-based methods)."""

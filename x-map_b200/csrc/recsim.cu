@@ -181,35 +181,66 @@ __device__ __forceinline__ double rs_bound_rating(double x) {      // :19-24, in
     return 1.0 * (double)max(0, min(v, 5));
 }
 
-__global__ void __launch_bounds__(128) recsim_predict_kernel(const int64_t *__restrict__ prof_ptr, const int32_t *__restrict__ prof_item,
-                                                             const double *__restrict__ prof_rating, const int64_t *__restrict__ prof_ts,
-                                                             const double *__restrict__ info, const int32_t *__restrict__ nb_idx,
-                                                             const double *__restrict__ nb_sim, const int32_t *__restrict__ nb_len, int32_t K,
-                                                             const int32_t *__restrict__ t_user, const int32_t *__restrict__ t_item,
-                                                             int64_t n_test, double alpha, double *__restrict__ pred0,
-                                                             double *__restrict__ pred1, int32_t *__restrict__ error_flag) {
-    const int64_t q = blockIdx.x * (int64_t)128 + threadIdx.x;
-    if (q >= n_test) return;
-    const int u = t_user[q], it = t_item[q];
-    const int L = nb_len[it];
-    if (L == 0) { pred0[q] = -1.0; pred1[q] = -1.0; return; }        // `iid not in sim_bd.value.keys()` -> ()
+// One user's records in profile list order (the test pairs of recsim_predict_kernel): the records on an item are
+// found by a scan.  first(nid) / after(e, nid) walk them in list order and give hi at the end.
+struct ListRecords {
+    const int32_t *item; const double *rating; const int64_t *ts; int64_t lo, hi;
+    __device__ __forceinline__ int64_t next(int64_t e, int nid) const {      // the first record on nid at or after e
+        while (e < hi && item[e] != nid) ++e;
+        return e;
+    }
+    __device__ __forceinline__ int64_t first(int nid) const { return next(lo, nid); }
+    __device__ __forceinline__ int64_t after(int64_t e, int nid) const { return next(e + 1, nid); }
+};
+
+// One user's records sorted by (item, list position) (the top-N kernels): the records on an item are one run, found
+// by a binary search, in list order -- the same records in the same order as ListRecords.
+__device__ __forceinline__ int64_t rs_lower_bound(const int32_t *a, int64_t lo, int64_t hi, int32_t v) {
+    while (lo < hi) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (a[mid] < v) lo = mid + 1; else hi = mid;
+    }
+    return lo;
+}
+
+struct SortedRecords {
+    const int32_t *item; const double *rating; const int64_t *ts; int64_t lo, hi;
+    __device__ __forceinline__ int64_t first(int nid) const {
+        const int64_t e = rs_lower_bound(item, lo, hi, nid);
+        return e < hi && item[e] == nid ? e : hi;
+    }
+    __device__ __forceinline__ int64_t after(int64_t e, int nid) const { return e + 1 < hi && item[e + 1] == nid ? e + 1 : hi; }
+    __device__ __forceinline__ bool has(int nid) const {
+        const int64_t e = rs_lower_bound(item, lo, hi, nid);
+        return e < hi && item[e] == nid;
+    }
+};
+
+// The prediction of item `it` (nb_len[it] = L > 0) for the user whose records `recs` holds, before bound_rating:
+// p0 without decay, p1 with decay.  Returns 0, or 4 when more than PRED_CAP records match (p0 / p1 are then
+// meaningless).  The one implementation of the formula: recsim_predict_kernel and the top-N kernels call it.
+template <class Records>
+__device__ __forceinline__ int rs_predict_raw(const Records &recs, int it, int L, const double *__restrict__ info,
+                                              const int32_t *__restrict__ nb_idx, const double *__restrict__ nb_sim,
+                                              int K, double alpha, double &p0, double &p1) {
     double ea[PRED_CAP], eb[PRED_CAP];
     long long et[PRED_CAP];
     int n = 0;
-    const int64_t lo = prof_ptr[u], hi = prof_ptr[u + 1];
     for (int r = 0; r < L; ++r) {
         const int nid = nb_idx[(size_t)it * K + r];
         const double ns = nb_sim[(size_t)it * K + r];
         const double avg_n = info[3 * (size_t)nid];
-        for (int64_t e = lo; e < hi; ++e) {
-            if (prof_item[e] != nid) continue;
-            if (n == PRED_CAP) { atomicExch(error_flag, 4); break; }
-            ea[n] = __dmul_rn(ns, __dsub_rn(prof_rating[e], avg_n)); eb[n] = fabs(ns); et[n] = prof_ts[e];
+        for (int64_t e = recs.first(nid); e < recs.hi; e = recs.after(e, nid)) {
+            if (n == PRED_CAP) { ++n; goto gathered; }               // n = PRED_CAP + 1 marks the overflow
+            ea[n] = __dmul_rn(ns, __dsub_rn(recs.rating[e], avg_n)); eb[n] = fabs(ns); et[n] = recs.ts[e];
             ++n;
         }
     }
+gathered:
+    const int err = n > PRED_CAP ? 4 : 0;
+    n = min(n, PRED_CAP);
     const double avg = info[3 * (size_t)it];
-    double p0 = avg, p1 = avg;
+    p0 = avg; p1 = avg;
     if (n > 0) {
         double sa = 0.0, sb = 0.0;
         for (int k = 0; k < n; ++k) { sa = __dadd_rn(sa, ea[k]); sb = __dadd_rn(sb, eb[k]); }
@@ -232,7 +263,224 @@ __global__ void __launch_bounds__(128) recsim_predict_kernel(const int64_t *__re
         }
         p1 = __dadd_rn(avg, __ddiv_rn(sa, sb));
     }
+    return err;
+}
+
+__global__ void __launch_bounds__(128) recsim_predict_kernel(const int64_t *__restrict__ prof_ptr, const int32_t *__restrict__ prof_item,
+                                                             const double *__restrict__ prof_rating, const int64_t *__restrict__ prof_ts,
+                                                             const double *__restrict__ info, const int32_t *__restrict__ nb_idx,
+                                                             const double *__restrict__ nb_sim, const int32_t *__restrict__ nb_len, int32_t K,
+                                                             const int32_t *__restrict__ t_user, const int32_t *__restrict__ t_item,
+                                                             int64_t n_test, double alpha, double *__restrict__ pred0,
+                                                             double *__restrict__ pred1, int32_t *__restrict__ error_flag) {
+    const int64_t q = blockIdx.x * (int64_t)128 + threadIdx.x;
+    if (q >= n_test) return;
+    const int u = t_user[q], it = t_item[q];
+    const int L = nb_len[it];
+    if (L == 0) { pred0[q] = -1.0; pred1[q] = -1.0; return; }        // `iid not in sim_bd.value.keys()` -> ()
+    const ListRecords recs{prof_item, prof_rating, prof_ts, prof_ptr[u], prof_ptr[u + 1]};
+    double p0, p1;
+    if (rs_predict_raw(recs, it, L, info, nb_idx, nb_sim, K, alpha, p0, p1)) atomicExch(error_flag, 4);
     pred0[q] = rs_bound_rating(p0); pred1[q] = rs_bound_rating(p1);
+}
+
+// ---- top-N recommendation: every user's first n items by the prediction before bound_rating (score descending, then
+// the smaller item index; -0.0 equals 0.0; a NaN score is never recommended) among the items with a neighbour list
+// that the user has no record on.  Only the items that list one of the user's items as a neighbour (the overlap
+// candidates, found through the reverse index rev) can score anything but their average; each is scored once, by
+// rs_predict_raw, when first seen.  The others score avg_i and come from `fallback`, the items with neighbours sorted by
+// (avg desc, index asc), merged last.  Both shapes keep their lists in registers: nothing per candidate goes to HBM.
+constexpr unsigned FULL = 0xffffffffu;
+constexpr int TOPN_SET_LG = 12;                         // warp shape: hash set of 4096 item slots per warp
+constexpr int TOPN_WARPS = 2;                           // warps per block of the warp shape (2 x 16 KB)
+constexpr int TOPN_CTA_WARPS = 8;
+constexpr int TOPN_TILE_ITEMS = 1 << 19;                // CTA shape: one bitmap bit per item of a tile (64 KB)
+static_assert(XMAP_TOPN_WARP_BOUND * 2 <= (1 << TOPN_SET_LG), "the warp shape's hash set stays at most half full");
+
+__device__ __forceinline__ bool rs_before(double sa, int ia, double sb, int ib) {
+    return sa > sb || (sa == sb && ia < ib);
+}
+
+// The running top-n (n <= 64) of one warp: position p is held by lane p & 31 in slot p >> 5; (ts, ti) is the n-th
+// entry once the list is full.  Every lane calls every member with the same arguments, except offer's own candidate.
+struct WarpTopN {
+    double s0, s1, ts;
+    int i0, i1, ti, cnt, n;
+
+    __device__ __forceinline__ void init(int n_) { s0 = s1 = ts = 0.0; i0 = i1 = ti = -1; cnt = 0; n = n_; }
+    __device__ __forceinline__ bool admits(double s, int i) const { return cnt < n || rs_before(s, i, ts, ti); }
+
+    __device__ __forceinline__ void insert(double s, int i, int lane) {
+        const int pos = __popc(__ballot_sync(FULL, lane < cnt && rs_before(s0, i0, s, i))) +
+                        __popc(__ballot_sync(FULL, lane + 32 < cnt && rs_before(s1, i1, s, i)));
+        if (pos >= n) return;
+        const double u0 = __shfl_up_sync(FULL, s0, 1), u1 = __shfl_up_sync(FULL, s1, 1), c = __shfl_sync(FULL, s0, 31);
+        const int j0 = __shfl_up_sync(FULL, i0, 1), j1 = __shfl_up_sync(FULL, i1, 1), ci = __shfl_sync(FULL, i0, 31);
+        if (lane > pos) { s0 = u0; i0 = j0; } else if (lane == pos) { s0 = s; i0 = i; }
+        if (lane + 32 > pos) { s1 = lane ? u1 : c; i1 = lane ? j1 : ci; } else if (lane + 32 == pos) { s1 = s; i1 = i; }
+        cnt = min(cnt + 1, n);
+        if (cnt == n) {
+            ts = __shfl_sync(FULL, n > 32 ? s1 : s0, (n - 1) & 31);
+            ti = __shfl_sync(FULL, n > 32 ? i1 : i0, (n - 1) & 31);
+        }
+    }
+
+    // each lane may hold one candidate (has); the admitted ones go in one at a time
+    __device__ __forceinline__ void offer(bool has, double s, int i, int lane) {
+        unsigned m = __ballot_sync(FULL, has && admits(s, i));
+        while (m) {
+            const int src = __ffs(m) - 1;
+            m &= m - 1;
+            insert(__shfl_sync(FULL, s, src), __shfl_sync(FULL, i, src), lane);
+        }
+    }
+
+    __device__ __forceinline__ void store(int32_t *idx, double *score, int32_t *len, int lane) const {
+        const double nan = __longlong_as_double(0x7FF8000000000000ll);
+        if (lane < n) { idx[lane] = lane < cnt ? i0 : -1; score[lane] = lane < cnt ? s0 : nan; }
+        if (lane + 32 < n) { idx[lane + 32] = lane + 32 < cnt ? i1 : -1; score[lane + 32] = lane + 32 < cnt ? s1 : nan; }
+        if (lane == 0) *len = cnt;
+    }
+};
+
+struct TopNArgs {
+    const int64_t *prof_ptr; const int32_t *item; const double *rating; const int64_t *ts;
+    const double *info; const int32_t *nb_idx; const double *nb_sim; const int32_t *nb_len; int K, n_items;
+    const int64_t *rev_ptr; const int32_t *rev_item; const int32_t *fallback; int n_fallback;
+    int n; double alpha; int decay;
+    int32_t *out_idx; double *out_score; int32_t *out_len; unsigned long long *stats; int32_t *error_flag;
+};
+
+__device__ __forceinline__ SortedRecords rs_user_records(const TopNArgs &a, int u) {
+    return SortedRecords{a.item, a.rating, a.ts, a.prof_ptr[u], a.prof_ptr[u + 1]};
+}
+
+// An overlap candidate seen for the first time: false if the user rated it; else its score (NaN when it has none).
+__device__ __forceinline__ bool rs_score_candidate(const TopNArgs &a, const SortedRecords &recs, int i, double &s) {
+    if (recs.has(i)) return false;
+    double p0, p1;
+    if (rs_predict_raw(recs, i, a.nb_len[i], a.info, a.nb_idx, a.nb_sim, a.K, a.alpha, p0, p1)) atomicExch(a.error_flag, 4);
+    s = a.decay ? p1 : p0;
+    return true;
+}
+
+// Merge the avg_i order: fallback items the user rated, or that have a neighbour the user rated (overlap candidates,
+// already scored), are skipped; the walk ends at the first item the list does not admit, since every later one comes
+// after it -- at most n + |overlap| + |records| steps.
+__device__ __forceinline__ void rs_merge_fallback(const TopNArgs &a, const SortedRecords &recs, WarpTopN &t, int lane) {
+    for (int base = 0; base < a.n_fallback; base += 32) {
+        const int g = base + lane;
+        const int i = g < a.n_fallback ? a.fallback[g] : -1;
+        const double avg = i >= 0 ? a.info[3 * (size_t)i] : 0.0;
+        const bool ok = i >= 0 && t.admits(avg, i);
+        const bool end = __ballot_sync(FULL, !ok) != 0u;
+        bool has = ok && !recs.has(i);
+        for (int r = 0; has && r < a.nb_len[i]; ++r) has = !recs.has(a.nb_idx[(size_t)i * a.K + r]);
+        t.offer(has, avg, i, lane);
+        if (end) break;
+    }
+}
+
+__device__ __forceinline__ void rs_add_stats(const TopNArgs &a, unsigned long long visits, unsigned long long cands) {
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) cands += __shfl_xor_sync(FULL, cands, off);
+    if ((threadIdx.x & 31) == 0) { atomicAdd(a.stats, visits); atomicAdd(a.stats + 1, cands); }
+}
+
+// Warp shape: one warp per user whose bound sum_{j in P_u} |rev(j)| is at most XMAP_TOPN_WARP_BOUND; the overlap
+// candidates are deduplicated in a shared-memory hash set (open addressing, at most half full).
+__global__ void __launch_bounds__(32 * TOPN_WARPS) recsim_topn_warp_kernel(TopNArgs a, const int32_t *__restrict__ users, int n_users) {
+    __shared__ int set[TOPN_WARPS][1 << TOPN_SET_LG];
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const int q = blockIdx.x * TOPN_WARPS + w;
+    if (q >= n_users) return;
+    const int u = users[q];
+    const SortedRecords recs = rs_user_records(a, u);
+    // the visits of this user (repeated items skipped) size the set: at least twice as many slots
+    unsigned long long visits = 0, cands = 0;
+    for (int64_t e = recs.lo + lane; e < recs.hi; e += 32) {
+        const int j = recs.item[e];
+        if (e == recs.lo || recs.item[e - 1] != j) visits += a.rev_ptr[j + 1] - a.rev_ptr[j];
+    }
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) visits += __shfl_xor_sync(FULL, visits, off);
+    int lg = 5;
+    while (lg < TOPN_SET_LG && (1ull << lg) < 2 * visits) ++lg;
+    int *hs = set[w];
+    for (int s = lane; s < (1 << lg); s += 32) hs[s] = -1;
+    __syncwarp();
+    WarpTopN t;
+    t.init(a.n);
+    for (int64_t e = recs.lo; e < recs.hi; ++e) {
+        const int j = recs.item[e];
+        if (e > recs.lo && recs.item[e - 1] == j) continue;            // a repeated item lists the same candidates
+        const int64_t lo = a.rev_ptr[j], hi = a.rev_ptr[j + 1];
+        for (int64_t base = lo; base < hi; base += 32) {
+            bool has = false;
+            double s = 0.0;
+            int i = -1;
+            if (base + lane < hi) {
+                i = a.rev_item[base + lane];
+                unsigned h = ((unsigned)i * 2654435761u) >> (32 - lg);
+                int old;
+                while ((old = atomicCAS(hs + h, -1, i)) != -1 && old != i) h = (h + 1) & ((1u << lg) - 1);
+                if (old == -1 && rs_score_candidate(a, recs, i, s)) { ++cands; has = s == s; }
+            }
+            t.offer(has, s, i, lane);
+        }
+    }
+    rs_merge_fallback(a, recs, t, lane);
+    t.store(a.out_idx + (size_t)u * a.n, a.out_score + (size_t)u * a.n, a.out_len + u, lane);
+    rs_add_stats(a, lane == 0 ? visits : 0, cands);
+}
+
+// CTA shape: one CTA per heavier user; the overlap candidates are deduplicated in a shared-memory bitmap over the item
+// axis, one tile of at most TOPN_TILE_ITEMS items at a time (rev lists are sorted by item, so a tile's part of each is
+// one binary search away).  Each warp keeps its own list; warp 0 merges them, then the avg_i order.
+__global__ void __launch_bounds__(32 * TOPN_CTA_WARPS, 1) recsim_topn_cta_kernel(TopNArgs a, const int32_t *__restrict__ users, int tile) {
+    extern __shared__ unsigned bm[];
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const int u = users[blockIdx.x];
+    const SortedRecords recs = rs_user_records(a, u);
+    WarpTopN t;
+    t.init(a.n);
+    unsigned long long visits = 0, cands = 0;
+    for (int t0 = 0; t0 < a.n_items; t0 += tile) {
+        const int t1 = min(a.n_items, t0 + tile);
+        for (int s = threadIdx.x; s < (t1 - t0 + 31) / 32; s += blockDim.x) bm[s] = 0u;
+        __syncthreads();
+        for (int64_t e = recs.lo + w; e < recs.hi; e += TOPN_CTA_WARPS) {
+            const int j = recs.item[e];
+            if (e > recs.lo && recs.item[e - 1] == j) continue;
+            int64_t lo = a.rev_ptr[j], hi = a.rev_ptr[j + 1];
+            if (tile < a.n_items) { lo = rs_lower_bound(a.rev_item, lo, hi, t0); hi = rs_lower_bound(a.rev_item, lo, hi, t1); }
+            visits += hi - lo;
+            for (int64_t base = lo; base < hi; base += 32) {
+                bool has = false;
+                double s = 0.0;
+                int i = -1;
+                if (base + lane < hi) {
+                    i = a.rev_item[base + lane];
+                    const unsigned bit = 1u << ((i - t0) & 31);
+                    if (!(atomicOr(bm + ((i - t0) >> 5), bit) & bit) && rs_score_candidate(a, recs, i, s)) { ++cands; has = s == s; }
+                }
+                t.offer(has, s, i, lane);
+            }
+        }
+        __syncthreads();
+    }
+    rs_add_stats(a, lane == 0 ? visits : 0, cands);
+    double *ms = reinterpret_cast<double *>(bm);                // the warps' lists, in the bitmap's place
+    int *mi = reinterpret_cast<int *>(ms + TOPN_CTA_WARPS * 64), *mc = mi + TOPN_CTA_WARPS * 64;
+    ms[w * 64 + lane] = t.s0; ms[w * 64 + lane + 32] = t.s1;
+    mi[w * 64 + lane] = t.i0; mi[w * 64 + lane + 32] = t.i1;
+    if (lane == 0) mc[w] = t.cnt;
+    __syncthreads();
+    if (w != 0) return;
+    for (int v = 1; v < TOPN_CTA_WARPS; ++v)
+        for (int p = lane; p < 64; p += 32) t.offer(p < mc[v], ms[v * 64 + p], mi[v * 64 + p], lane);
+    rs_merge_fallback(a, recs, t, lane);
+    t.store(a.out_idx + (size_t)u * a.n, a.out_score + (size_t)u * a.n, a.out_len + u, lane);
 }
 
 
@@ -420,6 +668,35 @@ extern "C" int xmap_recsim_predict(const int64_t *prof_ptr, const int32_t *prof_
         prof_ptr, prof_item, prof_rating, prof_ts, info, nb_idx, nb_sim, nb_len, k, t_user, t_item, n_test, alpha,
         pred_nodecay, pred_decay, error_flag);
     XMAP_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int xmap_recsim_top_n(const int64_t *prof_ptr, const int32_t *prof_item, const double *prof_rating,
+                                 const int64_t *prof_ts, const double *info, const int32_t *nb_idx, const double *nb_sim,
+                                 const int32_t *nb_len, int32_t k, int32_t n_items, const int64_t *rev_ptr,
+                                 const int32_t *rev_item, const int32_t *fallback, int32_t n_fallback,
+                                 const int32_t *warp_users, int32_t n_warp_users, const int32_t *cta_users,
+                                 int32_t n_cta_users, int32_t n, double alpha, int32_t decay, int32_t *out_idx,
+                                 double *out_score, int32_t *out_len, unsigned long long *stats, int32_t *error_flag,
+                                 void *stream_) {
+    if (n < 1 || n > XMAP_TOPN_MAX) return fail_msg("xmap_recsim_top_n: n out of [1, 64]");
+    if (n_warp_users < 0 || n_cta_users < 0 || n_items < 0 || n_fallback < 0) return fail_msg("xmap_recsim_top_n: negative size");
+    const TopNArgs a{prof_ptr, prof_item, prof_rating, prof_ts, info, nb_idx, nb_sim, nb_len, k, n_items, rev_ptr, rev_item,
+                     fallback, n_fallback, n, alpha, decay, out_idx, out_score, out_len, stats, error_flag};
+    cudaStream_t st = (cudaStream_t)stream_;
+    if (n_warp_users > 0) {
+        recsim_topn_warp_kernel<<<(unsigned)((n_warp_users + TOPN_WARPS - 1) / TOPN_WARPS), 32 * TOPN_WARPS, 0, st>>>(
+            a, warp_users, n_warp_users);
+        XMAP_LAUNCH_CHECK();
+    }
+    if (n_cta_users > 0) {
+        const int tile = min(n_items, TOPN_TILE_ITEMS);
+        const size_t merge = TOPN_CTA_WARPS * 64 * (sizeof(double) + sizeof(int)) + TOPN_CTA_WARPS * sizeof(int);
+        const size_t smem = max((size_t)(tile + 31) / 32 * sizeof(unsigned), merge);
+        XMAP_CUDA(cudaFuncSetAttribute(recsim_topn_cta_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        recsim_topn_cta_kernel<<<(unsigned)n_cta_users, 32 * TOPN_CTA_WARPS, smem, st>>>(a, cta_users, max(tile, 1));
+        XMAP_LAUNCH_CHECK();
+    }
     return 0;
 }
 

@@ -353,3 +353,104 @@ def predict(user, item, rating, ts, n_users, rs, nb, test_user, test_item, test_
             mae0 = float((tr[ok] - p0[ok]).abs().sum().item()) / cnt          # recommenderPrediction.py:116-139
             mae1 = float((tr[ok] - p1[ok]).abs().sum().item()) / cnt
     return p0, p1, mae0, mae1
+
+
+@dataclass
+class TopN:
+    """top_n's result: every user's list, and what the kernels did for the users this process ran."""
+    idx: torch.Tensor        # int32 [n_users, n], -1 padded
+    score: torch.Tensor      # f64   [n_users, n], NaN padded: the prediction before bound_rating
+    len: torch.Tensor        # int32 [n_users]
+    visits: int              # reverse-index entries visited
+    candidates: int          # distinct overlap candidates scored or found NaN
+    warp_users: int          # users of the one-warp shape
+    cta_users: int           # users of the one-CTA shape
+
+
+def reverse_index(nb):
+    """For every item j the items i that list j as a neighbour, ascending: (rev_ptr int64 [n_items + 1], rev_item int32).
+    One sort of the (neighbour, item) keys."""
+    n_items, k = int(nb.idx.shape[0]), int(nb.idx.shape[1])
+    dev = nb.idx.device
+    valid = torch.arange(k, device=dev).unsqueeze(0) < nb.len.long().unsqueeze(1)
+    j = nb.idx.long()[valid]
+    i = torch.arange(n_items, device=dev).unsqueeze(1).expand(n_items, k)[valid]
+    key = torch.sort(j * n_items + i).values
+    rev_ptr = torch.zeros(n_items + 1, dtype=torch.int64, device=dev)
+    rev_ptr[1:] = torch.cumsum(torch.bincount(j, minlength=n_items), 0)
+    return rev_ptr, (key % max(n_items, 1)).to(torch.int32).contiguous()
+
+
+def top_n(user, item, rating, ts, n_users, knn, nb, n, decay=False, alpha=0.03, shard=False, group=None):
+    """Every user's first n items (1 <= n <= 64) by the item-based prediction BEFORE bound_rating
+    (recommenderPrediction.py:26-103, the value predict rounds), without or with temporal decay.  The reference has
+    no such function.  Candidates are the items with a neighbour list the user has no record on (real and synthetic
+    records alike); order: score descending, then the smaller item index (-0.0 equals 0.0); a NaN score is never
+    recommended.  An item none of whose neighbours the user rated scores its average, so a user without records gets
+    the top of the average order, and a user with fewer than n candidates a shorter list.
+
+    user / item / rating / ts: the profile records in list order; knn: an ItemKnn or a RecSim (its item info is read);
+    nb: the neighbour tables (any k).  shard: split the users over the ranks of `group` (torch.distributed; every rank
+    passes the whole profile and tables) in contiguous blocks of equal work; one all-gather then gives every rank
+    every list.  The result does not depend on the launch shape, the tiling of the item axis or the world size.
+    Raises NativeError (error 4) when a candidate gathers more than 128 matching profile records, as predict does."""
+    if isinstance(n, bool) or int(n) != n or not 1 <= int(n) <= N.TOPN_MAX:
+        raise ValueError("n must be an integer in [1, %d], got %r" % (N.TOPN_MAX, n))
+    n = int(n)
+    L = N.lib()
+    dev = knn.info.device
+    n_items = int(nb.idx.shape[0])
+    # checked in int64 before the narrowing copies: the kernels index the profile by user and the tables by item
+    user = torch.as_tensor(user, dtype=torch.int64).to(dev).flatten()
+    item = torch.as_tensor(item, dtype=torch.int64).to(dev).flatten()
+    n_rec = int(user.numel())
+    if int(item.numel()) != n_rec:
+        raise ValueError("user and item differ in length (%d, %d)" % (n_rec, int(item.numel())))
+    if n_users < 0 or (n_rec and (int(user.min()) < 0 or int(user.max()) >= n_users)):
+        raise ValueError("user outside [0, %d)" % n_users)
+    if n_rec and (int(item.min()) < 0 or int(item.max()) >= n_items):
+        raise ValueError("item outside [0, %d)" % n_items)
+    # the records grouped by user, stably by item inside each user: a candidate's entries are runs in list order
+    o = torch.argsort(user * n_items + item, stable=True)
+    prof_ptr = torch.zeros(n_users + 1, dtype=torch.int64, device=dev)
+    prof_ptr[1:] = torch.cumsum(torch.bincount(user, minlength=n_users), 0)
+    p_item = item[o].to(torch.int32).contiguous()
+    p_rating = torch.as_tensor(rating, dtype=torch.float64).to(dev).flatten()[o].contiguous()
+    p_ts = torch.as_tensor(ts, dtype=torch.int64).to(dev).flatten()[o].contiguous()
+    rev_ptr, rev_item = reverse_index(nb)
+    # per user: sum over its records j of |rev(j)|, the bound on the overlap candidates it visits (one scatter-add)
+    bound = torch.zeros(n_users, dtype=torch.int64, device=dev).index_add_(0, user, (rev_ptr[1:] - rev_ptr[:-1])[item])
+    sh = None
+    lo, hi = 0, n_users
+    if shard:
+        import torch.distributed as dist
+        from .multi import RowShard
+        sh = RowShard(bound, dist.get_rank(group), dist.get_world_size(group))
+        lo, hi = sh.lo, sh.hi
+    mine = torch.arange(lo, hi, dtype=torch.int64, device=dev)
+    light = bound[lo:hi] <= N.TOPN_WARP_BOUND
+    warp_users = mine[light].to(torch.int32).contiguous()
+    heavy = mine[~light]
+    cta_users = heavy[torch.argsort(bound[heavy], descending=True, stable=True)].to(torch.int32).contiguous()
+    # the items that score their average when unreached, by (average desc, index asc); + 0.0 makes -0.0 sort as 0.0
+    avg = knn.info[:, 0]
+    fb = torch.nonzero((nb.len > 0) & (avg == avg)).flatten()
+    fb = fb[torch.sort(avg[fb] + 0.0, descending=True, stable=True).indices].to(torch.int32).contiguous()
+    out_idx = torch.full((n_users, n), -1, dtype=torch.int32, device=dev)
+    out_score = torch.full((n_users, n), float("nan"), dtype=torch.float64, device=dev)
+    out_len = torch.zeros(n_users, dtype=torch.int32, device=dev)
+    stats = torch.zeros(2, dtype=torch.int64, device=dev)
+    err = torch.zeros(1, dtype=torch.int32, device=dev)
+    N.check(L.xmap_recsim_top_n(N.ptr(prof_ptr), N.ptr(p_item), N.ptr(p_rating), N.ptr(p_ts), N.ptr(knn.info.contiguous()),
+                                N.ptr(nb.idx.contiguous()), N.ptr(nb.sim.contiguous()), N.ptr(nb.len.contiguous()),
+                                int(nb.idx.shape[1]), n_items, N.ptr(rev_ptr), N.ptr(rev_item), N.ptr(fb), int(fb.numel()),
+                                N.ptr(warp_users), int(warp_users.numel()), N.ptr(cta_users), int(cta_users.numel()), n,
+                                float(alpha), 1 if decay else 0, N.ptr(out_idx), N.ptr(out_score), N.ptr(out_len),
+                                N.ptr(stats), N.ptr(err), _st()), "xmap_recsim_top_n")
+    if int(err.item()):
+        raise N.NativeError("top-N kernel error %d (4: more than 128 matching profile records)" % int(err.item()))
+    if sh is not None:
+        from .multi import allgather_rows
+        allgather_rows([out_idx, out_score, out_len], sh, group)
+    visits, cands = stats.tolist()
+    return TopN(out_idx, out_score, out_len, visits, cands, int(warp_users.numel()), int(cta_users.numel()))
