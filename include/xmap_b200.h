@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define XMAP_B200_ABI_VERSION 11
+#define XMAP_B200_ABI_VERSION 12
 #define XMAP_KMAX 64                 /* largest supported top-k (extend_among_topk) */
 #define XMAP_METHOD_ADJUST_COSINE 0  /* baselinerSim.py:144-174 */
 #define XMAP_METHOD_COSINE 1         /* baselinerSim.py:115-142 */
@@ -382,6 +382,20 @@ int xmap_recsim_top_n(const int64_t *prof_ptr, const int32_t *prof_item, const d
                       int32_t n_fallback, const int32_t *warp_users, int32_t n_warp_users, const int32_t *cta_users,
                       int32_t n_cta_users, int32_t n, double alpha, int32_t decay, int32_t *out_idx, double *out_score,
                       int32_t *out_len, unsigned long long *stats, int32_t *error_flag, void *stream);
+
+/* (5e) Ranking metrics of top-N lists against held-out relevant items (the reference has no ranking metrics; the
+ * definitions are the project's, DESIGN.md section 3.6).  One warp per evaluated user q (user index users[q]):
+ *   top_idx [*][width], top_len: the lists of xmap_recsim_top_n; the first l = min(top_len[u], n) slots count;
+ *   rel_ptr [n_users + 1], rel_item: user q's relevant items, sorted ascending and unique, at least one per user (an
+ *       item no list can hold, e.g. one without a neighbour list, still counts in |R|);
+ *   disc [XMAP_TOPN_MAX]: disc[p] = 1 / log2(p + 2), computed by the caller;
+ *   hits[q] = #hits in slots < l; precision = hits / n; recall = hits / |R|;
+ *   ndcg = sum_{p < l, hit} disc[p] / sum_{p < min(n, |R|)} disc[p];
+ *   ap = sum_{p < l, hit} (hits in slots 0..p) / (p + 1) / min(n, |R|);
+ * every sum formed in slot order. */
+int xmap_recsim_rank_metrics(const int32_t *top_idx, const int32_t *top_len, int32_t width, const int32_t *users,
+                             int32_t n_users, const int64_t *rel_ptr, const int32_t *rel_item, const double *disc, int32_t n,
+                             int32_t *hits, double *precision, double *recall, double *ndcg, double *ap, void *stream);
 
 /* (5c) PRIVATE neighbour selection + noise perturbation (RecommenderPrivacy.private_neighbor_selection +
  * noise_perturbation, recommenderPrivacy.py:35-139, 152-171) as the reference behaves under Python 3 (one neighbour per

@@ -14,7 +14,7 @@ KMAX = 64
 XSIM_MAX_CELLS_LG = 13    # XMAP_XSIM_MAX_CELLS_LG
 METHODS = {"adjust_cosine": 0, "cosine": 1}
 SELECT_LONG = 8192            # XMAP_SELECT_LONG
-ABI_VERSION = 11
+ABI_VERSION = 12
 ROW_HDR_BYTES = 48          # XMAP_SIM_ROW_HDR_BYTES
 INGEST_ID_MAX = 48          # XMAP_INGEST_ID_MAX
 TOPN_MAX = 64               # XMAP_TOPN_MAX
@@ -85,6 +85,8 @@ _SIGS = {
     "xmap_recsim_top_n": (C.c_int, [_p, _p, _p, _p, _p, _p, _p, _p, C.c_int32, C.c_int32, _p, _p, _p, C.c_int32,
                                     _p, C.c_int32, _p, C.c_int32, C.c_int32, C.c_double, C.c_int32, _p, _p, _p, _p, _p,
                                     _p]),
+    "xmap_recsim_rank_metrics": (C.c_int, [_p, _p, C.c_int32, _p, C.c_int32, _p, _p, _p, C.c_int32, _p, _p, _p, _p, _p,
+                                           _p]),
     "xmap_recsim_private_neighbor": (C.c_int, [_p, _p, _p, _p, C.c_int32, C.c_int32, C.c_double, C.c_double, _p, _p, C.c_uint64,
                                                _p, _p, _p, _p, _p]),
     "xmap_clean_records": (C.c_int, [_p, _p, _p, _p, C.c_int64, C.c_int32, C.c_double, C.c_double, C.c_int32, _p, _p, _p]),

@@ -82,6 +82,14 @@ class Generator(object):
         return LocalRDD(alterego_records(sess, torch.as_tensor(mp).to(sess.device)))
 
 
+def alterego_mapping(privatemap_tool, sess, extended_simRDD, private):
+    """The {source: target} item map generator_pipeline applies (assist.py:136-150): [n_items] int32 on the device,
+    -1 for an unmapped item.  private selects the tool's private_mode, else the non-private mapping."""
+    mode = privatemap_tool.private_mode if private else "nonprivate"
+    xres, chosen = privatemap_tool._map(extended_simRDD, sess, mode)
+    return G.invert_mapping(xres.start_item, chosen, sess.enc.n_items)
+
+
 def alterego_records(sess, mapping):
     enc = sess.enc
     ou, oi, orr, ot = G.build_alterego(sess.layout, np.arange(len(enc.user), dtype=np.int64), mapping)

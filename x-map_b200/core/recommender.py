@@ -39,6 +39,18 @@ class ProfileState(object):
         self.knn = None          # recsim.ItemKnn: item info and the neighbour tables
         self.nb = None           # recsim.Neighbors
 
+    @classmethod
+    def from_arrays(cls, user, item, rating, ts, uids, iids):
+        """The profile as device arrays (list order; user / item index the sorted id arrays uids / iids, which may
+        hold ids without records), for the array-level pipeline (evaluate.py).  No Python object per record, so the
+        string-keyed lookups of item_based_recommendation are not available on it."""
+        self = cls.__new__(cls)
+        self.records, self.upos, self.ipos = None, None, None
+        self.uids, self.iids = uids, iids
+        self.user, self.item, self.rating, self.ts = user, item, rating, ts
+        self.num_atleast = self.knn = self.nb = None
+        return self
+
 
 class HandleDict(dict):
     """A plain dict for callers, plus the device state for the next pipeline stage."""

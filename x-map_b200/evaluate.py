@@ -1,0 +1,141 @@
+"""Held-out evaluation of the two-domain experiment on the device: the test split of ingest_arrays against the item-based
+predictions (MAE) and the top-N lists (precision, recall, NDCG, MAP at n, coverage) of the AlterEgo profile.
+
+    A = ingest.ingest_arrays(clean_source, clean_target, split_tool, path_source, path_target, False)
+    ev = evaluate.evaluate(A, sim_tool, extend_tool, generator, private_gen, rec_sim_tool, privacy_tool, private_rec)
+
+The tools are the facade chain's (BaselinerSim, ExtendSim, Generator, RecommenderSim, RecommenderPrivacy), so every
+parameter, private mode and seed means what it means there, and the predictions, the MAE and the lists equal those of
+clean_split_pipeline -> ... -> recommender_prediction_pipeline / recommend_top_n (with the time zone at UTC: the
+facade turns times into local datetimes and back with timegm).  Every array stays on the device; no Python object is
+made per record.  The reference has no ranking metrics: their definitions are in DESIGN.md section 3.6."""
+from dataclasses import dataclass
+
+import torch
+
+from . import generate as G
+from . import ingest as I
+from . import recsim as RS
+from .core.baselinerSim import SimHandle
+from .core.generator import alterego_mapping
+from .core.recommender import ProfileState, recommender_privacy_pipeline
+from .session import Session
+
+
+@dataclass
+class Evaluation:
+    """evaluate's result.  Held-out pairs follow A.test_* order; evaluated users are ids of A.all_uids."""
+    mae_nodecay: float           # None when no pair was predicted
+    mae_decay: float
+    pred_nodecay: torch.Tensor   # f64 [n_test] bounded prediction, -1 where the pair was skipped
+    pred_decay: torch.Tensor
+    users: torch.Tensor          # int64 [n_eval] all_uids index of each evaluated user
+    metrics: RS.RankMetrics      # per evaluated user, the means and the coverage
+    top: RS.TopN                 # rows indexed by train user; items index profile_items
+    profile_items: torch.Tensor  # int64: train item index of every profile item (profile item index = position)
+    n: int
+    counts: dict
+    stage_ms: dict               # device time per stage when events were passed, else None
+
+
+def evaluate(A, sim_tool, extend_tool, generator, private_gen, rec_sim_tool, privacy_tool, private_rec, n=10,
+             threshold=None, alpha=0.03, events=None):
+    """Train arrays -> similarity -> X-SIM -> mapping -> AlterEgo profile -> item-kNN, then the held-out MAE of the
+    test pairs and the top-n accuracy of the test users.  private_gen / private_rec: the generator's private mode and
+    the private neighbour selection, as generator_pipeline's and recommender_privacy_pipeline's flags.  threshold: a
+    held-out record is relevant when its rating >= threshold (None: every one).  events: optional dict that receives
+    CUDA-event pairs per stage; their times are then in stage_ms."""
+    dev = A.user.device
+    timer = I._Timer(events)
+    counts = {}
+    if sim_tool.method not in ("cosine", "adjust_cosine"):
+        raise ValueError("unknown similarity method %r" % (sim_tool.method,))
+    if A.train_user_of is None or A.train_item_of is None:
+        raise ValueError("the arrays carry no train index maps (train_user_of / train_item_of)")
+
+    # ---- AlterEgo profile, in the facade's list order: target records in training order, then the synthetic ones ----
+    with timer("session"):
+        sess = Session(I.encoded(A), dev, user=A.user, item=A.item, rating=A.rating, meta=A.meta)
+    with timer("similarity_xsim"):
+        xs = extend_tool.extend(SimHandle(sess, sim_tool.method, sim_tool.num_atleast))
+    with timer("alterego"):
+        mapping = alterego_mapping(generator, sess, xs, private_gen)
+        ou, oi, orr, ot = G.build_alterego(sess.layout, torch.arange(sess.layout.nnz, device=dev), mapping)
+        keep = A.meta.has_T[A.item.long()]
+        pu = torch.cat([A.user.long()[keep], ou.long()])
+        pi = torch.cat([A.item.long()[keep], oi.long()])
+        pr = torch.cat([A.rating[keep], orr])
+        pt = torch.floor(torch.cat([A.ts[keep], A.ts[ot.long()]])).long()      # timegm of the facade's datetimes
+        # profile items numbered by rank among the items present, as the facade's np.unique over id strings does (the
+        # private selection draws per item index); users keep the train numbering (only their order matters)
+        profile_items, pi = torch.unique(pi, return_inverse=True)
+        n_users, n_items = len(A.uids), int(profile_items.numel())
+    counts["profile_records"], counts["synthetic_records"] = int(pu.numel()), int(ou.numel())
+    del sess, xs, mapping, ou, oi, orr, ot
+
+    with timer("item_knn"):
+        state = ProfileState.from_arrays(pu, pi, pr, pt, A.uids, A.iids[profile_items.cpu().numpy()])
+        recommender_privacy_pipeline(privacy_tool, rec_sim_tool.calculate_sim(state), private_rec)
+        knn, nb = state.knn, state.nb
+
+    # ---- held-out pairs -> train numbering -> profile numbering ----------------------------------------------------
+    with timer("prediction"):
+        n_test = int(A.test_user.numel())
+        in_prof_user = torch.bincount(pu, minlength=n_users) > 0
+        prof_of = torch.full((len(A.iids),), -1, dtype=torch.int64, device=dev)
+        prof_of[profile_items] = torch.arange(n_items, device=dev)
+        tu = A.train_user_of[A.test_user.long()].long()
+        ti = A.train_item_of[A.test_item.long()].long()
+        untrained = (tu < 0) | (ti < 0)
+        tpi = torch.where(untrained, -1, prof_of[ti.clamp(min=0)])
+        no_profile = ~untrained & ((tpi < 0) | ~in_prof_user[tu.clamp(min=0)])
+        ok = torch.nonzero(~untrained & ~no_profile).flatten()
+        p0, p1, mae0, mae1 = RS.predict(pu, pi, pr, pt, n_users, knn, nb, tu[ok], tpi[ok], A.test_rating[ok], alpha)
+        pred0 = torch.full((n_test,), -1.0, dtype=torch.float64, device=dev)
+        pred1 = torch.full((n_test,), -1.0, dtype=torch.float64, device=dev)
+        pred0[ok], pred1[ok] = p0, p1
+        n_pred = int((p0 >= 0).sum())
+    counts.update(test_pairs=n_test, predicted=n_pred, skipped_untrained=int(untrained.sum()),
+                  skipped_no_profile=int(no_profile.sum()), skipped_no_neighbours=int(ok.numel()) - n_pred)
+
+    # ---- top-n of the test users with a relevant held-out record -----------------------------------------------------
+    with timer("top_n"):
+        rel = torch.ones(n_test, dtype=torch.bool, device=dev) if threshold is None else A.test_rating >= threshold
+        is_test = torch.zeros(len(A.all_uids), dtype=torch.bool, device=dev)
+        is_test[torch.from_numpy(A.test_users).to(dev)] = True
+        rel &= is_test[A.test_user.long()]
+        has_rel = torch.zeros(len(A.all_uids), dtype=torch.bool, device=dev)
+        has_rel[A.test_user.long()[rel]] = True
+        trained = A.train_user_of >= 0
+        users = torch.nonzero(has_rel & trained).flatten()          # ascending all_uids index
+        run = A.train_user_of[users].long()
+        top = RS.top_n(pu, pi, pr, pt, n_users, knn, nb, n, alpha=alpha, users=run)
+    with timer("rank_metrics"):
+        # relevant items in profile numbering; an item outside the profile gets a code past every profile item
+        q_of = torch.full((len(A.all_uids),), -1, dtype=torch.int64, device=dev)
+        q_of[users] = torch.arange(int(users.numel()), device=dev)
+        rq = q_of[A.test_user.long()[rel]]
+        keep_r = rq >= 0
+        rq, ri_all = rq[keep_r], A.test_item.long()[rel][keep_r]
+        rti = A.train_item_of[ri_all].long()
+        code = torch.where(rti >= 0, prof_of[rti.clamp(min=0)], -1)
+        code = torch.where(code >= 0, code, n_items + ri_all)
+        key = torch.unique(rq * (n_items + len(A.all_iids)) + code)
+        rq, code = key // (n_items + len(A.all_iids)), key % (n_items + len(A.all_iids))
+        rel_ptr = torch.zeros(int(users.numel()) + 1, dtype=torch.int64, device=dev)
+        rel_ptr[1:] = torch.cumsum(torch.bincount(rq, minlength=int(users.numel())), 0)
+        catalogue = int((nb.len > 0).sum())
+        metrics = RS.rank_metrics(top, run, rel_ptr, code, n, catalogue=catalogue)
+        reachable = torch.zeros(int(code.numel()), dtype=torch.bool, device=dev)
+        in_prof = code < n_items
+        reachable[in_prof] = nb.len[code[in_prof]] > 0
+    counts.update(eval_users=int(users.numel()), eval_users_without_profile=int((~in_prof_user[run]).sum()),
+                  test_users_untrained=int((has_rel & ~trained).sum()),
+                  test_users_without_relevant=int(len(A.test_users)) - int((has_rel & is_test).sum()),
+                  relevant_items=int(code.numel()), unreachable_items=int((~reachable).sum()),
+                  catalogue_items=catalogue)
+    stage_ms = None
+    if events is not None:
+        torch.cuda.synchronize(dev)
+        stage_ms = {k: sum(a.elapsed_time(b) for a, b in v) for k, v in events.items()}
+    return Evaluation(mae0, mae1, pred0, pred1, users, metrics, top, profile_items, n, counts, stage_ms)

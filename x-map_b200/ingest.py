@@ -106,7 +106,8 @@ class IngestArrays:
     the item codes of `iids`.  Test records index `all_uids` / `all_iids` (every id of the two files, sorted).
     train_users / train_ptr: the train RDD's records in order, record k = user all_uids[train_users[k]] with the
     train arrays [train_ptr[k], train_ptr[k+1]) (a test user may have none); test_users / test_ptr the same for
-    the test records."""
+    the test records.  train_user_of / train_item_of (int32, device): the train index of every id of all_uids /
+    all_iids, -1 for an id without training records."""
     user: torch.Tensor
     item: torch.Tensor
     rating: torch.Tensor
@@ -125,6 +126,8 @@ class IngestArrays:
     test_users: np.ndarray
     test_ptr: np.ndarray
     codes: dict = field(default_factory=dict)      # the item codes on the host (encode.item_codes names)
+    train_user_of: torch.Tensor = None
+    train_item_of: torch.Tensor = None
 
 
 # ---- reading and parsing -------------------------------------------------------------------------------------------
@@ -395,8 +398,10 @@ def ingest_arrays(clean_source, clean_target, split_tool, path_source, path_targ
         used_i = torch.zeros(n_items, dtype=torch.int32, device=dev)
         used_u[tu_all] = 1
         used_i[ti_all] = 1
-        user = (torch.cumsum(used_u, 0, dtype=torch.int32) - 1)[tu_all] if n_users else tu_all.int()
-        item = (torch.cumsum(used_i, 0, dtype=torch.int32) - 1)[ti_all] if n_items else ti_all.int()
+        user_of = torch.where(used_u > 0, torch.cumsum(used_u, 0, dtype=torch.int32) - 1, -1).to(torch.int32)
+        item_of = torch.where(used_i > 0, torch.cumsum(used_i, 0, dtype=torch.int32) - 1, -1).to(torch.int32)
+        user = user_of[tu_all] if n_users else tu_all.int()
+        item = item_of[ti_all] if n_items else ti_all.int()
         used_u_h, used_i_h = used_u.bool().cpu().numpy(), used_i.bool().cpu().numpy()
     n_train_items = int(used_i_h.sum())
     if n_train_items > MAX_ITEMS:
@@ -424,7 +429,8 @@ def ingest_arrays(clean_source, clean_target, split_tool, path_source, path_targ
                         test_ts=P.ts[test_line], uids=all_uids[used_u_h], iids=all_iids[used_i_h],
                         all_uids=all_uids, all_iids=all_iids, meta=meta,
                         train_users=train_users, train_ptr=ptr(train_users, tcount),
-                        test_users=test_users.astype(np.int64), test_ptr=ptr(test_users, ecount), codes=codes)
+                        test_users=test_users.astype(np.int64), test_ptr=ptr(test_users, ecount), codes=codes,
+                        train_user_of=user_of, train_item_of=item_of)
 
 
 # ---- RDD facade ----------------------------------------------------------------------------------------------------

@@ -6,6 +6,7 @@ assist.recommender_calculate_sim_pipeline (assist.py:153-175).
 """
 from dataclasses import dataclass
 
+import numpy as np
 import torch
 
 from . import _native as N
@@ -13,6 +14,7 @@ from . import _native as N
 # Peak device bytes per co-rating entry while a pass runs: key and record positions (16), the stable sort's keys,
 # permutation and scratch (~32), the permuted positions (8), rounded up for the pair outputs.
 ENTRY_BYTES = 64
+INT32_MAX = (1 << 31) - 1
 
 
 def _st():
@@ -381,7 +383,7 @@ def reverse_index(nb):
     return rev_ptr, (key % max(n_items, 1)).to(torch.int32).contiguous()
 
 
-def top_n(user, item, rating, ts, n_users, knn, nb, n, decay=False, alpha=0.03, shard=False, group=None):
+def top_n(user, item, rating, ts, n_users, knn, nb, n, decay=False, alpha=0.03, shard=False, group=None, users=None):
     """Every user's first n items (1 <= n <= 64) by the item-based prediction BEFORE bound_rating
     (recommenderPrediction.py:26-103, the value predict rounds), without or with temporal decay.  The reference has
     no such function.  Candidates are the items with a neighbour list the user has no record on (real and synthetic
@@ -393,6 +395,8 @@ def top_n(user, item, rating, ts, n_users, knn, nb, n, decay=False, alpha=0.03, 
     nb: the neighbour tables (any k).  shard: split the users over the ranks of `group` (torch.distributed; every rank
     passes the whole profile and tables) in contiguous blocks of equal work; one all-gather then gives every rank
     every list.  The result does not depend on the launch shape, the tiling of the item axis or the world size.
+    users: None for every user, or a 1-D integer tensor of distinct users in [0, n_users): only their rows are filled
+    (the others keep the padding), and the counts refer to them; shard then splits these users.
     Raises NativeError (error 4) when a candidate gathers more than 128 matching profile records, as predict does."""
     if isinstance(n, bool) or int(n) != n or not 1 <= int(n) <= N.TOPN_MAX:
         raise ValueError("n must be an integer in [1, %d], got %r" % (N.TOPN_MAX, n))
@@ -410,6 +414,17 @@ def top_n(user, item, rating, ts, n_users, knn, nb, n, decay=False, alpha=0.03, 
         raise ValueError("user outside [0, %d)" % n_users)
     if n_rec and (int(item.min()) < 0 or int(item.max()) >= n_items):
         raise ValueError("item outside [0, %d)" % n_items)
+    if users is None:
+        sel = torch.arange(max(n_users, 0), dtype=torch.int64, device=dev)
+    else:
+        sel = torch.as_tensor(users)
+        if sel.dim() != 1 or sel.dtype.is_floating_point or sel.dtype.is_complex or sel.dtype == torch.bool:
+            raise ValueError("users must be a 1-D integer tensor")
+        sel = sel.to(device=dev, dtype=torch.int64)
+        if sel.numel() and (int(sel.min()) < 0 or int(sel.max()) >= n_users):
+            raise ValueError("users outside [0, %d)" % n_users)
+        if int(torch.unique(sel).numel()) != int(sel.numel()):
+            raise ValueError("users must be distinct")
     # the records grouped by user, stably by item inside each user: a candidate's entries are runs in list order
     o = torch.argsort(user * n_items + item, stable=True)
     prof_ptr = torch.zeros(n_users + 1, dtype=torch.int64, device=dev)
@@ -421,14 +436,13 @@ def top_n(user, item, rating, ts, n_users, knn, nb, n, decay=False, alpha=0.03, 
     # per user: sum over its records j of |rev(j)|, the bound on the overlap candidates it visits (one scatter-add)
     bound = torch.zeros(n_users, dtype=torch.int64, device=dev).index_add_(0, user, (rev_ptr[1:] - rev_ptr[:-1])[item])
     sh = None
-    lo, hi = 0, n_users
+    mine = sel
     if shard:
         import torch.distributed as dist
         from .multi import RowShard
-        sh = RowShard(bound, dist.get_rank(group), dist.get_world_size(group))
-        lo, hi = sh.lo, sh.hi
-    mine = torch.arange(lo, hi, dtype=torch.int64, device=dev)
-    light = bound[lo:hi] <= N.TOPN_WARP_BOUND
+        sh = RowShard(bound[sel], dist.get_rank(group), dist.get_world_size(group))
+        mine = sel[sh.lo:sh.hi]
+    light = bound[mine] <= N.TOPN_WARP_BOUND
     warp_users = mine[light].to(torch.int32).contiguous()
     heavy = mine[~light]
     cta_users = heavy[torch.argsort(bound[heavy], descending=True, stable=True)].to(torch.int32).contiguous()
@@ -451,6 +465,81 @@ def top_n(user, item, rating, ts, n_users, knn, nb, n, decay=False, alpha=0.03, 
         raise N.NativeError("top-N kernel error %d (4: more than 128 matching profile records)" % int(err.item()))
     if sh is not None:
         from .multi import allgather_rows
-        allgather_rows([out_idx, out_score, out_len], sh, group)
+        if users is None:
+            allgather_rows([out_idx, out_score, out_len], sh, group)
+        else:                                   # the selected rows side by side, in the order of `users`
+            rows = [out_idx[sel], out_score[sel], out_len[sel]]
+            allgather_rows(rows, sh, group)
+            out_idx[sel], out_score[sel], out_len[sel] = rows
     visits, cands = stats.tolist()
     return TopN(out_idx, out_score, out_len, visits, cands, int(warp_users.numel()), int(cta_users.numel()))
+
+
+# 1 / log2(p + 2) for the list slots, computed on the host so that no device log2 enters a metric
+DISCOUNT = 1.0 / np.log2(np.arange(N.TOPN_MAX, dtype=np.float64) + 2.0)
+
+
+@dataclass
+class RankMetrics:
+    """rank_metrics' result: per evaluated user (in the order given) and the means over them."""
+    hits: torch.Tensor       # int32 [n_eval]   hits among the first n slots
+    precision: torch.Tensor  # f64   hits / n
+    recall: torch.Tensor     # f64   hits / |R|
+    ndcg: torch.Tensor       # f64   DCG / ideal DCG of min(n, |R|) hits
+    ap: torch.Tensor         # f64   average precision, over min(n, |R|)
+    mean: dict               # precision, recall, ndcg, map: exact sum (math.fsum) / n_eval; None without users
+    coverage: float          # distinct recommended items / catalogue (None without a catalogue size)
+
+
+def rank_metrics(top, users, rel_ptr, rel_item, n, catalogue=None):
+    """Precision, recall, NDCG and average precision at n of the top-N lists of `users` (a TopN, or anything with
+    idx [n_users, width] and len) against each user's relevant items: user users[q] has rel_item[rel_ptr[q]:
+    rel_ptr[q + 1]], sorted ascending and unique, at least one (an item no list can hold still counts in |R|).
+    The first min(len, n) slots of a list count (1 <= n <= width).  The reference has no ranking metrics; the
+    definitions are in DESIGN.md section 3.6.  catalogue: the number of items that can be recommended (those with a
+    neighbour list); coverage = distinct items in the counted slots / catalogue.  Raises ValueError before the launch."""
+    import math
+    idx, ln = top.idx, top.len
+    dev = idx.device
+    if idx.dim() != 2 or ln.dim() != 1 or int(ln.numel()) != int(idx.shape[0]):
+        raise ValueError("top lists: idx must be [n_users, width] and len [n_users]")
+    width = int(idx.shape[1])
+    if isinstance(n, bool) or int(n) != n or not 1 <= int(n) <= min(width, N.TOPN_MAX):
+        raise ValueError("n must be an integer in [1, %d], got %r" % (min(width, N.TOPN_MAX), n))
+    n = int(n)
+    u = torch.as_tensor(users)
+    if u.dim() != 1 or u.dtype.is_floating_point or u.dtype == torch.bool:
+        raise ValueError("users must be a 1-D integer tensor")
+    u = u.to(device=dev, dtype=torch.int64)
+    m = int(u.numel())
+    if m and (int(u.min()) < 0 or int(u.max()) >= int(idx.shape[0])):
+        raise ValueError("users outside [0, %d)" % int(idx.shape[0]))
+    ptr = torch.as_tensor(rel_ptr).to(device=dev, dtype=torch.int64).flatten()
+    it = torch.as_tensor(rel_item).to(device=dev, dtype=torch.int64).flatten()
+    if int(ptr.numel()) != m + 1 or int(ptr[0]) != 0 or int(ptr[-1]) != int(it.numel()):
+        raise ValueError("rel_ptr must have len(users) + 1 entries, from 0 to len(rel_item)")
+    if m and int((ptr[1:] - ptr[:-1]).min()) < 1:
+        raise ValueError("every evaluated user needs at least one relevant item")
+    if it.numel() and (int(it.min()) < 0 or int(it.max()) > INT32_MAX):
+        raise ValueError("rel_item outside [0, 2^31)")
+    if it.numel() > 1:
+        start = torch.zeros(int(it.numel()), dtype=torch.bool, device=dev)
+        start[ptr[:-1]] = True
+        if bool(((it[1:] <= it[:-1]) & ~start[1:]).any()):
+            raise ValueError("each user's relevant items must be sorted ascending and unique")
+    out = [torch.zeros(m, dtype=torch.int32, device=dev)] + [torch.zeros(m, dtype=torch.float64, device=dev)
+                                                             for _ in range(4)]
+    # the narrowed copies stay referenced until the launch: a freed temporary's block could back the next one
+    disc = torch.from_numpy(DISCOUNT).to(dev)
+    idx_c, ln32 = idx.contiguous(), ln.to(torch.int32).contiguous()
+    u32, it32 = u.to(torch.int32).contiguous(), it.to(torch.int32).contiguous()
+    N.check(N.lib().xmap_recsim_rank_metrics(N.ptr(idx_c), N.ptr(ln32), width, N.ptr(u32), m, N.ptr(ptr), N.ptr(it32),
+                                             N.ptr(disc), n, *(N.ptr(t) for t in out), _st()), "xmap_recsim_rank_metrics")
+    mean = None
+    if m:
+        mean = {k: math.fsum(t.cpu().tolist()) / m for k, t in zip(("precision", "recall", "ndcg", "map"), out[1:])}
+    coverage = None
+    if catalogue:
+        slots = torch.arange(n, device=dev).unsqueeze(0) < ln[u].long().unsqueeze(1)
+        coverage = int(torch.unique(idx[u][:, :n][slots]).numel()) / int(catalogue)
+    return RankMetrics(*out, mean, coverage)

@@ -58,14 +58,10 @@ def extract_siminfo(sc, classfied_items):
 
 def generator_pipeline(privatemap_tool, trainRDD, extended_simRDD, private):
     """assist.py:136-150."""
-    from ..core.generator import alterego_records
-    from .. import generate as G
+    from ..core.generator import alterego_mapping, alterego_records
     from ..session import session_of
     sess = session_of(trainRDD)
-    mode = privatemap_tool.private_mode if private else "nonprivate"
-    xres, chosen = privatemap_tool._map(extended_simRDD, sess, mode)
-    mapping = G.invert_mapping(xres.start_item, chosen, sess.enc.n_items)
-    records = alterego_records(sess, mapping)
+    records = alterego_records(sess, alterego_mapping(privatemap_tool, sess, extended_simRDD, private))
     ctx = getattr(trainRDD, "context", None)
     return ctx.parallelize(records) if ctx is not None else LocalRDD(records)
 
