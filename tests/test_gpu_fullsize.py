@@ -100,7 +100,10 @@ def test_cfg2_sampled_rows_vs_oracle(cfg2):
 
 def test_cfg2_xsim_sampled_starts_vs_plan_evaluation(cfg2):
     """X-SIM at the benchmarked size: the rows of sampled starts (light, median, multi-pass and the heaviest below
-    2e6 paths) recomputed in numpy from the plan arrays; distinct ends, path counts, top-10 (ends and values)."""
+    2e6 paths) recomputed in numpy from the plan arrays; distinct ends, path counts, top-10 (ends and values).  The
+    same starts against the extended-precision reference of tests/xsim_exact.py: every top-10 value within the
+    derived rounding bound of its cell, and a top-10 position may name another end only where the two exact values
+    lie within the sum of their bounds."""
     import torch
     from tests import parity as PT
     from xmap_b200 import extend as X
@@ -129,6 +132,12 @@ def test_cfg2_xsim_sampled_starts_vs_plan_evaluation(cfg2):
             assert np.allclose(np.abs(tx[x, :L]), np.abs(xs[o]), rtol=1e-9, atol=0), "top-10 of start %d differs" % x
         else:
             assert np.allclose(tx[x, :L], xs[o], rtol=1e-9, atol=0)
+    from tests import xsim_exact as XE
+    exact = XE.exact_rows(plan, starts)
+    for x in starts:
+        row = exact[int(x)]
+        assert row["paths"] == ub[x] and cnt[x] == len(row["end"])
+        XE.check_top(te[x], tx[x], tl[x], row, 10)
     assert int(xe.T.max()) > 8 and xe.n_units > plan.start_item.numel()   # multi-pass and multi-unit starts exist
 
 
