@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define XMAP_B200_ABI_VERSION 12
+#define XMAP_B200_ABI_VERSION 13
 #define XMAP_KMAX 64                 /* largest supported top-k (extend_among_topk) */
 #define XMAP_METHOD_ADJUST_COSINE 0  /* baselinerSim.py:144-174 */
 #define XMAP_METHOD_COSINE 1         /* baselinerSim.py:115-142 */
@@ -485,6 +485,40 @@ int xmap_ingest_item_codes(const uint64_t *iid_words, int64_t ld, const uint8_t 
                            uint8_t *dom_code, uint8_t *contains, bool *has_S, bool *has_T, void *stream);
 int xmap_ingest_train_keys(const int32_t *user, const int32_t *item, const int8_t *grp, const int32_t *upos,
                            const bool *has_S, const int32_t *srank, int64_t n, int64_t *key, void *stream);
+
+/* ---------------------------------------------------------------------------
+ * (8) Explicit-feedback ALS (ALS-WR, the form of MLlib's explicit ALS; DESIGN.md section 3.8).  Factors are fp32
+ * [rows][rank], 1 <= rank <= XMAP_ALS_RANK_MAX; normal equations, Cholesky factor and solve are fp64.  The facade is
+ * x-map_b200/als.py.
+ *
+ * xmap_als_init: out[row] = Philox4x32-10(seed, (row, block)) -> rank standard normals (Box-Muller) / their L2 norm.
+ * xmap_als_normal: one segment (at most XMAP_ALS_SEGMENT records of one row, in list order) per entry:
+ *   records seg_lo[s] .. seg_lo[s] + seg_n[s] - 1 of col / rating (the other side's index and the rating);
+ *   partial[s] = (A packed, b), stride T + rank with T = rank (rank + 1) / 2; A packed lower, column-major (column j
+ *   holds rows j .. rank-1), A_ij = sum y_i y_j, b_i = sum r y_i, each summed in record order from +0.0.
+ * xmap_als_solve: row q (index rows[q]) owns the partials row_seg[q] .. row_seg[q + 1] - 1, added in that order; then
+ *   lam * row_n[q] on the diagonal, Cholesky, forward and back substitution (DESIGN.md 3.8); out[rows[q]] = the
+ *   solution rounded to fp32.  status[rows[q]] = 1 when a pivot is not > 0 (the row is then zero), else 0.
+ *   Dynamic shared memory: xmap_als_solve_smem_bytes(rank).
+ * xmap_als_predict: score[t] = sum_k X[pu[t]][k] Y[pi[t]][k] in fp64, NaN when x_n[pu[t]] or y_n[pi[t]] is 0.
+ * xmap_als_top_n: for every users[q], the first n (1..XMAP_TOPN_MAX) of the candidates cand (ascending, distinct, every
+ *   one with factors) minus, when rated_ptr is not NULL, rated_item[rated_ptr[u] .. rated_ptr[u + 1]) (ascending), by
+ *   score descending then the smaller item; NaN never listed.  Rows users[q] of out_idx / out_score [*][n] and out_len
+ *   are written (the first out_len slots); other rows are left as they are.
+ * ------------------------------------------------------------------------- */
+#define XMAP_ALS_SEGMENT 2048          /* records per segment of a row's normal equations: a constant of the library */
+#define XMAP_ALS_RANK_MAX 64
+int xmap_als_init(int32_t n_rows, int32_t rank, uint64_t seed, float *out, void *stream);
+int xmap_als_normal(const int32_t *col, const double *rating, const int64_t *seg_lo, const int32_t *seg_n, int64_t n_seg,
+                    const float *factors, int32_t rank, double *partial, void *stream);
+size_t xmap_als_solve_smem_bytes(int32_t rank);
+int xmap_als_solve(const int32_t *rows, const int64_t *row_seg, const int64_t *row_n, int32_t n_rows,
+                   const double *partial, int32_t rank, double lam, float *out, int8_t *status, void *stream);
+int xmap_als_predict(const float *X, const float *Y, const int64_t *x_n, const int64_t *y_n, int32_t rank,
+                     const int32_t *pu, const int32_t *pi, int64_t n_pairs, double *score, void *stream);
+int xmap_als_top_n(const float *X, const float *Y, int32_t rank, const int32_t *users, int32_t n_users,
+                   const int32_t *cand, int32_t n_cand, const int64_t *rated_ptr, const int32_t *rated_item, int32_t n,
+                   int32_t *out_idx, double *out_score, int32_t *out_len, void *stream);
 
 #ifdef __cplusplus
 }

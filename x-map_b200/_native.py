@@ -14,11 +14,13 @@ KMAX = 64
 XSIM_MAX_CELLS_LG = 13    # XMAP_XSIM_MAX_CELLS_LG
 METHODS = {"adjust_cosine": 0, "cosine": 1}
 SELECT_LONG = 8192            # XMAP_SELECT_LONG
-ABI_VERSION = 12
+ABI_VERSION = 13
 ROW_HDR_BYTES = 48          # XMAP_SIM_ROW_HDR_BYTES
 INGEST_ID_MAX = 48          # XMAP_INGEST_ID_MAX
 TOPN_MAX = 64               # XMAP_TOPN_MAX
 TOPN_WARP_BOUND = 2048      # XMAP_TOPN_WARP_BOUND
+ALS_SEGMENT = 2048          # XMAP_ALS_SEGMENT
+ALS_RANK_MAX = 64           # XMAP_ALS_RANK_MAX
 
 _p = C.c_void_p
 
@@ -106,6 +108,12 @@ _SIGS = {
     "xmap_ingest_item_suffix": (C.c_int, [_p, C.c_int64, _p, _p, C.c_int32, _p, _p]),
     "xmap_ingest_item_codes": (C.c_int, [_p, C.c_int64, _p, _p, C.c_int32, _p, C.c_int32, _p, _p, _p, _p, _p, _p]),
     "xmap_ingest_train_keys": (C.c_int, [_p, _p, _p, _p, _p, _p, C.c_int64, _p, _p]),
+    "xmap_als_init": (C.c_int, [C.c_int32, C.c_int32, C.c_uint64, _p, _p]),
+    "xmap_als_normal": (C.c_int, [_p, _p, _p, _p, C.c_int64, _p, C.c_int32, _p, _p]),
+    "xmap_als_solve_smem_bytes": (C.c_size_t, [C.c_int32]),
+    "xmap_als_solve": (C.c_int, [_p, _p, _p, C.c_int32, _p, C.c_int32, C.c_double, _p, _p, _p]),
+    "xmap_als_predict": (C.c_int, [_p, _p, _p, _p, C.c_int32, _p, _p, C.c_int64, _p, _p]),
+    "xmap_als_top_n": (C.c_int, [_p, _p, C.c_int32, _p, C.c_int32, _p, C.c_int32, _p, _p, C.c_int32, _p, _p, _p, _p]),
 }
 
 EXPORTED_SYMBOLS = tuple(_SIGS)

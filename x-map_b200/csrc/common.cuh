@@ -69,6 +69,20 @@ __device__ __forceinline__ int sim_bin(unsigned long long key_bits) {
     return max(0, min(SIM_BINS - 1, hi - base));
 }
 
+// Philox4x32-10 (counter-based; Salmon et al. 2011): the generator of generate.cu and als.cu
+__host__ __device__ inline void philox4x32_10(uint32_t c[4], uint32_t k0, uint32_t k1) {
+    const uint32_t M0 = 0xD2511F53u, M1 = 0xCD9E8D57u, W0 = 0x9E3779B9u, W1 = 0xBB67AE85u;
+    for (int r = 0; r < 10; ++r) {
+        uint64_t p0 = (uint64_t)M0 * c[0], p1 = (uint64_t)M1 * c[2];
+        uint32_t n0 = (uint32_t)(p1 >> 32) ^ c[1] ^ k0;
+        uint32_t n1 = (uint32_t)p1;
+        uint32_t n2 = (uint32_t)(p0 >> 32) ^ c[3] ^ k1;
+        uint32_t n3 = (uint32_t)p0;
+        c[0] = n0; c[1] = n1; c[2] = n2; c[3] = n3;
+        k0 += W0; k1 += W1;
+    }
+}
+
 // warp arg-best over (key, tie, pos); every lane gets the winner.
 __device__ __forceinline__ void warp_argbest(unsigned long long &key, int &tie, int &pos) {
 #pragma unroll

@@ -8,11 +8,18 @@ The tools are the facade chain's (BaselinerSim, ExtendSim, Generator, Recommende
 parameter, private mode and seed means what it means there, and the predictions, the MAE and the lists equal those of
 clean_split_pipeline -> ... -> recommender_prediction_pipeline / recommend_top_n (with the time zone at UTC: the
 facade turns times into local datetimes and back with timegm).  Every array stays on the device; no Python object is
-made per record.  The reference has no ranking metrics: their definitions are in DESIGN.md section 3.6."""
+made per record.  The reference has no ranking metrics: their definitions are in DESIGN.md section 3.6.
+
+    ev = evaluate.evaluate_als(A, rank=10, iterations=5, lambda_=0.01)          # the MLlib-ALS baseline
+
+evaluate_als runs the same held-out evaluation on explicit ALS (als.py, DESIGN.md section 3.8), trained on every
+training record of both domains or on the AlterEgo profile."""
+import math
 from dataclasses import dataclass
 
 import torch
 
+from . import als as ALS
 from . import generate as G
 from . import ingest as I
 from . import recsim as RS
@@ -38,22 +45,16 @@ class Evaluation:
     stage_ms: dict               # device time per stage when events were passed, else None
 
 
-def evaluate(A, sim_tool, extend_tool, generator, private_gen, rec_sim_tool, privacy_tool, private_rec, n=10,
-             threshold=None, alpha=0.03, events=None):
-    """Train arrays -> similarity -> X-SIM -> mapping -> AlterEgo profile -> item-kNN, then the held-out MAE of the
-    test pairs and the top-n accuracy of the test users.  private_gen / private_rec: the generator's private mode and
-    the private neighbour selection, as generator_pipeline's and recommender_privacy_pipeline's flags.  threshold: a
-    held-out record is relevant when its rating >= threshold (None: every one).  events: optional dict that receives
-    CUDA-event pairs per stage; their times are then in stage_ms."""
+def _alterego_profile(A, sim_tool, extend_tool, generator, private_gen, timer):
+    """Train arrays -> similarity -> X-SIM -> mapping -> the AlterEgo profile in the facade's list order (target records
+    in training order, then the synthetic ones): (user, item, rating, ts, profile_items, synthetic record count).
+    Profile items are numbered by rank among the items present, as the facade's np.unique over id strings does (the
+    private selection draws per item index); users keep the train numbering (only their order matters)."""
     dev = A.user.device
-    timer = I._Timer(events)
-    counts = {}
     if sim_tool.method not in ("cosine", "adjust_cosine"):
         raise ValueError("unknown similarity method %r" % (sim_tool.method,))
     if A.train_user_of is None or A.train_item_of is None:
         raise ValueError("the arrays carry no train index maps (train_user_of / train_item_of)")
-
-    # ---- AlterEgo profile, in the facade's list order: target records in training order, then the synthetic ones ----
     with timer("session"):
         sess = Session(I.encoded(A), dev, user=A.user, item=A.item, rating=A.rating, meta=A.meta)
     with timer("similarity_xsim"):
@@ -66,12 +67,75 @@ def evaluate(A, sim_tool, extend_tool, generator, private_gen, rec_sim_tool, pri
         pi = torch.cat([A.item.long()[keep], oi.long()])
         pr = torch.cat([A.rating[keep], orr])
         pt = torch.floor(torch.cat([A.ts[keep], A.ts[ot.long()]])).long()      # timegm of the facade's datetimes
-        # profile items numbered by rank among the items present, as the facade's np.unique over id strings does (the
-        # private selection draws per item index); users keep the train numbering (only their order matters)
         profile_items, pi = torch.unique(pi, return_inverse=True)
-        n_users, n_items = len(A.uids), int(profile_items.numel())
-    counts["profile_records"], counts["synthetic_records"] = int(pu.numel()), int(ou.numel())
-    del sess, xs, mapping, ou, oi, orr, ot
+    return pu, pi, pr, pt, profile_items, int(ou.numel())
+
+
+def _test_pairs(A, profile_items, in_prof_user):
+    """The held-out pairs in train numbering and then in profile numbering: (prof_of, tu, tpi, untrained,
+    no_profile); prof_of maps a train item to its profile index (-1 outside the profile)."""
+    dev = A.user.device
+    prof_of = torch.full((len(A.iids),), -1, dtype=torch.int64, device=dev)
+    prof_of[profile_items] = torch.arange(int(profile_items.numel()), device=dev)
+    tu = A.train_user_of[A.test_user.long()].long()
+    ti = A.train_item_of[A.test_item.long()].long()
+    untrained = (tu < 0) | (ti < 0)
+    tpi = torch.where(untrained, -1, prof_of[ti.clamp(min=0)])
+    no_profile = ~untrained & ((tpi < 0) | ~in_prof_user[tu.clamp(min=0)])
+    return prof_of, tu, tpi, untrained, no_profile
+
+
+def _eval_users(A, threshold):
+    """The relevant held-out records (rating >= threshold, of a test user) and the evaluated users, the trained test
+    users with one, ascending by all_uids index: (rel, is_test, has_rel, trained, users, run = their train index)."""
+    dev = A.user.device
+    n_test = int(A.test_user.numel())
+    rel = torch.ones(n_test, dtype=torch.bool, device=dev) if threshold is None else A.test_rating >= threshold
+    is_test = torch.zeros(len(A.all_uids), dtype=torch.bool, device=dev)
+    is_test[torch.from_numpy(A.test_users).to(dev)] = True
+    rel &= is_test[A.test_user.long()]
+    has_rel = torch.zeros(len(A.all_uids), dtype=torch.bool, device=dev)
+    has_rel[A.test_user.long()[rel]] = True
+    trained = A.train_user_of >= 0
+    users = torch.nonzero(has_rel & trained).flatten()          # ascending all_uids index
+    run = A.train_user_of[users].long()
+    return rel, is_test, has_rel, trained, users, run
+
+
+def _relevant_csr(A, rel, users, prof_of, n_items):
+    """Each evaluated user's relevant items in profile numbering, sorted and unique: (rel_ptr, code).  An item outside
+    the profile gets a code past every profile item."""
+    dev = A.user.device
+    q_of = torch.full((len(A.all_uids),), -1, dtype=torch.int64, device=dev)
+    q_of[users] = torch.arange(int(users.numel()), device=dev)
+    rq = q_of[A.test_user.long()[rel]]
+    keep_r = rq >= 0
+    rq, ri_all = rq[keep_r], A.test_item.long()[rel][keep_r]
+    rti = A.train_item_of[ri_all].long()
+    code = torch.where(rti >= 0, prof_of[rti.clamp(min=0)], -1)
+    code = torch.where(code >= 0, code, n_items + ri_all)
+    key = torch.unique(rq * (n_items + len(A.all_iids)) + code)
+    rq, code = key // (n_items + len(A.all_iids)), key % (n_items + len(A.all_iids))
+    rel_ptr = torch.zeros(int(users.numel()) + 1, dtype=torch.int64, device=dev)
+    rel_ptr[1:] = torch.cumsum(torch.bincount(rq, minlength=int(users.numel())), 0)
+    return rel_ptr, code
+
+
+def evaluate(A, sim_tool, extend_tool, generator, private_gen, rec_sim_tool, privacy_tool, private_rec, n=10,
+             threshold=None, alpha=0.03, events=None):
+    """Train arrays -> similarity -> X-SIM -> mapping -> AlterEgo profile -> item-kNN, then the held-out MAE of the
+    test pairs and the top-n accuracy of the test users.  private_gen / private_rec: the generator's private mode and
+    the private neighbour selection, as generator_pipeline's and recommender_privacy_pipeline's flags.  threshold: a
+    held-out record is relevant when its rating >= threshold (None: every one).  events: optional dict that receives
+    CUDA-event pairs per stage; their times are then in stage_ms."""
+    dev = A.user.device
+    timer = I._Timer(events)
+    counts = {}
+
+    # ---- AlterEgo profile, in the facade's list order: target records in training order, then the synthetic ones ----
+    pu, pi, pr, pt, profile_items, n_synth = _alterego_profile(A, sim_tool, extend_tool, generator, private_gen, timer)
+    n_users, n_items = len(A.uids), int(profile_items.numel())
+    counts["profile_records"], counts["synthetic_records"] = int(pu.numel()), n_synth
 
     with timer("item_knn"):
         state = ProfileState.from_arrays(pu, pi, pr, pt, A.uids, A.iids[profile_items.cpu().numpy()])
@@ -82,13 +146,7 @@ def evaluate(A, sim_tool, extend_tool, generator, private_gen, rec_sim_tool, pri
     with timer("prediction"):
         n_test = int(A.test_user.numel())
         in_prof_user = torch.bincount(pu, minlength=n_users) > 0
-        prof_of = torch.full((len(A.iids),), -1, dtype=torch.int64, device=dev)
-        prof_of[profile_items] = torch.arange(n_items, device=dev)
-        tu = A.train_user_of[A.test_user.long()].long()
-        ti = A.train_item_of[A.test_item.long()].long()
-        untrained = (tu < 0) | (ti < 0)
-        tpi = torch.where(untrained, -1, prof_of[ti.clamp(min=0)])
-        no_profile = ~untrained & ((tpi < 0) | ~in_prof_user[tu.clamp(min=0)])
+        prof_of, tu, tpi, untrained, no_profile = _test_pairs(A, profile_items, in_prof_user)
         ok = torch.nonzero(~untrained & ~no_profile).flatten()
         p0, p1, mae0, mae1 = RS.predict(pu, pi, pr, pt, n_users, knn, nb, tu[ok], tpi[ok], A.test_rating[ok], alpha)
         pred0 = torch.full((n_test,), -1.0, dtype=torch.float64, device=dev)
@@ -100,30 +158,10 @@ def evaluate(A, sim_tool, extend_tool, generator, private_gen, rec_sim_tool, pri
 
     # ---- top-n of the test users with a relevant held-out record -----------------------------------------------------
     with timer("top_n"):
-        rel = torch.ones(n_test, dtype=torch.bool, device=dev) if threshold is None else A.test_rating >= threshold
-        is_test = torch.zeros(len(A.all_uids), dtype=torch.bool, device=dev)
-        is_test[torch.from_numpy(A.test_users).to(dev)] = True
-        rel &= is_test[A.test_user.long()]
-        has_rel = torch.zeros(len(A.all_uids), dtype=torch.bool, device=dev)
-        has_rel[A.test_user.long()[rel]] = True
-        trained = A.train_user_of >= 0
-        users = torch.nonzero(has_rel & trained).flatten()          # ascending all_uids index
-        run = A.train_user_of[users].long()
+        rel, is_test, has_rel, trained, users, run = _eval_users(A, threshold)
         top = RS.top_n(pu, pi, pr, pt, n_users, knn, nb, n, alpha=alpha, users=run)
     with timer("rank_metrics"):
-        # relevant items in profile numbering; an item outside the profile gets a code past every profile item
-        q_of = torch.full((len(A.all_uids),), -1, dtype=torch.int64, device=dev)
-        q_of[users] = torch.arange(int(users.numel()), device=dev)
-        rq = q_of[A.test_user.long()[rel]]
-        keep_r = rq >= 0
-        rq, ri_all = rq[keep_r], A.test_item.long()[rel][keep_r]
-        rti = A.train_item_of[ri_all].long()
-        code = torch.where(rti >= 0, prof_of[rti.clamp(min=0)], -1)
-        code = torch.where(code >= 0, code, n_items + ri_all)
-        key = torch.unique(rq * (n_items + len(A.all_iids)) + code)
-        rq, code = key // (n_items + len(A.all_iids)), key % (n_items + len(A.all_iids))
-        rel_ptr = torch.zeros(int(users.numel()) + 1, dtype=torch.int64, device=dev)
-        rel_ptr[1:] = torch.cumsum(torch.bincount(rq, minlength=int(users.numel())), 0)
+        rel_ptr, code = _relevant_csr(A, rel, users, prof_of, n_items)
         catalogue = int((nb.len > 0).sum())
         metrics = RS.rank_metrics(top, run, rel_ptr, code, n, catalogue=catalogue)
         reachable = torch.zeros(int(code.numel()), dtype=torch.bool, device=dev)
@@ -139,3 +177,94 @@ def evaluate(A, sim_tool, extend_tool, generator, private_gen, rec_sim_tool, pri
         torch.cuda.synchronize(dev)
         stage_ms = {k: sum(a.elapsed_time(b) for a, b in v) for k, v in events.items()}
     return Evaluation(mae0, mae1, pred0, pred1, users, metrics, top, profile_items, n, counts, stage_ms)
+
+
+@dataclass
+class AlsEvaluation:
+    """evaluate_als's result.  Held-out pairs follow A.test_* order; evaluated users are ids of A.all_uids."""
+    mae: float                   # mean |rating - score| over the predicted pairs (None when none was)
+    mae_bounded: float           # the same with the score rounded as rs_bound_rating does: int(x + 0.5) within [0, 5]
+    pred: torch.Tensor           # f64 [n_test] raw score, NaN where the pair was skipped
+    users: torch.Tensor          # int64 [n_eval] all_uids index of each evaluated user
+    metrics: RS.RankMetrics
+    top: ALS.AlsTopN             # rows indexed by train user; items index profile_items
+    model: ALS.AlsModel          # users in train numbering, items in profile numbering
+    profile_items: torch.Tensor  # int64: train item index of every trained item (trained item index = position)
+    train_user: torch.Tensor     # int64: the records the model was trained on
+    train_item: torch.Tensor     # int64, profile numbering
+    train_rating: torch.Tensor   # f64
+    n: int
+    counts: dict
+    stage_ms: dict               # device time per stage when events were passed, else None
+
+
+def evaluate_als(A, rank=10, iterations=5, lambda_=0.01, seed=None, alterego=None, n=10, threshold=None, events=None):
+    """Explicit ALS (als.train, DESIGN.md 3.8) on the training split, then the held-out MAE of the test pairs and the
+    top-n accuracy of the test users, as evaluate reports them for item-kNN.
+    alterego: None trains on every training record of both domains (the baseline: a test user keeps its source-domain
+    records, so every trained test user has factors); (sim_tool, extend_tool, generator, private_gen) builds the
+    AlterEgo profile as evaluate does and trains on it ("X-MAP + ALS").
+    mae uses the raw score, as MLlib's predict returns it; mae_bounded rounds it as the item-kNN prediction does.
+    The lists cover the target-domain items with factors, minus the user's training records; the catalogue is those
+    items.  threshold / events: as in evaluate; with events the model also carries its per-half-step kernel times."""
+    dev = A.user.device
+    timer = I._Timer(events)
+    counts = {}
+    if A.train_user_of is None or A.train_item_of is None:
+        raise ValueError("the arrays carry no train index maps (train_user_of / train_item_of)")
+    n_users = len(A.uids)
+    if alterego is None:
+        pu, pi, pr = A.user.long(), A.item.long(), A.rating
+        profile_items = torch.arange(len(A.iids), device=dev)
+    else:
+        sim_tool, extend_tool, generator, private_gen = alterego
+        pu, pi, pr, _, profile_items, n_synth = _alterego_profile(A, sim_tool, extend_tool, generator, private_gen,
+                                                                  timer)
+        counts["synthetic_records"] = n_synth
+    n_items = int(profile_items.numel())
+    counts["train_records"] = int(pu.numel())
+
+    with timer("als_train"):
+        model = ALS.train(pu, pi, pr, n_users, n_items, rank, iterations, lambda_, seed=seed, device=dev,
+                          events={} if events is not None else None)
+
+    with timer("prediction"):
+        n_test = int(A.test_user.numel())
+        prof_of, tu, tpi, untrained, no_profile = _test_pairs(A, profile_items, model.user_count > 0)
+        no_factors = ~untrained & ~no_profile & (model.item_count[tpi.clamp(min=0)] == 0)
+        ok = torch.nonzero(~untrained & ~no_profile & ~no_factors).flatten()
+        p = ALS.predict(model, tu[ok], tpi[ok])
+        pred = torch.full((n_test,), float("nan"), dtype=torch.float64, device=dev)
+        pred[ok] = p
+        mae = mae_b = None
+        if int(ok.numel()):
+            tr = A.test_rating[ok]
+            bounded = torch.clamp(torch.trunc(p + 0.5), 0, 5)
+            mae = math.fsum((tr - p).abs().cpu().tolist()) / int(ok.numel())
+            mae_b = math.fsum((tr - bounded).abs().cpu().tolist()) / int(ok.numel())
+    counts.update(test_pairs=n_test, predicted=int(ok.numel()), skipped_untrained=int(untrained.sum()),
+                  skipped_no_profile=int(no_profile.sum()), skipped_no_factors=int(no_factors.sum()))
+
+    with timer("top_n"):
+        rel, is_test, has_rel, trained, users, run = _eval_users(A, threshold)
+        cand = torch.nonzero(A.meta.has_T[profile_items] & (model.item_count > 0)).flatten()
+        top = ALS.top_n(model, n, pu, pi, candidates=cand, users=run)
+    with timer("rank_metrics"):
+        rel_ptr, code = _relevant_csr(A, rel, users, prof_of, n_items)
+        catalogue = int(cand.numel())
+        metrics = RS.rank_metrics(top, run, rel_ptr, code, n, catalogue=catalogue)
+        is_cand = torch.zeros(n_items, dtype=torch.bool, device=dev)
+        is_cand[cand] = True
+        in_prof = code < n_items
+        reachable = torch.zeros(int(code.numel()), dtype=torch.bool, device=dev)
+        reachable[in_prof] = is_cand[code[in_prof]]
+    counts.update(eval_users=int(users.numel()), eval_users_without_factors=int((model.user_count[run] == 0).sum()),
+                  test_users_untrained=int((has_rel & ~trained).sum()),
+                  test_users_without_relevant=int(len(A.test_users)) - int((has_rel & is_test).sum()),
+                  relevant_items=int(code.numel()), unreachable_items=int((~reachable).sum()),
+                  catalogue_items=catalogue)
+    stage_ms = None
+    if events is not None:
+        torch.cuda.synchronize(dev)
+        stage_ms = {k: sum(a.elapsed_time(b) for a, b in v) for k, v in events.items()}
+    return AlsEvaluation(mae, mae_b, pred, users, metrics, top, model, profile_items, pu, pi, pr, n, counts, stage_ms)
