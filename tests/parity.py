@@ -97,7 +97,9 @@ def multi_domain_cases(n_users, n_items, n_draws, overlap, seed, n_domains=3):
 
 
 def run_gpu_sim(user, item, rating, n_users, n_items, meta, method, num_atleast, k, emit=True, **engine_kw):
-    """engine_kw: SimEngine options (max_smem_cells, rec_budget)."""
+    """engine_kw: SimEngine options (max_smem_cells, rec_budget).  With emit, the neighbour tables must also equal,
+    bit for bit, the exact selection (tests/select_exact.py) over the engine's own records: what differs from the
+    oracle after that comes from accumulation alone."""
     import torch
     from xmap_b200 import engine as E
     lay = E.build_layout(user, item, rating, n_users, n_items)
@@ -105,6 +107,9 @@ def run_gpu_sim(user, item, rating, n_users, n_items, meta, method, num_atleast,
     tabs = eng.run()
     pairs = eng.emit_pairs() if emit else None
     torch.cuda.synchronize()
+    if emit:
+        from tests import select_exact as SE
+        SE.assert_engine_selection(eng, meta, pairs=pairs)
     return lay, eng, tabs, pairs
 
 

@@ -96,6 +96,15 @@ def test_cfg2_sampled_rows_vs_oracle(cfg2):
     assert near <= 12, "%d of %d sampled lists differ by near-ties (regression ceiling)" % (near, n_lists)
     print("cfg2 sampled parity: %d rows, %d kept pairs, sim max rel err %.3g, %d fragile, %d/%d near-tie lists"
           % (len(rows), len(Q["i"]), rel, len(fragile), near, n_lists))
+    # the selection itself is exact on its own records: the sampled rows and every row of the CTA kernel
+    from tests import select_exact as SE
+    long_rows = np.nonzero(cnt > SE.SELECT_LONG)[0]
+    sel_rows = torch.as_tensor(np.union1d(rows, long_rows), device=cfg2["dev"])
+    n = SE.assert_engine_selection(eng, wl["meta"], sel_rows)
+    ri, rj, rs = SE.engine_records(eng, sel_rows)
+    labels, _ = SE.classify(ri, rj, rs, flags, dom, contains, k, I)
+    print("cfg2 exact re-selection: %d rows, %d of them with more than %d records; paths %s"
+          % (n, len(long_rows), SE.SELECT_LONG, SE.path_counts(labels[sel_rows.cpu().numpy()])))
 
 
 def test_cfg2_xsim_sampled_starts_vs_plan_evaluation(cfg2):
