@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define XMAP_B200_ABI_VERSION 13
+#define XMAP_B200_ABI_VERSION 14
 #define XMAP_KMAX 64                 /* largest supported top-k (extend_among_topk) */
 #define XMAP_METHOD_ADJUST_COSINE 0  /* baselinerSim.py:144-174 */
 #define XMAP_METHOD_COSINE 1         /* baselinerSim.py:115-142 */
@@ -519,6 +519,48 @@ int xmap_als_predict(const float *X, const float *Y, const int64_t *x_n, const i
 int xmap_als_top_n(const float *X, const float *Y, int32_t rank, const int32_t *users, int32_t n_users,
                    const int32_t *cand, int32_t n_cand, const int64_t *rated_ptr, const int32_t *rated_item, int32_t n,
                    int32_t *out_idx, double *out_score, int32_t *out_len, void *stream);
+
+/* ---------------------------------------------------------------------------
+ * (9) User-based kNN on the AlterEgo profile (DESIGN.md section 3.9): RecommenderSim "cosine_user", defined by this
+ * project as the item-based stage with the roles of user and item exchanged.  The profile is given twice:
+ *   item_ptr [n_items + 1], t_user, t_item, t_rating: the records grouped by item, sorted by (item, user, list position);
+ *   u_ptr [n_users + 1], u_rec: each user's records as positions in that order, ascending;
+ *   info [n_users][3] = (average, norm2, count) over the user's records; uexp[u] = E with 2^(E-1) <= norm2 < 2^E
+ *   (0 for a zero norm); qbase = 62 - ceil(log2 m), m the largest record count of one (user, item).
+ * xmap_usersim_rows: the similarity rows of users rows[0 .. n_rows), one warp (cta = 0) or one CTA of 8 warps (cta = 1)
+ *   each, in passes over tiles of `tile` users of the neighbour axis (dynamic shared memory
+ *   xmap_usersim_smem_bytes(tile, cta, emit), at most 227 KB).
+ *   select (emit_ptr NULL): nb_idx / nb_sim [n_users][k] (k <= XMAP_KMAX), nb_len: the first k neighbours of each row by
+ *     |sim| descending, ties to the smaller user; rows not listed are left as they are.
+ *   emit (emit_ptr [n_rows + 1]): (e_v, e_n, e_sim, e_ls) of every pair of row q, in user order, at
+ *     emit_ptr[q] ..; e_len[q] = the pairs of the row.  error_flag 2 when a row has more pairs than its extent (the
+ *     pairs past it are not written).
+ *   stats[0] += co-rating products, stats[1] += distinct (row, neighbour) pairs, stats[2] += passes (unsigned 64-bit).
+ * xmap_usersim_top_n: the first n (1..XMAP_TOPN_MAX) items of users[q] by the score of xmap_recsim_predict on the
+ *   transposed profile before bound_rating (decay 0 / 1), over the items the user has no record on; score descending,
+ *   then the smaller item; NaN never listed; empty for a user without a neighbour list.  up_ptr [n_users + 1], up_item:
+ *   the records sorted by (user, item, list position); t_ts: the times in the item order above; one warp (cta = 0) or
+ *   one CTA per user; the item axis in tiles of `tile` items (0: XMAP_USERSIM_TOPN_WARP_TILE / _CTA_TILE; >= 32).  stats[0] += neighbour
+ *   records visited, stats[1] += candidates scored; error_flag 4 as in xmap_recsim_predict.
+ * ------------------------------------------------------------------------- */
+#define XMAP_USERSIM_WARP_BOUND 4096       /* rows with sum over their records of the item's record count above it take a CTA */
+#define XMAP_USERSIM_WARP_TILE 4096
+#define XMAP_USERSIM_CTA_TILE 16384
+#define XMAP_USERSIM_EMIT_CTA_TILE 8192
+#define XMAP_USERSIM_TOPN_WARP_TILE (1 << 15)
+#define XMAP_USERSIM_TOPN_CTA_TILE (1 << 19)
+size_t xmap_usersim_smem_bytes(int32_t tile, int32_t cta, int32_t emit);
+int xmap_usersim_rows(const int64_t *item_ptr, const int32_t *t_user, const int32_t *t_item, const double *t_rating,
+                      const int64_t *u_ptr, const int64_t *u_rec, const double *info, const int32_t *uexp, int32_t n_users,
+                      int32_t qbase, int32_t num_atleast, int32_t k, const int32_t *rows, int32_t n_rows, int32_t cta,
+                      int32_t tile, int32_t *nb_idx, double *nb_sim, int32_t *nb_len, const int64_t *emit_ptr,
+                      int32_t *e_v, int64_t *e_n, double *e_sim, double *e_ls, int64_t *e_len,
+                      unsigned long long *stats, int32_t *error_flag, void *stream);
+int xmap_usersim_top_n(const int64_t *up_ptr, const int32_t *up_item, const int64_t *item_ptr, const int32_t *t_user,
+                       const double *t_rating, const int64_t *t_ts, const double *info, const int32_t *nb_idx,
+                       const double *nb_sim, const int32_t *nb_len, int32_t k, int32_t n_items, const int32_t *users,
+                       int32_t n_users, int32_t cta, int32_t tile, int32_t n, double alpha, int32_t decay, int32_t *out_idx,
+                       double *out_score, int32_t *out_len, unsigned long long *stats, int32_t *error_flag, void *stream);
 
 #ifdef __cplusplus
 }

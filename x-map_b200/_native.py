@@ -14,13 +14,17 @@ KMAX = 64
 XSIM_MAX_CELLS_LG = 13    # XMAP_XSIM_MAX_CELLS_LG
 METHODS = {"adjust_cosine": 0, "cosine": 1}
 SELECT_LONG = 8192            # XMAP_SELECT_LONG
-ABI_VERSION = 13
+ABI_VERSION = 14
 ROW_HDR_BYTES = 48          # XMAP_SIM_ROW_HDR_BYTES
 INGEST_ID_MAX = 48          # XMAP_INGEST_ID_MAX
 TOPN_MAX = 64               # XMAP_TOPN_MAX
 TOPN_WARP_BOUND = 2048      # XMAP_TOPN_WARP_BOUND
 ALS_SEGMENT = 2048          # XMAP_ALS_SEGMENT
 ALS_RANK_MAX = 64           # XMAP_ALS_RANK_MAX
+USERSIM_WARP_BOUND = 4096   # XMAP_USERSIM_WARP_BOUND
+USERSIM_WARP_TILE = 4096    # XMAP_USERSIM_WARP_TILE
+USERSIM_CTA_TILE = 16384    # XMAP_USERSIM_CTA_TILE
+USERSIM_EMIT_CTA_TILE = 8192    # XMAP_USERSIM_EMIT_CTA_TILE
 
 _p = C.c_void_p
 
@@ -114,6 +118,11 @@ _SIGS = {
     "xmap_als_solve": (C.c_int, [_p, _p, _p, C.c_int32, _p, C.c_int32, C.c_double, _p, _p, _p]),
     "xmap_als_predict": (C.c_int, [_p, _p, _p, _p, C.c_int32, _p, _p, C.c_int64, _p, _p]),
     "xmap_als_top_n": (C.c_int, [_p, _p, C.c_int32, _p, C.c_int32, _p, C.c_int32, _p, _p, C.c_int32, _p, _p, _p, _p]),
+    "xmap_usersim_smem_bytes": (C.c_size_t, [C.c_int32, C.c_int32, C.c_int32]),
+    "xmap_usersim_rows": (C.c_int, [_p, _p, _p, _p, _p, _p, _p, _p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _p,
+                                    C.c_int32, C.c_int32, C.c_int32, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p]),
+    "xmap_usersim_top_n": (C.c_int, [_p, _p, _p, _p, _p, _p, _p, _p, _p, _p, C.c_int32, C.c_int32, _p, C.c_int32,
+                                     C.c_int32, C.c_int32, C.c_int32, C.c_double, C.c_int32, _p, _p, _p, _p, _p, _p]),
 }
 
 EXPORTED_SYMBOLS = tuple(_SIGS)

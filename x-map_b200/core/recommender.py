@@ -3,8 +3,10 @@
 
 Offered: item-based `cosine_item` similarity with local sensitivity, NON-private neighbour selection, item-based
 prediction with and without temporal decay, MAE.  `adjust_cosine_item` is accepted and, as in the reference (whose
-dispatch tests the substring "cosine_item" first, recommenderSim.py:188), runs the same cosine_item path.  Not offered
-(ValueError): the user-based variants (absent from the reference's own source tree, SURVEY.md 2.1).  The private neighbour
+dispatch tests the substring "cosine_item" first, recommenderSim.py:188), runs the same cosine_item path.  The
+user-based variants `cosine_user` / `adjust_cosine_user` (one path) follow the project's own definition, the
+item-based stage with the roles of user and item exchanged (DESIGN.md 3.9; usersim.py): the reference's source tree
+no longer defines them (SURVEY.md 2.1), so no parity with it is claimed.  The private neighbour
 selection (recommenderPrivacy.py:70-139, 152-171) is offered as it behaves under Python 3, with injectable uniforms.  The work happens in csrc/recsim.cu; these classes
 encode the flat (uid, iid, rating, time) records once and keep the device state on the objects they return.
 """
@@ -36,6 +38,8 @@ class ProfileState(object):
         self.upos = {s: n for n, s in enumerate(self.uids)}
         self.ipos = {s: n for n, s in enumerate(self.iids)}
         self.num_atleast = None  # set by RecommenderSim.calculate_sim
+        self.query_users = None  # user-based: None for every row, or the users whose rows are needed
+        self.user_based = False  # set by RecommenderSim.calculate_sim: the method is a user-based one
         self.knn = None          # recsim.ItemKnn: item info and the neighbour tables
         self.nb = None           # recsim.Neighbors
 
@@ -49,6 +53,8 @@ class ProfileState(object):
         self.uids, self.iids = uids, iids
         self.user, self.item, self.rating, self.ts = user, item, rating, ts
         self.num_atleast = self.knn = self.nb = None
+        self.user_based = False
+        self.query_users = None
         return self
 
 
@@ -76,10 +82,22 @@ class RecommenderSim(object):
         """((iid1, iid2), [sim, local sensitivity])* -- recommenderSim.py:186-195.  The reference dispatches on
         `"cosine_item" in self.method` FIRST (:188), and "adjust_cosine_item" contains that substring, so both method
         names run cosine_sim there (adjusted_cosine_sim, :135-184, is unreachable); both are accepted here and mean
-        the same.  Anything else (the user-based names) returns None in the reference and raises here."""
+        the same.  "cosine_user" / "adjust_cosine_user" give ((uid1, uid2), [sim, local sensitivity])* of the
+        project's user-based definition (DESIGN.md 3.9), one block of users at a time.  Anything else raises."""
+        if "cosine_user" in self.method:
+            state.num_atleast, state.user_based = self.num_atleast, True
+
+            def build_users():
+                from .. import usersim as US
+                for u, v, _n, sim, ls in US.pair_blocks(state.user, state.item, state.rating, len(state.uids),
+                                                        len(state.iids), self.num_atleast):
+                    u, v, sim, ls = u.cpu().numpy(), v.cpu().numpy(), sim.cpu().numpy(), ls.cpu().numpy()
+                    for q in range(len(u)):
+                        yield (str(state.uids[u[q]]), str(state.uids[v[q]])), [sim[q], ls[q]]
+            return LazyRDD(build_users, handle=state)
         if "cosine_item" not in self.method:
-            raise ValueError("only the item-based similarities are offered (got %r)" % (self.method,))
-        state.num_atleast = self.num_atleast
+            raise ValueError("unknown similarity method %r" % (self.method,))
+        state.num_atleast, state.user_based = self.num_atleast, False
 
         def build():
             # only when the records are collected, one block of item rows at a time; the neighbour selection
@@ -106,21 +124,32 @@ class RecommenderPrivacy(object):
         self.seed, self._calls = int(seed), 0
 
     def _neighbour_rdd(self, state):
+        ids = state.uids if state.user_based else state.iids
+
         def build():
             ln, idx, sim = state.nb.len.cpu().numpy(), state.nb.idx.cpu().numpy(), state.nb.sim.cpu().numpy()
             for it in np.flatnonzero(ln):
-                yield str(state.iids[it]), [(str(state.iids[idx[it, r]]), sim[it, r]) for r in range(ln[it])]
+                yield str(ids[it]), [(str(ids[idx[it, r]]), sim[it, r]) for r in range(ln[it])]
         out = LazyRDD(build, handle=state)
         out.collectAsMap = lambda: _handle_dict(out.collect(), state)
         return out
 
+    def _knn(self, state, private=None):
+        if state.user_based:
+            from .. import usersim as US
+            state.knn = US.user_knn(state.user, state.item, state.rating, len(state.uids), len(state.iids),
+                                    state.num_atleast, int(self.mapping_range), private=private, users=state.query_users)
+        else:
+            state.knn = RS.item_knn(state.user, state.item, state.rating, len(state.iids), state.num_atleast,
+                                    int(self.mapping_range), private=private)
+        state.nb = state.knn.nb
+
     def nonprivate_neighbor_selection(self, rdd):
         """(iid, [(neighbour, [sim, ls])*]) -- recommenderPrivacy.py:141-150; here the sensitivity is already dropped
-        (nonnoise_perturbation, :180-189), which is all the non-private pipeline keeps."""
+        (nonnoise_perturbation, :180-189), which is all the non-private pipeline keeps.  With a user-based method:
+        (uid, [(neighbour uid, sim)*])."""
         state = rdd.handle
-        state.knn = RS.item_knn(state.user, state.item, state.rating, len(state.iids), state.num_atleast,
-                                int(self.mapping_range))
-        state.nb = state.knn.nb
+        self._knn(state)
         return self._neighbour_rdd(state)
 
     def nonnoise_perturbation(self, rdd):
@@ -134,10 +163,8 @@ class RecommenderPrivacy(object):
         up, un = self.uniforms if self.uniforms is not None else (None, None)
         seed = (self.seed + 0x9E3779B97F4A7C15 * self._calls) & (2 ** 64 - 1)
         self._calls += 1
-        state.knn = RS.item_knn(state.user, state.item, state.rating, len(state.iids), state.num_atleast,
-                                int(self.mapping_range), private=dict(privacy_epsilon=2 * self.privacy_epsilon, rpo=self.rpo,
-                                                                      u_pick=up, u_noise=un, seed=seed))
-        state.nb = state.knn.nb
+        self._knn(state, private=dict(privacy_epsilon=2 * self.privacy_epsilon, rpo=self.rpo, u_pick=up, u_noise=un,
+                                      seed=seed))
         return self._neighbour_rdd(state)
 
     def noise_perturbation(self, rdd):
@@ -168,6 +195,30 @@ class RecommenderPrediction(object):
                 if str(iid) in state.ipos and str(uid) in state.upos:
                     tu.append(state.upos[str(uid)]); ti.append(state.ipos[str(iid)]); tr.append(float(r)); where.append((a, b))
         p0, p1, _, _ = RS.predict(state.user, state.item, state.rating, state.ts, len(state.uids), state.knn, state.nb,
+                                  np.array(tu, dtype=np.int32), np.array(ti, dtype=np.int32), None, self.alpha)
+        p0, p1 = p0.cpu().numpy(), p1.cpu().numpy()
+        out = [(uid, [() for _ in lst]) for uid, lst in test]
+        for q, (a, b) in enumerate(where):
+            if p0[q] >= 0:
+                iid, r, _t = test[a][1][b]
+                out[a][1][b] = (iid, r, float(p0[q]), float(p1[q]))
+        return LocalRDD(out)
+
+    def user_based_recommendation(self, test_dataRDD, user_based_dict_bd, simpair_dict_bd, user_info_bd):
+        """(uid, [(iid, real rating, prediction, prediction with decay)*])*, shaped like item_based_recommendation's:
+        the user-based prediction (usersim.predict, DESIGN.md 3.9); () where the user has no neighbour list."""
+        state = getattr(getattr(simpair_dict_bd, "value", simpair_dict_bd), "handle", None)
+        if state is None or state.nb is None or state.knn is None or not state.user_based:
+            raise TypeError("expected the user neighbour dictionary returned by recommender_privacy_pipeline "
+                            "(it carries the device-resident tables)")
+        from .. import usersim as US
+        test = records_of(test_dataRDD)
+        tu, ti, where = [], [], []
+        for a, (uid, lst) in enumerate(test):
+            for b, (iid, r, _t) in enumerate(lst):
+                if str(iid) in state.ipos and str(uid) in state.upos:
+                    tu.append(state.upos[str(uid)]); ti.append(state.ipos[str(iid)]); where.append((a, b))
+        p0, p1, _, _ = US.predict(state.user, state.item, state.rating, state.ts, len(state.iids), state.knn, state.nb,
                                   np.array(tu, dtype=np.int32), np.array(ti, dtype=np.int32), None, self.alpha)
         p0, p1 = p0.cpu().numpy(), p1.cpu().numpy()
         out = [(uid, [() for _ in lst]) for uid, lst in test]
@@ -216,13 +267,20 @@ def recommend_top_n(simpair_dict_bd, n, decay=False, alpha=0.03):
     """(uid, [(iid, score)*])* in uid order: every profile user's first n (1..64) items by score, best first.  The
     reference has no such function: the score is its item-based prediction (recommenderPrediction.py:26-103) before
     bound_rating rounds it, without or with temporal decay (weight alpha), over the items with a neighbour list the
-    user has no record on; ties go to the smaller item index (iids ordered as strings).  simpair_dict_bd: what
+    user has no record on; ties go to the smaller item index (iids ordered as strings).  With a user-based method the
+    score is the user-based prediction (DESIGN.md 3.9) over every profile item the user has no record on.  simpair_dict_bd: what
     recommender_privacy_pipeline(...).collectAsMap() returns, or its broadcast."""
     state = getattr(getattr(simpair_dict_bd, "value", simpair_dict_bd), "handle", None)
     if state is None or state.nb is None or state.knn is None:
         raise TypeError("expected the neighbour dictionary returned by recommender_privacy_pipeline "
                         "(it carries the device-resident tables)")
-    res = RS.top_n(state.user, state.item, state.rating, state.ts, len(state.uids), state.knn, state.nb, n, decay, alpha)
+    if state.user_based:
+        from .. import usersim as US
+        res = US.top_n(state.user, state.item, state.rating, state.ts, len(state.uids), len(state.iids), state.knn,
+                       state.nb, n, decay, alpha)
+    else:
+        res = RS.top_n(state.user, state.item, state.rating, state.ts, len(state.uids), state.knn, state.nb, n, decay,
+                       alpha)
     idx, score, ln = res.idx.cpu().numpy(), res.score.cpu().numpy(), res.len.cpu().numpy()
     return LocalRDD([(str(uid), [(str(state.iids[idx[u, p]]), float(score[u, p])) for p in range(ln[u])])
                      for u, uid in enumerate(state.uids)])
@@ -230,8 +288,10 @@ def recommend_top_n(simpair_dict_bd, n, decay=False, alpha=0.03):
 
 def recommender_prediction_pipeline(recommender_tool, cross_sim_tool, testRDD, simpair_dict_bd,
                                     user_based_dict_bd, item_based_dict_bd, user_info_bd, item_info_bd):
-    """assist.py:195-207 (item-based methods)."""
+    """assist.py:195-207: the user-based chain for a method naming "user", else the item-based one."""
     if "user" in cross_sim_tool.method:
-        raise ValueError("user-based recommendation is not offered")
-    predicted = recommender_tool.item_based_recommendation(testRDD, item_based_dict_bd, simpair_dict_bd, item_info_bd)
+        predicted = recommender_tool.user_based_recommendation(testRDD, user_based_dict_bd, simpair_dict_bd, user_info_bd)
+    else:
+        predicted = recommender_tool.item_based_recommendation(testRDD, item_based_dict_bd, simpair_dict_bd,
+                                                               item_info_bd)
     return recommender_tool.calculate_mae(predicted)

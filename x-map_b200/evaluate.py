@@ -123,8 +123,9 @@ def _relevant_csr(A, rel, users, prof_of, n_items):
 
 def evaluate(A, sim_tool, extend_tool, generator, private_gen, rec_sim_tool, privacy_tool, private_rec, n=10,
              threshold=None, alpha=0.03, events=None):
-    """Train arrays -> similarity -> X-SIM -> mapping -> AlterEgo profile -> item-kNN, then the held-out MAE of the
-    test pairs and the top-n accuracy of the test users.  private_gen / private_rec: the generator's private mode and
+    """Train arrays -> similarity -> X-SIM -> mapping -> AlterEgo profile -> item-kNN (or user-kNN when rec_sim_tool's
+    method is "cosine_user" / "adjust_cosine_user", DESIGN.md 3.9), then the held-out MAE of the test pairs and the
+    top-n accuracy of the test users.  private_gen / private_rec: the generator's private mode and
     the private neighbour selection, as generator_pipeline's and recommender_privacy_pipeline's flags.  threshold: a
     held-out record is relevant when its rating >= threshold (None: every one).  events: optional dict that receives
     CUDA-event pairs per stage; their times are then in stage_ms."""
@@ -137,36 +138,44 @@ def evaluate(A, sim_tool, extend_tool, generator, private_gen, rec_sim_tool, pri
     n_users, n_items = len(A.uids), int(profile_items.numel())
     counts["profile_records"], counts["synthetic_records"] = int(pu.numel()), n_synth
 
-    with timer("item_knn"):
-        state = ProfileState.from_arrays(pu, pi, pr, pt, A.uids, A.iids[profile_items.cpu().numpy()])
-        recommender_privacy_pipeline(privacy_tool, rec_sim_tool.calculate_sim(state), private_rec)
-        knn, nb = state.knn, state.nb
-
-    # ---- held-out pairs -> train numbering -> profile numbering ----------------------------------------------------
-    with timer("prediction"):
-        n_test = int(A.test_user.numel())
-        in_prof_user = torch.bincount(pu, minlength=n_users) > 0
-        prof_of, tu, tpi, untrained, no_profile = _test_pairs(A, profile_items, in_prof_user)
-        ok = torch.nonzero(~untrained & ~no_profile).flatten()
-        p0, p1, mae0, mae1 = RS.predict(pu, pi, pr, pt, n_users, knn, nb, tu[ok], tpi[ok], A.test_rating[ok], alpha)
-        pred0 = torch.full((n_test,), -1.0, dtype=torch.float64, device=dev)
-        pred1 = torch.full((n_test,), -1.0, dtype=torch.float64, device=dev)
-        pred0[ok], pred1[ok] = p0, p1
-        n_pred = int((p0 >= 0).sum())
-    counts.update(test_pairs=n_test, predicted=n_pred, skipped_untrained=int(untrained.sum()),
-                  skipped_no_profile=int(no_profile.sum()), skipped_no_neighbours=int(ok.numel()) - n_pred)
-
-    # ---- top-n of the test users with a relevant held-out record -----------------------------------------------------
-    with timer("top_n"):
+    if "cosine_user" in rec_sim_tool.method:
+        top, pred0, pred1, mae0, mae1, catalogue, reachable_of = _user_based(
+            A, pu, pi, pr, pt, profile_items, rec_sim_tool, privacy_tool, private_rec, n, threshold, alpha, timer, counts)
         rel, is_test, has_rel, trained, users, run = _eval_users(A, threshold)
-        top = RS.top_n(pu, pi, pr, pt, n_users, knn, nb, n, alpha=alpha, users=run)
+        in_prof_user = torch.bincount(pu, minlength=n_users) > 0
+        prof_of = _test_pairs(A, profile_items, in_prof_user)[0]
+    else:
+        with timer("item_knn"):
+            state = ProfileState.from_arrays(pu, pi, pr, pt, A.uids, A.iids[profile_items.cpu().numpy()])
+            recommender_privacy_pipeline(privacy_tool, rec_sim_tool.calculate_sim(state), private_rec)
+            knn, nb = state.knn, state.nb
+
+        # ---- held-out pairs -> train numbering -> profile numbering ------------------------------------------------
+        with timer("prediction"):
+            n_test = int(A.test_user.numel())
+            in_prof_user = torch.bincount(pu, minlength=n_users) > 0
+            prof_of, tu, tpi, untrained, no_profile = _test_pairs(A, profile_items, in_prof_user)
+            ok = torch.nonzero(~untrained & ~no_profile).flatten()
+            p0, p1, mae0, mae1 = RS.predict(pu, pi, pr, pt, n_users, knn, nb, tu[ok], tpi[ok], A.test_rating[ok], alpha)
+            pred0 = torch.full((n_test,), -1.0, dtype=torch.float64, device=dev)
+            pred1 = torch.full((n_test,), -1.0, dtype=torch.float64, device=dev)
+            pred0[ok], pred1[ok] = p0, p1
+            n_pred = int((p0 >= 0).sum())
+        counts.update(test_pairs=n_test, predicted=n_pred, skipped_untrained=int(untrained.sum()),
+                      skipped_no_profile=int(no_profile.sum()), skipped_no_neighbours=int(ok.numel()) - n_pred)
+
+        # ---- top-n of the test users with a relevant held-out record -------------------------------------------------
+        with timer("top_n"):
+            rel, is_test, has_rel, trained, users, run = _eval_users(A, threshold)
+            top = RS.top_n(pu, pi, pr, pt, n_users, knn, nb, n, alpha=alpha, users=run)
+        catalogue = int((nb.len > 0).sum())
+        reachable_of = nb.len > 0
     with timer("rank_metrics"):
         rel_ptr, code = _relevant_csr(A, rel, users, prof_of, n_items)
-        catalogue = int((nb.len > 0).sum())
         metrics = RS.rank_metrics(top, run, rel_ptr, code, n, catalogue=catalogue)
         reachable = torch.zeros(int(code.numel()), dtype=torch.bool, device=dev)
         in_prof = code < n_items
-        reachable[in_prof] = nb.len[code[in_prof]] > 0
+        reachable[in_prof] = reachable_of[code[in_prof]]
     counts.update(eval_users=int(users.numel()), eval_users_without_profile=int((~in_prof_user[run]).sum()),
                   test_users_untrained=int((has_rel & ~trained).sum()),
                   test_users_without_relevant=int(len(A.test_users)) - int((has_rel & is_test).sum()),
@@ -177,6 +186,53 @@ def evaluate(A, sim_tool, extend_tool, generator, private_gen, rec_sim_tool, pri
         torch.cuda.synchronize(dev)
         stage_ms = {k: sum(a.elapsed_time(b) for a, b in v) for k, v in events.items()}
     return Evaluation(mae0, mae1, pred0, pred1, users, metrics, top, profile_items, n, counts, stage_ms)
+
+
+def _user_based(A, pu, pi, pr, pt, profile_items, rec_sim_tool, privacy_tool, private_rec, n, threshold, alpha, timer,
+                counts):
+    """The user-based chain of evaluate (DESIGN.md 3.9).  Users are renumbered by rank among the profile's users, as the
+    facade's np.unique over id strings numbers them (ties and private draws go by that index); only the rows of the
+    users with a held-out pair or a list to rank are computed.  Returns (top with rows by train user, pred0, pred1,
+    mae0, mae1, catalogue, which profile items can be listed)."""
+    from . import usersim as US
+    dev = A.user.device
+    n_users, n_items = len(A.uids), int(profile_items.numel())
+    profile_users, qu = torch.unique(pu, return_inverse=True)
+    n_pu = int(profile_users.numel())
+    q_of = torch.full((n_users,), -1, dtype=torch.int64, device=dev)
+    q_of[profile_users] = torch.arange(n_pu, device=dev)
+    in_prof_user = q_of >= 0
+    with timer("prediction_pairs"):
+        n_test = int(A.test_user.numel())
+        _, tu, tpi, untrained, no_profile = _test_pairs(A, profile_items, in_prof_user)
+        ok = torch.nonzero(~untrained & ~no_profile).flatten()
+        rel, is_test, has_rel, trained, users, run = _eval_users(A, threshold)
+        run_q = q_of[run]
+        query = torch.unique(torch.cat([q_of[tu[ok]], run_q[run_q >= 0]]))
+    with timer("user_knn"):
+        state = ProfileState.from_arrays(qu, pi, pr, pt, A.uids[profile_users.cpu().numpy()],
+                                         A.iids[profile_items.cpu().numpy()])
+        state.query_users = query
+        recommender_privacy_pipeline(privacy_tool, rec_sim_tool.calculate_sim(state), private_rec)
+        knn, nb = state.knn, state.nb
+    with timer("prediction"):
+        p0, p1, mae0, mae1 = US.predict(qu, pi, pr, pt, n_items, knn, nb, q_of[tu[ok]], tpi[ok], A.test_rating[ok],
+                                        alpha)
+        pred0 = torch.full((n_test,), -1.0, dtype=torch.float64, device=dev)
+        pred1 = torch.full((n_test,), -1.0, dtype=torch.float64, device=dev)
+        pred0[ok], pred1[ok] = p0, p1
+        n_pred = int((p0 >= 0).sum())
+    counts.update(test_pairs=n_test, predicted=n_pred, skipped_untrained=int(untrained.sum()),
+                  skipped_no_profile=int(no_profile.sum()), skipped_no_neighbours=int(ok.numel()) - n_pred)
+    with timer("top_n"):
+        t = US.top_n(qu, pi, pr, pt, n_pu, n_items, knn, nb, n, alpha=alpha, users=run_q[run_q >= 0])
+        idx = torch.full((n_users, n), -1, dtype=torch.int32, device=dev)
+        score = torch.full((n_users, n), float("nan"), dtype=torch.float64, device=dev)
+        ln = torch.zeros(n_users, dtype=torch.int32, device=dev)
+        idx[profile_users], score[profile_users], ln[profile_users] = t.idx, t.score, t.len
+        top = RS.TopN(idx, score, ln, t.visits, t.candidates, t.warp_users, t.cta_users)
+    # every profile item can be listed for a user without a record on it
+    return top, pred0, pred1, mae0, mae1, n_items, torch.ones(n_items, dtype=torch.bool, device=dev)
 
 
 @dataclass
