@@ -242,18 +242,12 @@ def _pairs_user(prof, cta, tile):
     rows = torch.arange(prof.n_users, dtype=torch.int64, device=prof.dev)
     stats = torch.zeros(3, dtype=torch.int64, device=prof.dev)
     err = torch.zeros(1, dtype=torch.int32, device=prof.dev)
-    parts = []
-    for r, (e_ptr, e_v, e_n, e_sim, e_ls, e_len) in usersim._emit_blocks(prof, [(rows, cta)], 50, 1 << 30, tile, None,
-                                                                         stats, err):
-        row_of = torch.repeat_interleave(torch.arange(int(r.numel()), device=prof.dev), e_ptr[1:] - e_ptr[:-1])
-        keep = torch.arange(int(row_of.numel()), device=prof.dev) - e_ptr[:-1][row_of] < e_len[row_of]
-        parts.append((r[row_of[keep]], e_v[:row_of.numel()][keep], e_n[:row_of.numel()][keep],
-                      e_sim[:row_of.numel()][keep], e_ls[:row_of.numel()][keep]))
+    parts = [blk[1:] for blk in usersim._emit_blocks(prof, [(rows, cta)], 50, 1 << 30, tile, None, stats, err)]
     return [torch.cat([p[f] for p in parts]) for f in range(5)]
 
 
 @pytest.mark.parametrize("crafted", [False, True])
-def test_emitted_pairs_and_nan_first_rule(crafted):
+def test_emitted_block_pairs_and_nan_first_rule(crafted):
     """Every emitted (u, v, n, sim, ls) equals recsim's pair kernel on the transposed profile, NaN pattern included.
     With finite ratings and true norms no deviation is NaN (norm_u >= |r| for each of u's records), so the crafted case
     sets each user's norm just below its largest |rating|: the records at that rating then give a NaN first deviation,

@@ -57,13 +57,13 @@ def test_scale_base_and_exponents():
     assert e.tolist() == [0, 0, 1, 1, 2, 10]           # 2^(E-1) <= norm < 2^E
 
 
-def test_emit_plan_respects_the_budget():
-    from xmap_b200 import recsim, usersim
+def test_emit_blocks_plan_respects_the_budget():
+    from xmap_b200 import recsim
     bound = torch.tensor([3, 0, 7, 1, 1, 10, 2], dtype=torch.int64)
     budget = 10 * recsim.ENTRY_BYTES
-    b = usersim.emit_plan(bound, budget)
+    b = recsim.pass_plan(bound, budget)
     assert b[0] == 0 and b[-1] == len(bound)
     for lo, hi in zip(b[:-1], b[1:]):
         assert hi > lo and int(bound[lo:hi].sum()) * recsim.ENTRY_BYTES <= budget
     with pytest.raises(ValueError):
-        usersim.emit_plan(torch.tensor([11]), budget)
+        recsim.pass_plan(torch.tensor([11]), budget)

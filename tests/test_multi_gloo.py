@@ -1,8 +1,10 @@
-"""CPU, world_size 2, gloo: work-balanced row sharding, the neighbour-record exchange and the table all-gather."""
+"""CPU, gloo: work-balanced row sharding, the neighbour-record exchange, the table all-gather and the gather of
+selected rows."""
 import os
 import socket
 
 import numpy as np
+import pytest
 import torch
 import torch.distributed as dist
 import torch.multiprocessing as mp
@@ -58,6 +60,51 @@ def test_row_shard_and_allgather_world2():
     assert all(ok for _, ok, _ in res)
     loads = res[0][2]
     assert max(loads) / (sum(loads) / 2) < 1.25        # blocks balanced by work, not by row count
+
+
+def _selected_worker(rank, world, port, q):
+    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
+    dist.init_process_group("gloo", rank=rank, world_size=world)
+    from xmap_b200.multi import gather_selected, shard_selected
+    n_rows, width = 500, 3
+    g = torch.Generator().manual_seed(7)
+    work = (torch.rand(n_rows, generator=g) ** 4 * 1e4).long()
+    subset = torch.randperm(n_rows, generator=g)[:317]          # a permuted subset of the rows
+
+    def lists(rows):                   # top-N-shaped tables with the rows `rows` filled by a function of the row
+        t = [torch.full((n_rows, width), -1, dtype=torch.int32), torch.full((n_rows, width), -1.0, dtype=torch.float64),
+             torch.zeros(n_rows, dtype=torch.int32)]
+        t[0][rows] = (rows.unsqueeze(1) * 10 + torch.arange(width)).int()
+        t[1][rows] = rows.unsqueeze(1).double() / 7.0 + torch.arange(width)
+        t[2][rows] = (rows % (width + 1)).int()
+        return t
+    ok = True
+    for sel in (subset, None):
+        rows = torch.arange(n_rows) if sel is None else sel
+        sh, mine = shard_selected(rows, work[rows])
+        got = lists(mine)
+        gather_selected(got, sh, sel)
+        ok = ok and all(bool(torch.equal(a, b)) for a, b in zip(got, lists(rows)))
+    q.put((rank, ok))
+    dist.destroy_process_group()
+
+
+@pytest.mark.parametrize("world", [2, 3])
+def test_gather_selected_rows_equals_unsharded(world):
+    """The shard-then-gather of the sharded top-N and user-kNN calls, on a permuted subset of the rows and on every
+    row in order: every rank ends with the tables one process computing every selected row would hold."""
+    from tests import parity  # noqa: F401
+    ctx = mp.get_context("spawn")
+    q = ctx.Queue()
+    port = _free_port()
+    procs = [ctx.Process(target=_selected_worker, args=(r, world, port, q)) for r in range(world)]
+    for p in procs:
+        p.start()
+    res = [q.get(timeout=120) for _ in procs]
+    for p in procs:
+        p.join(60)
+        assert p.exitcode == 0
+    assert all(ok for _, ok in res)
 
 
 def _exchange_worker(rank, world, port, q):

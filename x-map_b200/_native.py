@@ -7,6 +7,8 @@ g; g.build()"`` (nvcc, sm_100a).
 import ctypes as C
 import os
 
+import torch
+
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("XMAP_B200_LIB") or os.path.join(_HERE, "libxmap_b200.so")
 
@@ -161,3 +163,8 @@ def check(rc, what):
 def ptr(t):
     """Device pointer of a torch tensor (None -> NULL)."""
     return None if t is None else t.data_ptr()
+
+
+def stream():
+    """The current torch CUDA stream, which every launch of the C ABI takes."""
+    return torch.cuda.current_stream().cuda_stream

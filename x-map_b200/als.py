@@ -12,15 +12,13 @@ from dataclasses import dataclass
 import torch
 
 from . import _native as N
+from . import multi as M
+from . import recsim as RS
 
 SEGMENT = N.ALS_SEGMENT
 # Bytes of segment partials (fp64 normal equations) one normal / solve launch pair may hold: the rows of a half-step
 # are cut into launches under it.  The factors do not depend on it; tests shrink it to run many launches.
 SCRATCH_BYTES = 1 << 31
-
-
-def _st():
-    return torch.cuda.current_stream().cuda_stream
 
 
 @dataclass
@@ -117,10 +115,10 @@ class _Side(object):
         for rows, seg_ptr, n, seg_lo, seg_n, total in self.launches:
             with _phase(timer, "normal"):
                 N.check(L.xmap_als_normal(N.ptr(self.col), N.ptr(self.rating), N.ptr(seg_lo), N.ptr(seg_n), total,
-                                          N.ptr(other), rank, N.ptr(partial), _st()), "xmap_als_normal")
+                                          N.ptr(other), rank, N.ptr(partial), N.stream()), "xmap_als_normal")
             with _phase(timer, "solve"):
                 N.check(L.xmap_als_solve(N.ptr(rows), N.ptr(seg_ptr), N.ptr(n), int(rows.numel()), N.ptr(partial),
-                                         rank, float(lam), N.ptr(out), N.ptr(status), _st()), "xmap_als_solve")
+                                         rank, float(lam), N.ptr(out), N.ptr(status), N.stream()), "xmap_als_solve")
         return out, status
 
 
@@ -156,7 +154,7 @@ def init_factors(n_rows, rank, seed=None, device="cuda"):
     rank = _int(rank, "rank", 1, N.ALS_RANK_MAX)
     seed = 0 if seed is None else _int(seed, "seed", 0, 2 ** 64 - 1)
     X = torch.empty((n_rows, rank), dtype=torch.float32, device=device)
-    N.check(N.lib().xmap_als_init(n_rows, rank, seed, N.ptr(X), _st()), "xmap_als_init")
+    N.check(N.lib().xmap_als_init(n_rows, rank, seed, N.ptr(X), N.stream()), "xmap_als_init")
     return X
 
 
@@ -186,11 +184,9 @@ def train(user, item, rating, n_users, n_items, rank, iterations, lam, seed=None
     N.lib()
     sh_u = sh_i = None
     if shard:
-        import torch.distributed as dist
-        from .multi import RowShard
-        rk, world = dist.get_rank(group), dist.get_world_size(group)
-        sh_i = RowShard(torch.bincount(i, minlength=n_items), rk, world)
-        sh_u = RowShard(torch.bincount(u, minlength=n_users), rk, world)
+        rk, world = M.dist.get_rank(group), M.dist.get_world_size(group)
+        sh_i = M.RowShard(torch.bincount(i, minlength=n_items), rk, world)
+        sh_u = M.RowShard(torch.bincount(u, minlength=n_users), rk, world)
     items = _Side(i, u, r, n_items, rank, *((sh_i.lo, sh_i.hi) if sh_i else (0, n_items)))
     users = _Side(u, i, r, n_users, rank, *((sh_u.lo, sh_u.hi) if sh_u else (0, n_users)))
     X = init.to(dev).contiguous().clone() if init is not None else init_factors(n_users, rank, seed, dev)
@@ -201,8 +197,7 @@ def train(user, item, rating, n_users, n_items, rank, iterations, lam, seed=None
             timer = {} if events is not None else None
             out, status = side.solve(X if name == "item" else Y, rank, lam, name, timer)
             if sh is not None:
-                from .multi import allgather_rows
-                allgather_rows([out, status], sh, group)
+                M.allgather_rows([out, status], sh, group)
             _check_status(status, name, lam)
             if name == "item":
                 Y = out
@@ -228,7 +223,7 @@ def predict(model, u, i):
     pu32, pi32 = pu.to(torch.int32).contiguous(), pi.to(torch.int32).contiguous()
     N.check(N.lib().xmap_als_predict(N.ptr(model.user_factors), N.ptr(model.item_factors), N.ptr(model.user_count),
                                      N.ptr(model.item_count), model.rank, N.ptr(pu32), N.ptr(pi32), int(pu.numel()),
-                                     N.ptr(out), _st()), "xmap_als_predict")
+                                     N.ptr(out), N.stream()), "xmap_als_predict")
     return out
 
 
@@ -241,16 +236,6 @@ class AlsTopN:
     candidates: int          # candidate items with factors
 
 
-def _index_set(t, n_max, name, dev):
-    t = torch.as_tensor(t)
-    if t.dim() != 1 or t.dtype.is_floating_point or t.dtype.is_complex or t.dtype == torch.bool:
-        raise ValueError("%s must be a 1-D integer tensor" % name)
-    t = t.to(device=dev, dtype=torch.int64)
-    if t.numel() and (int(t.min()) < 0 or int(t.max()) >= n_max):
-        raise ValueError("%s outside [0, %d)" % (name, n_max))
-    return t
-
-
 def top_n(model, n, user=None, item=None, candidates=None, users=None, exclude_rated=True, shard=False, group=None):
     """Each user's first n (1 <= n <= 64) candidate items by score descending, then the smaller item index (-0.0
     equals 0.0; a NaN score is never listed).  candidates: ascending distinct items (None: every item); items without
@@ -258,7 +243,7 @@ def top_n(model, n, user=None, item=None, candidates=None, users=None, exclude_r
     users: None for every user, or distinct users whose rows alone are filled (the others keep the padding).  A user
     without factors gets an empty list.  shard: split the users over the ranks of `group` and all-gather the lists.
     The result does not depend on the launch shape, the tiling or the world size."""
-    n = _int(n, "n", 1, N.TOPN_MAX)
+    n = RS.list_length(n)
     dev = model.user_factors.device
     n_users, n_items = int(model.user_factors.shape[0]), int(model.item_factors.shape[0])
     rated_ptr = rated_item = None
@@ -273,34 +258,18 @@ def top_n(model, n, user=None, item=None, candidates=None, users=None, exclude_r
     if candidates is None:
         cand = torch.arange(n_items, device=dev)
     else:
-        cand = _index_set(candidates, n_items, "candidates", dev)
+        cand = RS.index_set(candidates, n_items, dev, "candidates")
         if cand.numel() > 1 and bool((cand[1:] <= cand[:-1]).any()):
             raise ValueError("candidates must be ascending and distinct")
     cand = cand[model.item_count[cand] > 0].to(torch.int32).contiguous()
-    if users is None:
-        sel = torch.arange(n_users, device=dev)
-    else:
-        sel = _index_set(users, n_users, "users", dev)
-        if int(torch.unique(sel).numel()) != int(sel.numel()):
-            raise ValueError("users must be distinct")
-    sh = None
-    mine = sel
-    if shard:
-        import torch.distributed as dist
-        from .multi import RowShard
-        sh = RowShard(torch.zeros(int(sel.numel()), device=dev), dist.get_rank(group), dist.get_world_size(group))
-        mine = sel[sh.lo:sh.hi]
+    sel = RS.query_users(users, n_users, dev)
+    sh, mine = M.shard_selected(sel, torch.zeros(int(sel.numel()), device=dev), group) if shard else (None, sel)
     run = mine[model.user_count[mine] > 0].to(torch.int32).contiguous()
-    out_idx = torch.full((n_users, n), -1, dtype=torch.int32, device=dev)
-    out_score = torch.full((n_users, n), float("nan"), dtype=torch.float64, device=dev)
-    out_len = torch.zeros(n_users, dtype=torch.int32, device=dev)
+    out_idx, out_score, out_len = RS.empty_lists(n_users, n, dev)
     N.check(N.lib().xmap_als_top_n(N.ptr(model.user_factors), N.ptr(model.item_factors), model.rank, N.ptr(run),
                                    int(run.numel()), N.ptr(cand), int(cand.numel()), N.ptr(rated_ptr),
-                                   N.ptr(rated_item), n, N.ptr(out_idx), N.ptr(out_score), N.ptr(out_len), _st()),
+                                   N.ptr(rated_item), n, N.ptr(out_idx), N.ptr(out_score), N.ptr(out_len), N.stream()),
             "xmap_als_top_n")
     if sh is not None:
-        from .multi import allgather_rows
-        rows = [out_idx[sel], out_score[sel], out_len[sel]]      # the selected rows side by side, in the order of sel
-        allgather_rows(rows, sh, group)
-        out_idx[sel], out_score[sel], out_len[sel] = rows
+        M.gather_selected([out_idx, out_score, out_len], sh, None if users is None else sel, group)
     return AlsTopN(out_idx, out_score, out_len, int(cand.numel()))

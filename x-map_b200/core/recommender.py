@@ -188,21 +188,7 @@ class RecommenderPrediction(object):
         if state is None or state.nb is None or state.knn is None:
             raise TypeError("expected the neighbour dictionary returned by recommender_privacy_pipeline "
                             "(it carries the device-resident tables)")
-        test = records_of(test_dataRDD)
-        tu, ti, tr, where = [], [], [], []
-        for a, (uid, lst) in enumerate(test):
-            for b, (iid, r, _t) in enumerate(lst):
-                if str(iid) in state.ipos and str(uid) in state.upos:
-                    tu.append(state.upos[str(uid)]); ti.append(state.ipos[str(iid)]); tr.append(float(r)); where.append((a, b))
-        p0, p1, _, _ = RS.predict(state.user, state.item, state.rating, state.ts, len(state.uids), state.knn, state.nb,
-                                  np.array(tu, dtype=np.int32), np.array(ti, dtype=np.int32), None, self.alpha)
-        p0, p1 = p0.cpu().numpy(), p1.cpu().numpy()
-        out = [(uid, [() for _ in lst]) for uid, lst in test]
-        for q, (a, b) in enumerate(where):
-            if p0[q] >= 0:
-                iid, r, _t = test[a][1][b]
-                out[a][1][b] = (iid, r, float(p0[q]), float(p1[q]))
-        return LocalRDD(out)
+        return self._recommend(test_dataRDD, state, RS.predict, len(state.uids))
 
     def user_based_recommendation(self, test_dataRDD, user_based_dict_bd, simpair_dict_bd, user_info_bd):
         """(uid, [(iid, real rating, prediction, prediction with decay)*])*, shaped like item_based_recommendation's:
@@ -212,14 +198,19 @@ class RecommenderPrediction(object):
             raise TypeError("expected the user neighbour dictionary returned by recommender_privacy_pipeline "
                             "(it carries the device-resident tables)")
         from .. import usersim as US
+        return self._recommend(test_dataRDD, state, US.predict, len(state.iids))
+
+    def _recommend(self, test_dataRDD, state, predict, n_rows):
+        """The test records with the predictions of `predict` (recsim.predict or usersim.predict on the profile of
+        state, n_rows its n_users / n_items argument) filled in where the user and the item are in the profile."""
         test = records_of(test_dataRDD)
         tu, ti, where = [], [], []
         for a, (uid, lst) in enumerate(test):
             for b, (iid, r, _t) in enumerate(lst):
                 if str(iid) in state.ipos and str(uid) in state.upos:
                     tu.append(state.upos[str(uid)]); ti.append(state.ipos[str(iid)]); where.append((a, b))
-        p0, p1, _, _ = US.predict(state.user, state.item, state.rating, state.ts, len(state.iids), state.knn, state.nb,
-                                  np.array(tu, dtype=np.int32), np.array(ti, dtype=np.int32), None, self.alpha)
+        p0, p1, _, _ = predict(state.user, state.item, state.rating, state.ts, n_rows, state.knn, state.nb,
+                               np.array(tu, dtype=np.int32), np.array(ti, dtype=np.int32), None, self.alpha)
         p0, p1 = p0.cpu().numpy(), p1.cpu().numpy()
         out = [(uid, [() for _ in lst]) for uid, lst in test]
         for q, (a, b) in enumerate(where):

@@ -71,18 +71,35 @@ def _alterego_profile(A, sim_tool, extend_tool, generator, private_gen, timer):
     return pu, pi, pr, pt, profile_items, int(ou.numel())
 
 
+def _profile_index(A, profile_items):
+    """The profile index of every train item, -1 outside the profile."""
+    prof_of = torch.full((len(A.iids),), -1, dtype=torch.int64, device=A.user.device)
+    prof_of[profile_items] = torch.arange(int(profile_items.numel()), device=A.user.device)
+    return prof_of
+
+
 def _test_pairs(A, profile_items, in_prof_user):
-    """The held-out pairs in train numbering and then in profile numbering: (prof_of, tu, tpi, untrained,
-    no_profile); prof_of maps a train item to its profile index (-1 outside the profile)."""
-    dev = A.user.device
-    prof_of = torch.full((len(A.iids),), -1, dtype=torch.int64, device=dev)
-    prof_of[profile_items] = torch.arange(int(profile_items.numel()), device=dev)
+    """The held-out pairs in train numbering and then in profile numbering: (tu, tpi, untrained, no_profile)."""
     tu = A.train_user_of[A.test_user.long()].long()
     ti = A.train_item_of[A.test_item.long()].long()
     untrained = (tu < 0) | (ti < 0)
-    tpi = torch.where(untrained, -1, prof_of[ti.clamp(min=0)])
+    tpi = torch.where(untrained, -1, _profile_index(A, profile_items)[ti.clamp(min=0)])
     no_profile = ~untrained & ((tpi < 0) | ~in_prof_user[tu.clamp(min=0)])
-    return prof_of, tu, tpi, untrained, no_profile
+    return tu, tpi, untrained, no_profile
+
+
+def _scatter_predictions(counts, ok, preds, fill, untrained, no_profile, predicted, **skipped):
+    """preds (values of the held-out pairs ok) spread over every held-out pair, `fill` elsewhere; the pair counts go
+    into counts, the model's own reasons to skip a pair in `skipped`."""
+    n_test = int(untrained.numel())
+    out = []
+    for p in preds:
+        full = torch.full((n_test,), fill, dtype=torch.float64, device=p.device)
+        full[ok] = p
+        out.append(full)
+    counts.update(test_pairs=n_test, predicted=predicted, skipped_untrained=int(untrained.sum()),
+                  skipped_no_profile=int(no_profile.sum()), **skipped)
+    return out
 
 
 def _eval_users(A, threshold):
@@ -102,17 +119,18 @@ def _eval_users(A, threshold):
     return rel, is_test, has_rel, trained, users, run
 
 
-def _relevant_csr(A, rel, users, prof_of, n_items):
+def _relevant_csr(A, rel, users, profile_items):
     """Each evaluated user's relevant items in profile numbering, sorted and unique: (rel_ptr, code).  An item outside
     the profile gets a code past every profile item."""
     dev = A.user.device
+    n_items = int(profile_items.numel())
     q_of = torch.full((len(A.all_uids),), -1, dtype=torch.int64, device=dev)
     q_of[users] = torch.arange(int(users.numel()), device=dev)
     rq = q_of[A.test_user.long()[rel]]
     keep_r = rq >= 0
     rq, ri_all = rq[keep_r], A.test_item.long()[rel][keep_r]
     rti = A.train_item_of[ri_all].long()
-    code = torch.where(rti >= 0, prof_of[rti.clamp(min=0)], -1)
+    code = torch.where(rti >= 0, _profile_index(A, profile_items)[rti.clamp(min=0)], -1)
     code = torch.where(code >= 0, code, n_items + ri_all)
     key = torch.unique(rq * (n_items + len(A.all_iids)) + code)
     rq, code = key // (n_items + len(A.all_iids)), key % (n_items + len(A.all_iids))
@@ -129,71 +147,50 @@ def evaluate(A, sim_tool, extend_tool, generator, private_gen, rec_sim_tool, pri
     the private neighbour selection, as generator_pipeline's and recommender_privacy_pipeline's flags.  threshold: a
     held-out record is relevant when its rating >= threshold (None: every one).  events: optional dict that receives
     CUDA-event pairs per stage; their times are then in stage_ms."""
-    dev = A.user.device
     timer = I._Timer(events)
     counts = {}
 
     # ---- AlterEgo profile, in the facade's list order: target records in training order, then the synthetic ones ----
     pu, pi, pr, pt, profile_items, n_synth = _alterego_profile(A, sim_tool, extend_tool, generator, private_gen, timer)
-    n_users, n_items = len(A.uids), int(profile_items.numel())
     counts["profile_records"], counts["synthetic_records"] = int(pu.numel()), n_synth
-
-    if "cosine_user" in rec_sim_tool.method:
-        top, pred0, pred1, mae0, mae1, catalogue, reachable_of = _user_based(
-            A, pu, pi, pr, pt, profile_items, rec_sim_tool, privacy_tool, private_rec, n, threshold, alpha, timer, counts)
-        rel, is_test, has_rel, trained, users, run = _eval_users(A, threshold)
-        in_prof_user = torch.bincount(pu, minlength=n_users) > 0
-        prof_of = _test_pairs(A, profile_items, in_prof_user)[0]
-    else:
-        with timer("item_knn"):
-            state = ProfileState.from_arrays(pu, pi, pr, pt, A.uids, A.iids[profile_items.cpu().numpy()])
-            recommender_privacy_pipeline(privacy_tool, rec_sim_tool.calculate_sim(state), private_rec)
-            knn, nb = state.knn, state.nb
-
-        # ---- held-out pairs -> train numbering -> profile numbering ------------------------------------------------
-        with timer("prediction"):
-            n_test = int(A.test_user.numel())
-            in_prof_user = torch.bincount(pu, minlength=n_users) > 0
-            prof_of, tu, tpi, untrained, no_profile = _test_pairs(A, profile_items, in_prof_user)
-            ok = torch.nonzero(~untrained & ~no_profile).flatten()
-            p0, p1, mae0, mae1 = RS.predict(pu, pi, pr, pt, n_users, knn, nb, tu[ok], tpi[ok], A.test_rating[ok], alpha)
-            pred0 = torch.full((n_test,), -1.0, dtype=torch.float64, device=dev)
-            pred1 = torch.full((n_test,), -1.0, dtype=torch.float64, device=dev)
-            pred0[ok], pred1[ok] = p0, p1
-            n_pred = int((p0 >= 0).sum())
-        counts.update(test_pairs=n_test, predicted=n_pred, skipped_untrained=int(untrained.sum()),
-                      skipped_no_profile=int(no_profile.sum()), skipped_no_neighbours=int(ok.numel()) - n_pred)
-
-        # ---- top-n of the test users with a relevant held-out record -------------------------------------------------
-        with timer("top_n"):
-            rel, is_test, has_rel, trained, users, run = _eval_users(A, threshold)
-            top = RS.top_n(pu, pi, pr, pt, n_users, knn, nb, n, alpha=alpha, users=run)
-        catalogue = int((nb.len > 0).sum())
-        reachable_of = nb.len > 0
-    with timer("rank_metrics"):
-        rel_ptr, code = _relevant_csr(A, rel, users, prof_of, n_items)
-        metrics = RS.rank_metrics(top, run, rel_ptr, code, n, catalogue=catalogue)
-        reachable = torch.zeros(int(code.numel()), dtype=torch.bool, device=dev)
-        in_prof = code < n_items
-        reachable[in_prof] = reachable_of[code[in_prof]]
-    counts.update(eval_users=int(users.numel()), eval_users_without_profile=int((~in_prof_user[run]).sum()),
-                  test_users_untrained=int((has_rel & ~trained).sum()),
-                  test_users_without_relevant=int(len(A.test_users)) - int((has_rel & is_test).sum()),
-                  relevant_items=int(code.numel()), unreachable_items=int((~reachable).sum()),
-                  catalogue_items=catalogue)
-    stage_ms = None
-    if events is not None:
-        torch.cuda.synchronize(dev)
-        stage_ms = {k: sum(a.elapsed_time(b) for a, b in v) for k, v in events.items()}
-    return Evaluation(mae0, mae1, pred0, pred1, users, metrics, top, profile_items, n, counts, stage_ms)
+    ev = _eval_users(A, threshold)
+    users, run = ev[-2:]
+    in_prof_user = torch.bincount(pu, minlength=len(A.uids)) > 0
+    chain = _user_based if "cosine_user" in rec_sim_tool.method else _item_based
+    top, pred0, pred1, mae0, mae1, listable = chain(A, pu, pi, pr, pt, profile_items, in_prof_user, run, rec_sim_tool,
+                                                    privacy_tool, private_rec, n, alpha, timer, counts)
+    metrics = _rank_tail(A, ev, top, profile_items, listable, n, timer, counts,
+                         eval_users_without_profile=int((~in_prof_user[run]).sum()))
+    return Evaluation(mae0, mae1, pred0, pred1, users, metrics, top, profile_items, n, counts, timer.stage_ms())
 
 
-def _user_based(A, pu, pi, pr, pt, profile_items, rec_sim_tool, privacy_tool, private_rec, n, threshold, alpha, timer,
-                counts):
+def _item_based(A, pu, pi, pr, pt, profile_items, in_prof_user, run, rec_sim_tool, privacy_tool, private_rec, n,
+                alpha, timer, counts):
+    """The item-based chain of evaluate: item-kNN, the prediction of the held-out pairs and the top-n of the train
+    users `run`.  Returns (top, pred0, pred1, mae0, mae1, which profile items can be listed)."""
+    n_users = len(A.uids)
+    with timer("item_knn"):
+        state = ProfileState.from_arrays(pu, pi, pr, pt, A.uids, A.iids[profile_items.cpu().numpy()])
+        recommender_privacy_pipeline(privacy_tool, rec_sim_tool.calculate_sim(state), private_rec)
+        knn, nb = state.knn, state.nb
+    with timer("prediction"):
+        tu, tpi, untrained, no_profile = _test_pairs(A, profile_items, in_prof_user)
+        ok = torch.nonzero(~untrained & ~no_profile).flatten()
+        p0, p1, mae0, mae1 = RS.predict(pu, pi, pr, pt, n_users, knn, nb, tu[ok], tpi[ok], A.test_rating[ok], alpha)
+    n_pred = int((p0 >= 0).sum())
+    pred0, pred1 = _scatter_predictions(counts, ok, (p0, p1), -1.0, untrained, no_profile, n_pred,
+                                        skipped_no_neighbours=int(ok.numel()) - n_pred)
+    with timer("top_n"):
+        top = RS.top_n(pu, pi, pr, pt, n_users, knn, nb, n, alpha=alpha, users=run)
+    return top, pred0, pred1, mae0, mae1, nb.len > 0
+
+
+def _user_based(A, pu, pi, pr, pt, profile_items, in_prof_user, run, rec_sim_tool, privacy_tool, private_rec, n,
+                alpha, timer, counts):
     """The user-based chain of evaluate (DESIGN.md 3.9).  Users are renumbered by rank among the profile's users, as the
     facade's np.unique over id strings numbers them (ties and private draws go by that index); only the rows of the
-    users with a held-out pair or a list to rank are computed.  Returns (top with rows by train user, pred0, pred1,
-    mae0, mae1, catalogue, which profile items can be listed)."""
+    users with a held-out pair or a list to rank are computed.  Returns what _item_based returns, top's rows by train
+    user."""
     from . import usersim as US
     dev = A.user.device
     n_users, n_items = len(A.uids), int(profile_items.numel())
@@ -201,12 +198,9 @@ def _user_based(A, pu, pi, pr, pt, profile_items, rec_sim_tool, privacy_tool, pr
     n_pu = int(profile_users.numel())
     q_of = torch.full((n_users,), -1, dtype=torch.int64, device=dev)
     q_of[profile_users] = torch.arange(n_pu, device=dev)
-    in_prof_user = q_of >= 0
     with timer("prediction_pairs"):
-        n_test = int(A.test_user.numel())
-        _, tu, tpi, untrained, no_profile = _test_pairs(A, profile_items, in_prof_user)
+        tu, tpi, untrained, no_profile = _test_pairs(A, profile_items, in_prof_user)
         ok = torch.nonzero(~untrained & ~no_profile).flatten()
-        rel, is_test, has_rel, trained, users, run = _eval_users(A, threshold)
         run_q = q_of[run]
         query = torch.unique(torch.cat([q_of[tu[ok]], run_q[run_q >= 0]]))
     with timer("user_knn"):
@@ -218,21 +212,36 @@ def _user_based(A, pu, pi, pr, pt, profile_items, rec_sim_tool, privacy_tool, pr
     with timer("prediction"):
         p0, p1, mae0, mae1 = US.predict(qu, pi, pr, pt, n_items, knn, nb, q_of[tu[ok]], tpi[ok], A.test_rating[ok],
                                         alpha)
-        pred0 = torch.full((n_test,), -1.0, dtype=torch.float64, device=dev)
-        pred1 = torch.full((n_test,), -1.0, dtype=torch.float64, device=dev)
-        pred0[ok], pred1[ok] = p0, p1
-        n_pred = int((p0 >= 0).sum())
-    counts.update(test_pairs=n_test, predicted=n_pred, skipped_untrained=int(untrained.sum()),
-                  skipped_no_profile=int(no_profile.sum()), skipped_no_neighbours=int(ok.numel()) - n_pred)
+    n_pred = int((p0 >= 0).sum())
+    pred0, pred1 = _scatter_predictions(counts, ok, (p0, p1), -1.0, untrained, no_profile, n_pred,
+                                        skipped_no_neighbours=int(ok.numel()) - n_pred)
     with timer("top_n"):
         t = US.top_n(qu, pi, pr, pt, n_pu, n_items, knn, nb, n, alpha=alpha, users=run_q[run_q >= 0])
-        idx = torch.full((n_users, n), -1, dtype=torch.int32, device=dev)
-        score = torch.full((n_users, n), float("nan"), dtype=torch.float64, device=dev)
-        ln = torch.zeros(n_users, dtype=torch.int32, device=dev)
+        idx, score, ln = RS.empty_lists(n_users, n, dev)
         idx[profile_users], score[profile_users], ln[profile_users] = t.idx, t.score, t.len
         top = RS.TopN(idx, score, ln, t.visits, t.candidates, t.warp_users, t.cta_users)
     # every profile item can be listed for a user without a record on it
-    return top, pred0, pred1, mae0, mae1, n_items, torch.ones(n_items, dtype=torch.bool, device=dev)
+    return top, pred0, pred1, mae0, mae1, torch.ones(n_items, dtype=torch.bool, device=dev)
+
+
+def _rank_tail(A, ev, top, profile_items, listable, n, timer, counts, **model_count):
+    """rank_metrics of the evaluated users' lists against their relevant held-out items (ev: _eval_users; listable:
+    which profile items a list can hold, the catalogue), and the counts that do not depend on the model, with
+    model_count (the one that does) in its place among them."""
+    rel, is_test, has_rel, trained, users, run = ev
+    n_items = int(profile_items.numel())
+    with timer("rank_metrics"):
+        rel_ptr, code = _relevant_csr(A, rel, users, profile_items)
+        catalogue = int(listable.sum())
+        metrics = RS.rank_metrics(top, run, rel_ptr, code, n, catalogue=catalogue)
+        reachable = torch.zeros(int(code.numel()), dtype=torch.bool, device=code.device)
+        in_prof = code < n_items
+        reachable[in_prof] = listable[code[in_prof]]
+    counts.update(eval_users=int(users.numel()), **model_count, test_users_untrained=int((has_rel & ~trained).sum()),
+                  test_users_without_relevant=int(len(A.test_users)) - int((has_rel & is_test).sum()),
+                  relevant_items=int(code.numel()), unreachable_items=int((~reachable).sum()),
+                  catalogue_items=catalogue)
+    return metrics
 
 
 @dataclass
@@ -285,42 +294,25 @@ def evaluate_als(A, rank=10, iterations=5, lambda_=0.01, seed=None, alterego=Non
                           events={} if events is not None else None)
 
     with timer("prediction"):
-        n_test = int(A.test_user.numel())
-        prof_of, tu, tpi, untrained, no_profile = _test_pairs(A, profile_items, model.user_count > 0)
+        tu, tpi, untrained, no_profile = _test_pairs(A, profile_items, model.user_count > 0)
         no_factors = ~untrained & ~no_profile & (model.item_count[tpi.clamp(min=0)] == 0)
         ok = torch.nonzero(~untrained & ~no_profile & ~no_factors).flatten()
         p = ALS.predict(model, tu[ok], tpi[ok])
-        pred = torch.full((n_test,), float("nan"), dtype=torch.float64, device=dev)
-        pred[ok] = p
         mae = mae_b = None
         if int(ok.numel()):
             tr = A.test_rating[ok]
             bounded = torch.clamp(torch.trunc(p + 0.5), 0, 5)
             mae = math.fsum((tr - p).abs().cpu().tolist()) / int(ok.numel())
             mae_b = math.fsum((tr - bounded).abs().cpu().tolist()) / int(ok.numel())
-    counts.update(test_pairs=n_test, predicted=int(ok.numel()), skipped_untrained=int(untrained.sum()),
-                  skipped_no_profile=int(no_profile.sum()), skipped_no_factors=int(no_factors.sum()))
+    pred, = _scatter_predictions(counts, ok, (p,), float("nan"), untrained, no_profile, int(ok.numel()),
+                                 skipped_no_factors=int(no_factors.sum()))
 
+    ev = _eval_users(A, threshold)
+    users, run = ev[-2:]
     with timer("top_n"):
-        rel, is_test, has_rel, trained, users, run = _eval_users(A, threshold)
-        cand = torch.nonzero(A.meta.has_T[profile_items] & (model.item_count > 0)).flatten()
-        top = ALS.top_n(model, n, pu, pi, candidates=cand, users=run)
-    with timer("rank_metrics"):
-        rel_ptr, code = _relevant_csr(A, rel, users, prof_of, n_items)
-        catalogue = int(cand.numel())
-        metrics = RS.rank_metrics(top, run, rel_ptr, code, n, catalogue=catalogue)
-        is_cand = torch.zeros(n_items, dtype=torch.bool, device=dev)
-        is_cand[cand] = True
-        in_prof = code < n_items
-        reachable = torch.zeros(int(code.numel()), dtype=torch.bool, device=dev)
-        reachable[in_prof] = is_cand[code[in_prof]]
-    counts.update(eval_users=int(users.numel()), eval_users_without_factors=int((model.user_count[run] == 0).sum()),
-                  test_users_untrained=int((has_rel & ~trained).sum()),
-                  test_users_without_relevant=int(len(A.test_users)) - int((has_rel & is_test).sum()),
-                  relevant_items=int(code.numel()), unreachable_items=int((~reachable).sum()),
-                  catalogue_items=catalogue)
-    stage_ms = None
-    if events is not None:
-        torch.cuda.synchronize(dev)
-        stage_ms = {k: sum(a.elapsed_time(b) for a, b in v) for k, v in events.items()}
-    return AlsEvaluation(mae, mae_b, pred, users, metrics, top, model, profile_items, pu, pi, pr, n, counts, stage_ms)
+        listable = A.meta.has_T[profile_items] & (model.item_count > 0)
+        top = ALS.top_n(model, n, pu, pi, candidates=torch.nonzero(listable).flatten(), users=run)
+    metrics = _rank_tail(A, ev, top, profile_items, listable, n, timer, counts,
+                         eval_users_without_factors=int((model.user_count[run] == 0).sum()))
+    return AlsEvaluation(mae, mae_b, pred, users, metrics, top, model, profile_items, pu, pi, pr, n, counts,
+                         timer.stage_ms())

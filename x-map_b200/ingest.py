@@ -66,6 +66,13 @@ class _Timer(object):
     def __call__(self, name):
         return _Phase(self.events, name)
 
+    def stage_ms(self):
+        """Device time per phase in ms, summed over its event pairs, or None without events."""
+        if self.events is None:
+            return None
+        torch.cuda.synchronize()
+        return {k: sum(a.elapsed_time(b) for a, b in v) for k, v in self.events.items()}
+
 
 class _Phase(object):
     def __init__(self, events, name):

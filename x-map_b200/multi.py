@@ -91,6 +91,25 @@ def allgather_rows(t, shard, group=None):
     return t
 
 
+def shard_selected(sel, weight, group=None):
+    """Split the selected rows sel over the ranks of `group` in contiguous blocks of sel of equal total weight
+    (weight[q]: the work of row sel[q]).  Returns (the shard of positions in sel, the rows this rank computes)."""
+    sh = RowShard(weight, dist.get_rank(group), dist.get_world_size(group))
+    return sh, sel[sh.lo:sh.hi]
+
+
+def gather_selected(ts, shard, sel=None, group=None):
+    """ts: tensors whose dim 0 is the row axis, each rank having filled the rows sel[shard.lo:shard.hi].  After the
+    call every rank holds every selected row; sel None means every row in order."""
+    if sel is None:
+        allgather_rows(ts, shard, group)
+        return
+    rows = [t[sel] for t in ts]                 # the selected rows side by side, in the order of sel
+    allgather_rows(rows, shard, group)
+    for t, r in zip(ts, rows):
+        t[sel] = r
+
+
 def _all_to_all(recv, send, group=None):
     """dist.all_to_all where the backend has it (NCCL); point-to-point otherwise (gloo)."""
     if dist.get_backend(group) == "nccl":

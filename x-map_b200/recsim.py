@@ -10,15 +10,12 @@ import numpy as np
 import torch
 
 from . import _native as N
+from . import multi as M
 
 # Peak device bytes per co-rating entry while a pass runs: key and record positions (16), the stable sort's keys,
 # permutation and scratch (~32), the permuted positions (8), rounded up for the pair outputs.
 ENTRY_BYTES = 64
 INT32_MAX = (1 << 31) - 1
-
-
-def _st():
-    return torch.cuda.current_stream().cuda_stream
 
 
 @dataclass
@@ -79,8 +76,8 @@ def item_info(item, rating, n_items, device="cuda"):
     item_ptr = torch.zeros(n_items + 1, dtype=torch.int64, device=dev)
     item_ptr[1:] = torch.cumsum(torch.bincount(item, minlength=n_items), 0)
     info = torch.zeros((n_items, 3), dtype=torch.float64, device=dev)
-    N.check(L.xmap_recsim_item_info(N.ptr(item_ptr), N.ptr(rating[oi].contiguous()), n_items, N.ptr(info), _st()),
-            "xmap_recsim_item_info")
+    N.check(L.xmap_recsim_item_info(N.ptr(item_ptr), N.ptr(rating[oi].contiguous()), n_items, N.ptr(info),
+                                    N.stream()), "xmap_recsim_item_info")
     return info
 
 
@@ -121,7 +118,7 @@ class _Profile(object):
         src = torch.empty(total, **i64)
         N.check(L.xmap_recsim_fill_rows(N.ptr(self.user_ptr), self.n_users, N.ptr(in_before), N.ptr(ent_before), self.n_rec,
                                         N.ptr(self.item), self.n_items, int(i0), int(i1), total, N.ptr(key), N.ptr(src),
-                                        _st()), "xmap_recsim_fill_rows")
+                                        N.stream()), "xmap_recsim_fill_rows")
         del in_before, ent_before
         key_s, perm = torch.sort(key, stable=True)          # CUB radix sort (library plumbing); stable: arrival order kept
         del key
@@ -139,7 +136,7 @@ class _Profile(object):
         out_ls = torch.empty(n_pairs, dtype=torch.float64, device=dev)
         N.check(L.xmap_recsim_pairs(N.ptr(seg_ptr), N.ptr(seg_key.contiguous()), N.ptr(src_s), N.ptr(self.rating),
                                     N.ptr(self.info), self.n_items, n_pairs, int(num_atleast), N.ptr(out_i), N.ptr(out_j),
-                                    N.ptr(out_n), N.ptr(out_sim), N.ptr(out_ls), _st()), "xmap_recsim_pairs")
+                                    N.ptr(out_n), N.ptr(out_sim), N.ptr(out_ls), N.stream()), "xmap_recsim_pairs")
         return RecSim(out_i, out_j, out_n, out_sim, out_ls, self.info, total)
 
     def plan(self, budget, lo=0, hi=None):
@@ -182,26 +179,28 @@ def _row_ptr(i, lo, n_rows):
 def _neighbors_into(rs, i0, i1, nb):
     """Non-private selection for the rows [i0, i1) of nb (rs: the pairs of exactly those rows)."""
     N.check(N.lib().xmap_recsim_neighbors(N.ptr(_row_ptr(rs.i, i0, i1 - i0)), N.ptr(rs.j.contiguous()),
-                                          N.ptr(rs.sim.contiguous()), i1 - i0, int(nb.idx.shape[1]), N.ptr(nb.idx[i0:i1]),
-                                          N.ptr(nb.sim[i0:i1]), N.ptr(nb.len[i0:i1]), _st()), "xmap_recsim_neighbors")
+                                          N.ptr(rs.sim.contiguous()), i1 - i0, int(nb.idx.shape[1]),
+                                          N.ptr(nb.idx[i0:i1]), N.ptr(nb.sim[i0:i1]), N.ptr(nb.len[i0:i1]),
+                                          N.stream()), "xmap_recsim_neighbors")
 
 
-def _empty_tables(n_items, k, dev):
-    return Neighbors(torch.full((n_items, k), -1, dtype=torch.int32, device=dev),
-                     torch.zeros((n_items, k), dtype=torch.float64, device=dev),
-                     torch.zeros(n_items, dtype=torch.int32, device=dev))
+def empty_tables(n_rows, k, dev):
+    """Neighbour tables with no neighbour in any row: idx -1, sim 0, len 0."""
+    return Neighbors(torch.full((n_rows, k), -1, dtype=torch.int32, device=dev),
+                     torch.zeros((n_rows, k), dtype=torch.float64, device=dev),
+                     torch.zeros(n_rows, dtype=torch.int32, device=dev))
 
 
 def neighbors(rs, n_items, k=10):
     """RecommenderPrivacy.nonprivate_neighbor_selection + nonnoise_perturbation (recommenderPrivacy.py:141-189):
     {item: [(neighbour, sim)] first k by |sim|} as fixed-width tables."""
-    nb = _empty_tables(n_items, k, rs.i.device)
+    nb = empty_tables(n_items, k, rs.i.device)
     if n_items > 0:
         _neighbors_into(rs, 0, n_items, nb)
     return nb
 
 
-def _per_item_uniforms(u, have, n_items, dev):
+def per_item_uniforms(u, have, n_items, dev):
     """One injected uniform per item that has neighbours (have: those items, ascending) -> [n_items], or None."""
     if u is None:
         return None
@@ -213,26 +212,41 @@ def _per_item_uniforms(u, have, n_items, dev):
     return full
 
 
-def _private_into(rs, i0, i1, nb, n_items, mapping_range, privacy_epsilon, rpo, up, un, seed):
-    """Private selection for the rows [i0, i1) of nb (rs: the pairs of exactly those rows).  The kernel runs over
-    every item, so the Philox counter and the uniforms stay indexed by the global item; the other rows are empty."""
-    dev = rs.i.device
-    cnt = torch.zeros(n_items, dtype=torch.int64, device=dev)
-    cnt[i0:i1] = torch.bincount(rs.i.long() - i0, minlength=i1 - i0)
-    row_ptr = torch.zeros(n_items + 1, dtype=torch.int64, device=dev)
-    row_ptr[1:] = torch.cumsum(cnt, 0)
-    # |sim| descending, stable (ties keep the (i, j) order), inside every item (recommenderPrivacy.py:123)
-    o1 = torch.sort(rs.sim.abs(), descending=True, stable=True).indices
-    o = o1[torch.sort(rs.i.long()[o1], stable=True).indices]
-    nbr, sim, ls = rs.j[o].contiguous(), rs.sim[o].contiguous(), rs.ls[o].contiguous()
+def private_options(private, have, n_rows, dev):
+    """private (a dict of private_neighbors' keywords) over their defaults, with u_pick / u_noise spread to one uniform
+    per row (have: the rows that have a pair, ascending).  An unknown keyword raises TypeError."""
+    opts = dict(privacy_epsilon=0.6, rpo=0.1, u_pick=None, u_noise=None, seed=0)
+    unknown = set(private) - set(opts)
+    if unknown:
+        raise TypeError("unknown private selection options: %s" % sorted(unknown))
+    opts.update(private)
+    for u in ("u_pick", "u_noise"):
+        opts[u] = per_item_uniforms(opts[u], have, n_rows, dev)
+    return opts
+
+
+def private_draw(row, nbr, sim, ls, rows, nb, mapping_range, opts):
+    """Private selection into the rows `rows` (an index tensor or a slice) of nb from their pairs (row, nbr, sim, ls),
+    each row's pairs in neighbour order.  opts: private_options.  The kernel runs over every row of nb, so the Philox
+    counter and the uniforms stay indexed by the global row; rows without pairs here come out empty."""
+    dev = sim.device
+    n_rows = int(nb.idx.shape[0])
+    row_ptr = torch.zeros(n_rows + 1, dtype=torch.int64, device=dev)
+    row_ptr[1:] = torch.cumsum(torch.bincount(row, minlength=n_rows), 0)
+    # |sim| descending, stable (ties keep the neighbour order), inside every row (recommenderPrivacy.py:123)
+    o1 = torch.sort(sim.abs(), descending=True, stable=True).indices
+    o = o1[torch.sort(row[o1], stable=True).indices]
+    nbr, sim, ls = nbr[o].contiguous(), sim[o].contiguous(), ls[o].contiguous()
     scratch = torch.empty(max(int(sim.numel()), 1), dtype=torch.float64, device=dev)
-    out = _empty_tables(n_items, 1, dev)
-    N.check(N.lib().xmap_recsim_private_neighbor(N.ptr(row_ptr), N.ptr(nbr), N.ptr(sim), N.ptr(ls), n_items,
-                                                 int(mapping_range), float(privacy_epsilon) / 2.0, float(rpo), N.ptr(up),
-                                                 N.ptr(un), int(seed) & (2 ** 64 - 1), N.ptr(scratch), N.ptr(out.idx),
-                                                 N.ptr(out.sim), N.ptr(out.len), _st()), "xmap_recsim_private_neighbor")
+    out = empty_tables(n_rows, 1, dev)
+    N.check(N.lib().xmap_recsim_private_neighbor(N.ptr(row_ptr), N.ptr(nbr), N.ptr(sim), N.ptr(ls), n_rows,
+                                                 int(mapping_range), float(opts["privacy_epsilon"]) / 2.0,
+                                                 float(opts["rpo"]), N.ptr(opts["u_pick"]), N.ptr(opts["u_noise"]),
+                                                 int(opts["seed"]) & (2 ** 64 - 1), N.ptr(scratch), N.ptr(out.idx),
+                                                 N.ptr(out.sim), N.ptr(out.len), N.stream()),
+            "xmap_recsim_private_neighbor")
     for a, b in zip((nb.idx, nb.sim, nb.len), (out.idx, out.sim, out.len)):
-        a[i0:i1] = b[i0:i1]
+        a[rows] = b[rows]
 
 
 def private_neighbors(rs, n_items, mapping_range=10, privacy_epsilon=0.6, rpo=0.1, u_pick=None, u_noise=None, seed=0):
@@ -242,10 +256,11 @@ def private_neighbors(rs, n_items, mapping_range=10, privacy_epsilon=0.6, rpo=0.
     order (the reference's np.random draws replayed), or None -> Philox4x32-10(seed, item).  Returns Neighbors with k = 1."""
     dev = rs.i.device
     have = torch.nonzero(torch.bincount(rs.i.long(), minlength=n_items) > 0).flatten()
-    up, un = _per_item_uniforms(u_pick, have, n_items, dev), _per_item_uniforms(u_noise, have, n_items, dev)
-    nb = _empty_tables(n_items, 1, dev)
+    opts = private_options(dict(privacy_epsilon=privacy_epsilon, rpo=rpo, u_pick=u_pick, u_noise=u_noise, seed=seed),
+                           have, n_items, dev)
+    nb = empty_tables(n_items, 1, dev)
     if n_items > 0:
-        _private_into(rs, 0, n_items, nb, n_items, mapping_range, privacy_epsilon, rpo, up, un, seed)
+        private_draw(rs.i.long(), rs.j, rs.sim, rs.ls, slice(0, n_items), nb, mapping_range, opts)
     return nb
 
 
@@ -274,23 +289,13 @@ def item_knn(user, item, rating, n_items, num_atleast=50, k=10, private=None, bu
     dev = prof.dev
     if budget is None:
         budget = default_budget(dev)
-    sh = None
-    if shard:
-        import torch.distributed as dist
-        from .multi import RowShard
-        sh = RowShard(prof.row_ent, dist.get_rank(group), dist.get_world_size(group))
+    sh = M.RowShard(prof.row_ent, M.dist.get_rank(group), M.dist.get_world_size(group)) if shard else None
     lo, hi = (sh.lo, sh.hi) if sh is not None else (0, n_items)
     bounds = prof.plan(budget, lo, hi)                           # checks every row, so all ranks fail alike
     if private is not None:
-        opts = dict(privacy_epsilon=0.6, rpo=0.1, u_pick=None, u_noise=None, seed=0)
-        unknown = set(private) - set(opts)
-        if unknown:
-            raise TypeError("unknown private selection options: %s" % sorted(unknown))
-        opts.update(private)
-        have = torch.nonzero(prof.row_ent > 0).flatten()          # an item has a pair iff it owns an entry
-        up = _per_item_uniforms(opts["u_pick"], have, n_items, dev)
-        un = _per_item_uniforms(opts["u_noise"], have, n_items, dev)
-    nb = _empty_tables(n_items, 1 if private is not None else k, dev)
+        # an item has a pair iff it owns an entry
+        opts = private_options(private, torch.nonzero(prof.row_ent > 0).flatten(), n_items, dev)
+    nb = empty_tables(n_items, 1 if private is not None else k, dev)
     n_entries = passes = 0
     for i0, i1 in zip(bounds[:-1], bounds[1:]):
         if i1 == i0:
@@ -301,11 +306,10 @@ def item_knn(user, item, rating, n_items, num_atleast=50, k=10, private=None, bu
         if private is None:
             _neighbors_into(rs, i0, i1, nb)
         else:
-            _private_into(rs, i0, i1, nb, n_items, k, opts["privacy_epsilon"], opts["rpo"], up, un, opts["seed"])
+            private_draw(rs.i.long(), rs.j, rs.sim, rs.ls, slice(i0, i1), nb, k, opts)
         del rs
     if sh is not None:
-        from .multi import allgather_rows
-        allgather_rows([nb.idx, nb.sim, nb.len], sh, group)
+        M.gather_selected([nb.idx, nb.sim, nb.len], sh, group=group)
     return ItemKnn(nb, prof.info, n_entries, passes,
                    int(prof.row_ent.max().item()) if n_items else 0)
 
@@ -343,7 +347,7 @@ def predict(user, item, rating, ts, n_users, rs, nb, test_user, test_item, test_
     k = int(nb.idx.shape[1])
     N.check(L.xmap_recsim_predict(N.ptr(prof_ptr), N.ptr(p_item), N.ptr(p_rating), N.ptr(p_ts), N.ptr(rs.info),
                                   N.ptr(nb.idx), N.ptr(nb.sim), N.ptr(nb.len), k, N.ptr(tu), N.ptr(ti), n_test,
-                                  float(alpha), N.ptr(p0), N.ptr(p1), N.ptr(err), _st()), "xmap_recsim_predict")
+                                  float(alpha), N.ptr(p0), N.ptr(p1), N.ptr(err), N.stream()), "xmap_recsim_predict")
     if int(err.item()):
         raise N.NativeError("prediction kernel error %d (4: more than 128 matching profile records)" % int(err.item()))
     mae0 = mae1 = None
@@ -355,6 +359,41 @@ def predict(user, item, rating, ts, n_users, rs, nb, test_user, test_item, test_
             mae0 = float((tr[ok] - p0[ok]).abs().sum().item()) / cnt          # recommenderPrediction.py:116-139
             mae1 = float((tr[ok] - p1[ok]).abs().sum().item()) / cnt
     return p0, p1, mae0, mae1
+
+
+def index_set(t, n_max, dev, name="users"):
+    """t as int64 on dev, checked to be a 1-D integer tensor of indices in [0, n_max)."""
+    t = torch.as_tensor(t)
+    if t.dim() != 1 or t.dtype.is_floating_point or t.dtype.is_complex or t.dtype == torch.bool:
+        raise ValueError("%s must be a 1-D integer tensor" % name)
+    t = t.to(device=dev, dtype=torch.int64)
+    if t.numel() and (int(t.min()) < 0 or int(t.max()) >= n_max):
+        raise ValueError("%s outside [0, %d)" % (name, n_max))
+    return t
+
+
+def query_users(users, n_users, dev):
+    """The rows a call computes: every user for None, else `users` checked as an index set of distinct users."""
+    if users is None:
+        return torch.arange(max(n_users, 0), dtype=torch.int64, device=dev)
+    sel = index_set(users, n_users, dev)
+    if int(torch.unique(sel).numel()) != int(sel.numel()):
+        raise ValueError("users must be distinct")
+    return sel
+
+
+def list_length(n, hi=N.TOPN_MAX):
+    """n checked as the length of a top-N list: an integer in [1, hi]."""
+    if isinstance(n, bool) or int(n) != n or not 1 <= int(n) <= hi:
+        raise ValueError("n must be an integer in [1, %d], got %r" % (hi, n))
+    return int(n)
+
+
+def empty_lists(n_rows, n, dev):
+    """(idx, score, len) of n_rows top-N lists of width n before any is filled: idx -1, score NaN, len 0."""
+    return (torch.full((n_rows, n), -1, dtype=torch.int32, device=dev),
+            torch.full((n_rows, n), float("nan"), dtype=torch.float64, device=dev),
+            torch.zeros(n_rows, dtype=torch.int32, device=dev))
 
 
 @dataclass
@@ -398,9 +437,7 @@ def top_n(user, item, rating, ts, n_users, knn, nb, n, decay=False, alpha=0.03, 
     users: None for every user, or a 1-D integer tensor of distinct users in [0, n_users): only their rows are filled
     (the others keep the padding), and the counts refer to them; shard then splits these users.
     Raises NativeError (error 4) when a candidate gathers more than 128 matching profile records, as predict does."""
-    if isinstance(n, bool) or int(n) != n or not 1 <= int(n) <= N.TOPN_MAX:
-        raise ValueError("n must be an integer in [1, %d], got %r" % (N.TOPN_MAX, n))
-    n = int(n)
+    n = list_length(n)
     L = N.lib()
     dev = knn.info.device
     n_items = int(nb.idx.shape[0])
@@ -414,17 +451,7 @@ def top_n(user, item, rating, ts, n_users, knn, nb, n, decay=False, alpha=0.03, 
         raise ValueError("user outside [0, %d)" % n_users)
     if n_rec and (int(item.min()) < 0 or int(item.max()) >= n_items):
         raise ValueError("item outside [0, %d)" % n_items)
-    if users is None:
-        sel = torch.arange(max(n_users, 0), dtype=torch.int64, device=dev)
-    else:
-        sel = torch.as_tensor(users)
-        if sel.dim() != 1 or sel.dtype.is_floating_point or sel.dtype.is_complex or sel.dtype == torch.bool:
-            raise ValueError("users must be a 1-D integer tensor")
-        sel = sel.to(device=dev, dtype=torch.int64)
-        if sel.numel() and (int(sel.min()) < 0 or int(sel.max()) >= n_users):
-            raise ValueError("users outside [0, %d)" % n_users)
-        if int(torch.unique(sel).numel()) != int(sel.numel()):
-            raise ValueError("users must be distinct")
+    sel = query_users(users, n_users, dev)
     # the records grouped by user, stably by item inside each user: a candidate's entries are runs in list order
     o = torch.argsort(user * n_items + item, stable=True)
     prof_ptr = torch.zeros(n_users + 1, dtype=torch.int64, device=dev)
@@ -435,13 +462,7 @@ def top_n(user, item, rating, ts, n_users, knn, nb, n, decay=False, alpha=0.03, 
     rev_ptr, rev_item = reverse_index(nb)
     # per user: sum over its records j of |rev(j)|, the bound on the overlap candidates it visits (one scatter-add)
     bound = torch.zeros(n_users, dtype=torch.int64, device=dev).index_add_(0, user, (rev_ptr[1:] - rev_ptr[:-1])[item])
-    sh = None
-    mine = sel
-    if shard:
-        import torch.distributed as dist
-        from .multi import RowShard
-        sh = RowShard(bound[sel], dist.get_rank(group), dist.get_world_size(group))
-        mine = sel[sh.lo:sh.hi]
+    sh, mine = M.shard_selected(sel, bound[sel], group) if shard else (None, sel)
     light = bound[mine] <= N.TOPN_WARP_BOUND
     warp_users = mine[light].to(torch.int32).contiguous()
     heavy = mine[~light]
@@ -450,9 +471,7 @@ def top_n(user, item, rating, ts, n_users, knn, nb, n, decay=False, alpha=0.03, 
     avg = knn.info[:, 0]
     fb = torch.nonzero((nb.len > 0) & (avg == avg)).flatten()
     fb = fb[torch.sort(avg[fb] + 0.0, descending=True, stable=True).indices].to(torch.int32).contiguous()
-    out_idx = torch.full((n_users, n), -1, dtype=torch.int32, device=dev)
-    out_score = torch.full((n_users, n), float("nan"), dtype=torch.float64, device=dev)
-    out_len = torch.zeros(n_users, dtype=torch.int32, device=dev)
+    out_idx, out_score, out_len = empty_lists(n_users, n, dev)
     stats = torch.zeros(2, dtype=torch.int64, device=dev)
     err = torch.zeros(1, dtype=torch.int32, device=dev)
     N.check(L.xmap_recsim_top_n(N.ptr(prof_ptr), N.ptr(p_item), N.ptr(p_rating), N.ptr(p_ts), N.ptr(knn.info.contiguous()),
@@ -460,17 +479,11 @@ def top_n(user, item, rating, ts, n_users, knn, nb, n, decay=False, alpha=0.03, 
                                 int(nb.idx.shape[1]), n_items, N.ptr(rev_ptr), N.ptr(rev_item), N.ptr(fb), int(fb.numel()),
                                 N.ptr(warp_users), int(warp_users.numel()), N.ptr(cta_users), int(cta_users.numel()), n,
                                 float(alpha), 1 if decay else 0, N.ptr(out_idx), N.ptr(out_score), N.ptr(out_len),
-                                N.ptr(stats), N.ptr(err), _st()), "xmap_recsim_top_n")
+                                N.ptr(stats), N.ptr(err), N.stream()), "xmap_recsim_top_n")
     if int(err.item()):
         raise N.NativeError("top-N kernel error %d (4: more than 128 matching profile records)" % int(err.item()))
     if sh is not None:
-        from .multi import allgather_rows
-        if users is None:
-            allgather_rows([out_idx, out_score, out_len], sh, group)
-        else:                                   # the selected rows side by side, in the order of `users`
-            rows = [out_idx[sel], out_score[sel], out_len[sel]]
-            allgather_rows(rows, sh, group)
-            out_idx[sel], out_score[sel], out_len[sel] = rows
+        M.gather_selected([out_idx, out_score, out_len], sh, None if users is None else sel, group)
     visits, cands = stats.tolist()
     return TopN(out_idx, out_score, out_len, visits, cands, int(warp_users.numel()), int(cta_users.numel()))
 
@@ -504,16 +517,9 @@ def rank_metrics(top, users, rel_ptr, rel_item, n, catalogue=None):
     if idx.dim() != 2 or ln.dim() != 1 or int(ln.numel()) != int(idx.shape[0]):
         raise ValueError("top lists: idx must be [n_users, width] and len [n_users]")
     width = int(idx.shape[1])
-    if isinstance(n, bool) or int(n) != n or not 1 <= int(n) <= min(width, N.TOPN_MAX):
-        raise ValueError("n must be an integer in [1, %d], got %r" % (min(width, N.TOPN_MAX), n))
-    n = int(n)
-    u = torch.as_tensor(users)
-    if u.dim() != 1 or u.dtype.is_floating_point or u.dtype == torch.bool:
-        raise ValueError("users must be a 1-D integer tensor")
-    u = u.to(device=dev, dtype=torch.int64)
+    n = list_length(n, min(width, N.TOPN_MAX))
+    u = index_set(users, int(idx.shape[0]), dev)           # repeats allowed
     m = int(u.numel())
-    if m and (int(u.min()) < 0 or int(u.max()) >= int(idx.shape[0])):
-        raise ValueError("users outside [0, %d)" % int(idx.shape[0]))
     ptr = torch.as_tensor(rel_ptr).to(device=dev, dtype=torch.int64).flatten()
     it = torch.as_tensor(rel_item).to(device=dev, dtype=torch.int64).flatten()
     if int(ptr.numel()) != m + 1 or int(ptr[0]) != 0 or int(ptr[-1]) != int(it.numel()):
@@ -534,7 +540,8 @@ def rank_metrics(top, users, rel_ptr, rel_item, n, catalogue=None):
     idx_c, ln32 = idx.contiguous(), ln.to(torch.int32).contiguous()
     u32, it32 = u.to(torch.int32).contiguous(), it.to(torch.int32).contiguous()
     N.check(N.lib().xmap_recsim_rank_metrics(N.ptr(idx_c), N.ptr(ln32), width, N.ptr(u32), m, N.ptr(ptr), N.ptr(it32),
-                                             N.ptr(disc), n, *(N.ptr(t) for t in out), _st()), "xmap_recsim_rank_metrics")
+                                             N.ptr(disc), n, *(N.ptr(t) for t in out), N.stream()),
+            "xmap_recsim_rank_metrics")
     mean = None
     if m:
         mean = {k: math.fsum(t.cpu().tolist()) / m for k, t in zip(("precision", "recall", "ndcg", "map"), out[1:])}

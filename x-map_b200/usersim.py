@@ -10,25 +10,8 @@ from dataclasses import dataclass
 import torch
 
 from . import _native as N
+from . import multi as M
 from . import recsim as RS
-
-
-def _st():
-    return torch.cuda.current_stream().cuda_stream
-
-
-def _users_arg(users, n_users, dev):
-    if users is None:
-        return torch.arange(max(n_users, 0), dtype=torch.int64, device=dev)
-    sel = torch.as_tensor(users)
-    if sel.dim() != 1 or sel.dtype.is_floating_point or sel.dtype.is_complex or sel.dtype == torch.bool:
-        raise ValueError("users must be a 1-D integer tensor")
-    sel = sel.to(device=dev, dtype=torch.int64)
-    if sel.numel() and (int(sel.min()) < 0 or int(sel.max()) >= n_users):
-        raise ValueError("users outside [0, %d)" % n_users)
-    if int(torch.unique(sel).numel()) != int(sel.numel()):
-        raise ValueError("users must be distinct")
-    return sel
 
 
 def scale_base(max_dup):
@@ -104,14 +87,7 @@ def _launch(prof, rows, cta, tile, num_atleast, k, nb, emit, stats, err):
                                       1 if cta else 0, int(tile), N.ptr(nb.idx) if nb else None,
                                       N.ptr(nb.sim) if nb else None, N.ptr(nb.len) if nb else None, N.ptr(e_ptr),
                                       N.ptr(e_v), N.ptr(e_n), N.ptr(e_sim), N.ptr(e_ls), N.ptr(e_len), N.ptr(stats),
-                                      N.ptr(err), _st()), "xmap_usersim_rows")
-
-
-def emit_plan(bound, budget):
-    """Cut the query rows (bound: the pair bound of each, in order) into consecutive blocks of at most `budget` bytes,
-    recsim.ENTRY_BYTES per pair ((v, n, sim, ls) and the two stable sorts by |sim| and row fit in it).  Returns the
-    block bounds [0, ..., len].  A row over the budget raises ValueError."""
-    return RS.pass_plan(bound, budget)
+                                      N.ptr(err), N.stream()), "xmap_usersim_rows")
 
 
 def user_knn(user, item, rating, n_users, n_items, num_atleast=50, k=10, private=None, users=None, budget=None,
@@ -131,66 +107,54 @@ def user_knn(user, item, rating, n_users, n_items, num_atleast=50, k=10, private
     tile: cells per pass (None: the shape's default); emit_cap: per-row extent override, for tests of the overflow."""
     prof = UserProfile(user, item, rating, n_users, n_items, device)
     dev = prof.dev
-    sel = _users_arg(users, n_users, dev)
-    sh = None
-    mine = sel
-    if shard:
-        import torch.distributed as dist
-        from .multi import RowShard
-        sh = RowShard(prof.row_products[sel], dist.get_rank(group), dist.get_world_size(group))
-        mine = sel[sh.lo:sh.hi]
-    heavy = prof.row_products[mine] > N.USERSIM_WARP_BOUND
-    if shape == "warp":
-        heavy = torch.zeros_like(heavy)
-    elif shape == "cta":
-        heavy = torch.ones_like(heavy)
-    elif shape is not None:
-        raise ValueError("shape must be None, 'warp' or 'cta'")
+    sel = RS.query_users(users, n_users, dev)
+    sh, mine = M.shard_selected(sel, prof.row_products[sel], group) if shard else (None, sel)
+    heavy = _launch_shape(prof.row_products[mine] > N.USERSIM_WARP_BOUND, shape)
     groups = [(mine[~heavy], False), (mine[heavy], True)]
     stats = torch.zeros(3, dtype=torch.int64, device=dev)
     err = torch.zeros(1, dtype=torch.int32, device=dev)
     blocks = 0
     if private is None:
-        nb = RS._empty_tables(n_users, k, dev)
+        nb = RS.empty_tables(n_users, k, dev)
         for rows, cta in groups:
             t = tile or (N.USERSIM_CTA_TILE if cta else N.USERSIM_WARP_TILE)
             _launch(prof, rows.to(torch.int32).contiguous(), cta, t, num_atleast, k, nb, None, stats, err)
     else:
-        opts = dict(privacy_epsilon=0.6, rpo=0.1, u_pick=None, u_noise=None, seed=0)
-        unknown = set(private) - set(opts)
-        if unknown:
-            raise TypeError("unknown private selection options: %s" % sorted(unknown))
-        opts.update(private)
-        have = torch.nonzero(prof.row_products > 0).flatten()          # a user has a pair iff it owns a product
-        up = RS._per_item_uniforms(opts["u_pick"], have, n_users, dev)
-        un = RS._per_item_uniforms(opts["u_noise"], have, n_users, dev)
-        nb = RS._empty_tables(n_users, 1, dev)
-        for rows, emit in _emit_blocks(prof, groups, num_atleast, budget, tile, emit_cap, stats, err):
+        # a user has a pair iff it owns a product
+        opts = RS.private_options(private, torch.nonzero(prof.row_products > 0).flatten(), n_users, dev)
+        nb = RS.empty_tables(n_users, 1, dev)
+        for rows, row, v, _n, sim, ls in _emit_blocks(prof, groups, num_atleast, budget, tile, emit_cap, stats, err):
             blocks += 1
-            _private_rows(emit, rows, nb, n_users, k, opts, up, un)
+            RS.private_draw(row, v, sim, ls, rows, nb, k, opts)
     if int(err.item()):
         raise N.NativeError("user similarity kernel error %d" % int(err.item()))
     if sh is not None:
-        from .multi import allgather_rows
-        if users is None:
-            allgather_rows([nb.idx, nb.sim, nb.len], sh, group)
-        else:                                   # the selected rows side by side, in the order of `users`
-            rows = [nb.idx[sel], nb.sim[sel], nb.len[sel]]
-            allgather_rows(rows, sh, group)
-            nb.idx[sel], nb.sim[sel], nb.len[sel] = rows
+        M.gather_selected([nb.idx, nb.sim, nb.len], sh, None if users is None else sel, group)
     products, pairs, passes = stats.tolist()
     return UserKnn(nb, prof.info, products, pairs, passes, int((~heavy).sum()), int(heavy.sum()), blocks)
 
 
+def _launch_shape(heavy, shape):
+    """heavy (the rows their work sends to the one-CTA shape), or every row in the shape `shape` names."""
+    if shape == "warp":
+        return torch.zeros_like(heavy)
+    if shape == "cta":
+        return torch.ones_like(heavy)
+    if shape is not None:
+        raise ValueError("shape must be None, 'warp' or 'cta'")
+    return heavy
+
+
 def _emit_blocks(prof, groups, num_atleast, budget, tile, emit_cap, stats, err):
     """Emit mode over the query rows of each (rows, cta) group, in blocks of at most `budget` bytes: yields (rows of
-    the block, (e_ptr, e_v, e_n, e_sim, e_ls, e_len)), the pairs of row q at e_ptr[q] .. + e_len[q], in user order."""
+    the block, then of every pair emitted for them its row, v, n, sim and ls), each row's pairs in user order."""
     dev = prof.dev
     if budget is None:
         budget = RS.default_budget(dev)
     for rows, cta in groups:
         bound = torch.clamp(prof.row_products[rows], max=prof.n_users)
-        bounds = emit_plan(bound, budget)
+        # recsim.ENTRY_BYTES per pair: (v, n, sim, ls) and the private draw's two stable sorts fit in it
+        bounds = RS.pass_plan(bound, budget)
         t = tile or (N.USERSIM_EMIT_CTA_TILE if cta else N.USERSIM_WARP_TILE)
         for b0, b1 in zip(bounds[:-1], bounds[1:]):
             if b1 == b0:
@@ -199,15 +163,18 @@ def _emit_blocks(prof, groups, num_atleast, budget, tile, emit_cap, stats, err):
             cap = bound[b0:b1] if emit_cap is None else torch.full_like(bound[b0:b1], int(emit_cap))
             e_ptr = torch.zeros(b1 - b0 + 1, dtype=torch.int64, device=dev)
             e_ptr[1:] = torch.cumsum(cap, 0)
-            tot = max(int(e_ptr[-1]), 1)
-            emit = (e_ptr, torch.empty(tot, dtype=torch.int32, device=dev), torch.empty(tot, dtype=torch.int64, device=dev),
-                    torch.empty(tot, dtype=torch.float64, device=dev), torch.empty(tot, dtype=torch.float64, device=dev),
-                    torch.zeros(b1 - b0, dtype=torch.int64, device=dev))
-            _launch(prof, r.to(torch.int32).contiguous(), cta, t, num_atleast, 1, None, emit, stats, err)
+            tot = int(e_ptr[-1])
+            pairs = [torch.empty(max(tot, 1), dtype=dt, device=dev)                     # v, n, sim, ls
+                     for dt in (torch.int32, torch.int64, torch.float64, torch.float64)]
+            e_len = torch.zeros(b1 - b0, dtype=torch.int64, device=dev)
+            _launch(prof, r.to(torch.int32).contiguous(), cta, t, num_atleast, 1, None, (e_ptr, *pairs, e_len), stats,
+                    err)
             if int(err.item()):
                 raise N.NativeError("user similarity kernel error %d (2: a row has more pairs than its extent)"
                                     % int(err.item()))
-            yield r, emit
+            row_of = torch.repeat_interleave(torch.arange(b1 - b0, device=dev), cap)
+            keep = torch.arange(tot, device=dev) - e_ptr[:-1][row_of] < e_len[row_of]    # the written part of each extent
+            yield (r, r[row_of[keep]]) + tuple(p[:tot][keep] for p in pairs)
 
 
 def pair_blocks(user, item, rating, n_users, n_items, num_atleast=50, budget=None, device="cuda"):
@@ -217,44 +184,8 @@ def pair_blocks(user, item, rating, n_users, n_items, num_atleast=50, budget=Non
     rows = torch.arange(n_users, dtype=torch.int64, device=prof.dev)
     stats = torch.zeros(3, dtype=torch.int64, device=prof.dev)
     err = torch.zeros(1, dtype=torch.int32, device=prof.dev)
-    for r, (e_ptr, e_v, e_n, e_sim, e_ls, e_len) in _emit_blocks(prof, [(rows, False)], num_atleast, budget, None,
-                                                                None, stats, err):
-        row_of = torch.repeat_interleave(torch.arange(int(r.numel()), device=prof.dev), e_ptr[1:] - e_ptr[:-1])
-        tot = int(row_of.numel())
-        keep = torch.arange(tot, device=prof.dev) - e_ptr[:-1][row_of] < e_len[row_of]
-        yield (r[row_of[keep]].to(torch.int32), e_v[:tot][keep], e_n[:tot][keep], e_sim[:tot][keep], e_ls[:tot][keep])
-
-
-def _private_rows(emit, rows, nb, n_users, k, opts, up, un):
-    """The private draw for the emitted rows: each row's pairs sorted stably by |sim| descending (ties keep the user
-    order), then xmap_recsim_private_neighbor over the user axis (Philox counter and uniforms indexed by user)."""
-    e_ptr, e_v, _e_n, e_sim, e_ls, e_len = emit
-    dev = e_v.device
-    m = int(rows.numel())
-    row_of = torch.repeat_interleave(torch.arange(m, device=dev), e_ptr[1:] - e_ptr[:-1])
-    tot = int(row_of.numel())
-    keep = torch.arange(tot, device=dev) - e_ptr[:-1][row_of] < e_len[row_of]        # the written part of each extent
-    q = row_of[keep]
-    v, sim, ls = e_v[:tot][keep], e_sim[:tot][keep], e_ls[:tot][keep]
-    o1 = torch.sort(sim.abs(), descending=True, stable=True).indices
-    o = o1[torch.sort(q[o1], stable=True).indices]
-    u_of = rows[q[o]]
-    # rows ascending by user for the kernel's row_ptr
-    ou = torch.sort(u_of, stable=True).indices
-    nbr, sim_s, ls_s = v[o][ou].contiguous(), sim[o][ou].contiguous(), ls[o][ou].contiguous()
-    cnt = torch.zeros(n_users, dtype=torch.int64, device=dev)
-    cnt[rows] = e_len
-    row_ptr = torch.zeros(n_users + 1, dtype=torch.int64, device=dev)
-    row_ptr[1:] = torch.cumsum(cnt, 0)
-    scratch = torch.empty(max(int(sim_s.numel()), 1), dtype=torch.float64, device=dev)
-    out = RS._empty_tables(n_users, 1, dev)
-    N.check(N.lib().xmap_recsim_private_neighbor(N.ptr(row_ptr), N.ptr(nbr), N.ptr(sim_s), N.ptr(ls_s), n_users, int(k),
-                                                 float(opts["privacy_epsilon"]) / 2.0, float(opts["rpo"]), N.ptr(up),
-                                                 N.ptr(un), int(opts["seed"]) & (2 ** 64 - 1), N.ptr(scratch),
-                                                 N.ptr(out.idx), N.ptr(out.sim), N.ptr(out.len), _st()),
-            "xmap_recsim_private_neighbor")
-    for a, b in zip((nb.idx, nb.sim, nb.len), (out.idx, out.sim, out.len)):
-        a[rows] = b[rows]
+    for _, u, v, n, sim, ls in _emit_blocks(prof, [(rows, False)], num_atleast, budget, None, None, stats, err):
+        yield u.to(torch.int32), v, n, sim, ls
 
 
 def predict(user, item, rating, ts, n_items, knn, nb, test_user, test_item, test_rating=None, alpha=0.03):
@@ -271,16 +202,14 @@ def top_n(user, item, rating, ts, n_users, n_items, knn, nb, n, decay=False, alp
     item; NaN never listed.  An item none of the user's neighbours rated scores avg_u.  A user with no neighbour list
     gets an empty list.  Returns recsim.TopN (rows of users not listed keep the padding).  shape: None (one warp per user
     whose neighbours hold at most XMAP_TOPN_WARP_BOUND records, one CTA above), "warp" or "cta"."""
-    if isinstance(n, bool) or int(n) != n or not 1 <= int(n) <= N.TOPN_MAX:
-        raise ValueError("n must be an integer in [1, %d], got %r" % (N.TOPN_MAX, n))
+    n = RS.list_length(n)
     if ts is None:
         raise ValueError("ts is required: the decay order and the kernels read a time per record")
     if tile is not None and (isinstance(tile, bool) or int(tile) < 32):
         raise ValueError("tile must be an integer >= 32, got %r" % (tile,))
-    n = int(n)
     dev = knn.info.device
     prof = UserProfile(user, item, rating, n_users, n_items, dev, ts=ts)
-    sel = _users_arg(users, n_users, dev)
+    sel = RS.query_users(users, n_users, dev)
     user = torch.as_tensor(user, dtype=torch.int64).to(dev).flatten()
     item = torch.as_tensor(item, dtype=torch.int64).to(dev).flatten()
     o = torch.argsort(user * max(n_items, 1) + item, stable=True)
@@ -289,16 +218,8 @@ def top_n(user, item, rating, ts, n_users, n_items, knn, nb, n, decay=False, alp
     k = int(nb.idx.shape[1])
     valid = torch.arange(k, device=dev).unsqueeze(0) < nb.len.long().unsqueeze(1)
     bound = (d[nb.idx.long().clamp(min=0)] * valid).sum(1)
-    heavy = bound[sel] > N.TOPN_WARP_BOUND
-    if shape == "warp":
-        heavy = torch.zeros_like(heavy)
-    elif shape == "cta":
-        heavy = torch.ones_like(heavy)
-    elif shape is not None:
-        raise ValueError("shape must be None, 'warp' or 'cta'")
-    out_idx = torch.full((n_users, n), -1, dtype=torch.int32, device=dev)
-    out_score = torch.full((n_users, n), float("nan"), dtype=torch.float64, device=dev)
-    out_len = torch.zeros(n_users, dtype=torch.int32, device=dev)
+    heavy = _launch_shape(bound[sel] > N.TOPN_WARP_BOUND, shape)
+    out_idx, out_score, out_len = RS.empty_lists(n_users, n, dev)
     stats = torch.zeros(2, dtype=torch.int64, device=dev)
     err = torch.zeros(1, dtype=torch.int32, device=dev)
     info, nbi, nbs, nbl = knn.info.contiguous(), nb.idx.contiguous(), nb.sim.contiguous(), nb.len.contiguous()
@@ -311,7 +232,7 @@ def top_n(user, item, rating, ts, n_users, n_items, knn, nb, n, decay=False, alp
                                            N.ptr(nbl), k, n_items, N.ptr(rows), int(rows.numel()), 1 if cta else 0,
                                            int(tile or 0), n,
                                            float(alpha), 1 if decay else 0, N.ptr(out_idx), N.ptr(out_score),
-                                           N.ptr(out_len), N.ptr(stats), N.ptr(err), _st()), "xmap_usersim_top_n")
+                                           N.ptr(out_len), N.ptr(stats), N.ptr(err), N.stream()), "xmap_usersim_top_n")
     if int(err.item()):
         raise N.NativeError("top-N kernel error %d (4: more than 128 matching profile records)" % int(err.item()))
     visits, cands = stats.tolist()
